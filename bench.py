@@ -2,6 +2,7 @@
 """Benchmarks of the hot path on synthetic Avenue-shaped clips (BASELINE.json configs).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--batch B] [--frames u8|f32]
+                    [--dump-outputs DIR]
 
 Workloads (``--workload``; the default is the headline, BASELINE.json configs[1]):
   ma_train    C2  M-A (causal_anomaly_detection.py) training step, 32 clips x 16 frames x 240x360 per GPU, bf16 operands  [clips/s]
@@ -18,6 +19,10 @@ One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one
   roofline      the dominant kernel family timed with CUDA events inside the replayed step, against MEASURED_PEAKS.json
   cpu_baseline  the reference's own code (oracle/_ref, kind "reference") or its oracle port (kind "port") on the host cores, bounded sample
   self_check    (ma_train, mc_infer, mb_train) the first step's result against the committed golden fixture made by the unmodified reference
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy: every input and initial state is seeded, so two
+builds run with the same arguments can be compared output for output.  ma_train / mb_train: loss_components and the parameter arena
+after the step (M-A also its anomaly_scores); mc_infer / mc_long: scores_T<T> per sequence length; me_windows: scores, adjacency, features.
 """
 from __future__ import annotations
 
@@ -131,7 +136,23 @@ def ma_noise_for(B, xseed):
 
 
 def gold(name):
-    return torch.load(os.path.join(ROOT, "tests", "golden", name), map_location="cpu", weights_only=False)
+    import synth
+    return synth.golden(name)
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(path, arrays):
+    """``--dump-outputs``: one ``<name>.npy`` per array, float64 kept, everything else written as float32."""
+    import numpy as np
+    host = {k: v.detach().cpu().to(torch.float64 if v.dtype == torch.float64 else torch.float32) for k, v in arrays.items()}
+    total = sum(t.numel() * t.element_size() for t in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for k, t in host.items():
+        np.save(os.path.join(path, k + ".npy"), t.numpy())
 
 
 # ============================================================================================ the reference's CPU arm
@@ -405,8 +426,8 @@ def run_ma_train(args, rank, local, world, dev, dp):
     gs = None
     if args.no_graph:
         def step(x, y):
-            comp, _ = tr.train_step(x, y)
-            return comp
+            comp, out = tr.train_step(x, y)
+            return comp, out["anomaly_scores"]
     else:
         # the whole step (zero_grad, forward, loss, backward, all-reduce, clip+AdamW) is one CUDA graph (two around the all-reduce for N > 1)
         trace("batch resident; capturing the step")
@@ -415,7 +436,7 @@ def run_ma_train(args, rank, local, world, dev, dp):
         x_dev, y_dev = gs.static_inputs
 
         def step(x, y):
-            return gs(x, y)[0]
+            return gs(x, y)
 
     for _ in range(args.warmup):
         step(x_dev, y_dev)
@@ -429,19 +450,21 @@ def run_ma_train(args, rank, local, world, dev, dp):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step(x_dev, y_dev)
+        last = step(x_dev, y_dev)
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     trace(f"timed region done ({ms / args.steps:.3f} ms/step)")
     launches = ops.LAUNCHES[0] - n0
+    if args.dump_outputs and rank == 0:        # before the end-to-end steps below train the model further
+        dump_outputs(args.dump_outputs, {"loss_components": last[0], "anomaly_scores": last[1], "parameters": tr.optimizer.arena.p})
 
     # ---- end to end: pinned host batch -> H2D -> step -> D2H loss, through the public trainer API.  Every step's batch starts in pinned
     # host memory and its loss is read back to the host.  With the graphed trainer the H2D copy of step i+1 is issued before step i's
     # loss is read, so it overlaps step i's compute (all copies are inside the timed region: K+1 batches are copied for K timed steps).
     def e2e_step(first):
         if args.no_graph:
-            return step(x_pin.to(dev, non_blocking=True), y_pin.to(dev, non_blocking=True))
+            return step(x_pin.to(dev, non_blocking=True), y_pin.to(dev, non_blocking=True))[0]
         if first:
             gs.prefetch(x_pin, y_pin)
         out = gs.run_prefetched()[0]
@@ -594,6 +617,9 @@ def run_small(args, rank, local, world, dev, dp):
                 gph(s)
             return graphs[-1].outputs[0]
 
+        def named_outputs(last):
+            return {f"scores_T{t}": gph.outputs[0] for t, gph in zip(Ts, graphs)}
+
         def make_profiled():
             with torch.no_grad():
                 gps = [GraphedStep(lambda x: (model(x),), (h.to(dev),)) for h in hosts]
@@ -645,6 +671,9 @@ def run_small(args, rank, local, world, dev, dp):
         def step_dev():
             return gph(*gph.static_inputs)[0]
 
+        def named_outputs(last):
+            return {"loss_components": last, "parameters": tr.optimizer.arena.p}
+
         def make_profiled():
             gp = tr.graphed_train_step(x_host.to(dev), y_host.to(dev))
             return lambda: gp(*gp.static_inputs)
@@ -668,7 +697,10 @@ def run_small(args, rank, local, world, dev, dp):
         f_pin = frames.pin_memory()
 
         def step_dev():
-            return me.score_windows_device(model, f_dev)[0]
+            return me.score_windows_device(model, f_dev)
+
+        def named_outputs(last):
+            return dict(zip(("scores", "adjacency", "features"), last))
 
         def step_e2e():
             return me.score_windows(model, f_pin, device=dev)[1]
@@ -703,11 +735,13 @@ def run_small(args, rank, local, world, dev, dp):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step_dev()
+        last = step_dev()
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
     launches = ops.LAUNCHES[0] - n0
+    if args.dump_outputs and rank == 0:        # before the end-to-end steps below (mb_train: they train the model further)
+        dump_outputs(args.dump_outputs, named_outputs(last))
     for _ in range(2):
         step_e2e()
     barrier()
@@ -801,7 +835,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from Python instead of replaying one CUDA graph")
     ap.add_argument("--profile-calls", default="", help="write a per-ABI-call timing table of the replayed step graph to this file")
     ap.add_argument("--watchdog", type=int, default=420, help="seconds after which a stuck run dumps its stack and exits non-zero")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     import faulthandler
     faulthandler.dump_traceback_later(args.watchdog, exit=True)     # a hang must never eat the GPU budget
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup

@@ -8,6 +8,7 @@ from __future__ import annotations
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 import sys
 
@@ -19,6 +20,8 @@ LIB_PATH = os.path.join(PKG_DIR, "libcvad_b200.so")
 # development only: A/B a library built from another branch (tools/build_variant.sh) without touching the in-tree one
 LOAD_PATH = os.environ.get("CVAD_B200_LIB", LIB_PATH)
 
+# a login shell often lacks the toolkit's bin directory on PATH
+NVCC = shutil.which("nvcc") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc")
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "-I", os.path.join(ROOT, "include"), "-I", CSRC]
 
@@ -60,7 +63,7 @@ def build(force: bool = False, verbose: bool = True) -> str:
                 and os.path.getmtime(obj) > os.path.getmtime(HEADER)
                 and all(os.path.getmtime(obj) > os.path.getmtime(os.path.join(CSRC, f)) for f in os.listdir(CSRC) if f.endswith(".cuh"))):
             continue
-        cmd = ["nvcc"] + NVCC_FLAGS + ["-c", src, "-o", obj]
+        cmd = [NVCC] + NVCC_FLAGS + ["-c", src, "-o", obj]
         if verbose:
             print("[cvad_b200.build]", " ".join(cmd), flush=True)
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))
@@ -68,7 +71,7 @@ def build(force: bool = False, verbose: bool = True) -> str:
         out, _ = p.communicate()
         if p.returncode != 0:
             raise RuntimeError(f"nvcc failed for {src}:\n{out}")
-    cmd = ["nvcc", "-shared", "--cudart", "shared", "-o", LIB_PATH] + objs
+    cmd = [NVCC, "-shared", "--cudart", "shared", "-o", LIB_PATH] + objs
     r = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     if r.returncode != 0:
         raise RuntimeError(f"link failed:\n{r.stdout}")

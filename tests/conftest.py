@@ -15,11 +15,8 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def gold():
-    import torch
-
-    def load(name):
-        return torch.load(os.path.join(ROOT, "tests", "golden", name), map_location="cpu", weights_only=False)
-    return load
+    import synth
+    return synth.golden
 
 
 @pytest.fixture(scope="session")

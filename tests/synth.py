@@ -7,8 +7,39 @@ rebuild bit-identical tensors without shipping them.  SURVEY.md section 8(d) def
 from __future__ import annotations
 
 import math
+import os
 
 import torch
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# A checkpoint with AdamW state is stored in three files so that none exceeds 1 MB: ``<name>`` without the two moment tensors of each
+# optimizer state entry, and ``<stem>.exp_avg.pt`` / ``<stem>.exp_avg_sq.pt`` holding them as lists in state order.
+MOMENTS = ("exp_avg", "exp_avg_sq")
+
+
+def _moment_paths(name):
+    stem = name.rsplit(".", 1)[0]
+    return {m: os.path.join(GOLDEN, f"{stem}.{m}.pt") for m in MOMENTS}
+
+
+def golden(name):
+    """The committed fixture ``tests/golden/<name>``; a split checkpoint comes back whole."""
+    d = torch.load(os.path.join(GOLDEN, name), map_location="cpu", weights_only=False)
+    parts = _moment_paths(name)
+    if all(os.path.exists(p) for p in parts.values()):
+        moments = {m: torch.load(p, map_location="cpu", weights_only=True) for m, p in parts.items()}
+        for i, st in enumerate(d["optimizer_state_dict"]["state"].values()):
+            st.update((m, moments[m][i]) for m in MOMENTS)
+    return d
+
+
+def save_golden_checkpoint(ck, name):
+    """Store a checkpoint with AdamW state as ``golden(name)`` reads it back."""
+    opt = ck["optimizer_state_dict"]
+    state = {i: {k: v for k, v in st.items() if k not in MOMENTS} for i, st in opt["state"].items()}
+    torch.save({**ck, "optimizer_state_dict": {**opt, "state": state}}, os.path.join(GOLDEN, name))
+    for m, p in _moment_paths(name).items():
+        torch.save([st[m] for st in opt["state"].values()], p)
 
 
 def gen(seed: int) -> torch.Generator:

@@ -25,8 +25,8 @@ def test_reference_arm_prints_the_contract_line():
     # the M-A reference step is seconds of CPU work: at most 3 timed steps + 1 warm-up are run, and the line reports THAT, not the request
     assert d["steps"] == 3 and d["warmup"] == 1 and d["requested"] == {"steps": 7, "warmup": 2}
     cb = d["cpu_baseline"]
-    have_ref = os.path.exists(os.path.join(ROOT, "oracle", "_ref", "causal_anomaly_detection.py")) or os.path.exists("/root/reference")
-    assert cb["kind"] == ("reference" if have_ref else "port") and cb["cores"] >= 1 and cb["sample"] and cb["value"] == d["value"]
+    from oracle.ref_harness import reference_dir
+    assert cb["kind"] == ("reference" if reference_dir() is not None else "port") and cb["cores"] >= 1 and cb["sample"] and cb["value"] == d["value"]
     e = d["e2e"]
     assert e["value"] == d["value"] and e["unit"] == d["unit"] and e["h2d_bytes_per_step"] == 0 and e["d2h_bytes_per_step"] == 0
 

@@ -85,7 +85,17 @@ def test_mb_trajectory_with_oracle_optimizer(gold):
     assert step == g["final_opt_step"]
 
 
-def test_mc_matches_reference(gold):
+@pytest.fixture
+def golden_threads():
+    """The CPU thread count tools/make_golden.py computed the fixtures with.  The conv3d backward's reduction order follows the thread
+    count, and so does the round-off that forms a BatchNorm-fed bias's analytically zero gradient (M-C features.0.bias)."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(n)
+
+
+def test_mc_matches_reference(gold, golden_threads):
     g = gold("mc.pt")
     synth_state = synth.synth_fill(g["init_state"], seed=g["state_seed"])
     for k in synth_state:
@@ -300,11 +310,14 @@ def test_ma_trajectory_oracle_vs_reference_train_model(gold):
         eps, keep = ma_noise({"B": B, "T": T, "xseed": xs})
         losses.append(o_train.ma_train_step(P, opt, x, y, eps, keep)[0])
     assert abs(sum(losses) / 3 - g["mean_loss"]) < 1e-5 * g["mean_loss"]
+
+    def sample(t):              # the fixture keeps at most sample_cap elements of each tensor's strided sample
+        return synth.strided_sample(synth.strided_sample(t), g["sample_cap"])
     for k, ref in g["final_sample"].items():
         if "running" in k or synth.is_bn_fed_conv_bias(k):
             continue
-        moved = float((ref - synth.strided_sample(P0[k])).double().norm())
-        d = float((synth.strided_sample(P[k]) - ref).double().norm())
+        moved = float((ref - sample(P0[k])).double().norm())
+        d = float((sample(P[k]) - ref).double().norm())
         assert d <= 0.25 * moved + 1e-12, (k, d, moved)
 
 

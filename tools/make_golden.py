@@ -31,6 +31,8 @@ from oracle import md as o_md  # noqa: E402
 from oracle import optim as o_opt  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
+# elements kept of each final parameter's strided sample in ma_traj.pt (keeps the fixture under 1 MB)
+TRAJ_SAMPLE_CAP = 3072
 torch.set_num_threads(8)
 
 
@@ -47,8 +49,8 @@ def close(a, b, tol, what, floor=1e-3):
 def make_mb():
     print("== M-B (avenue_training_script2.py) ==")
     s2 = import_ref("avenue_training_script2")
-    ck = torch.load("/root/reference/best_improved_model.pth", map_location="cpu", weights_only=False)
-    torch.save(ck, os.path.join(GOLD, "best_improved_model.pth"))
+    ck = torch.load(os.path.join(os.path.dirname(s2.__file__), "best_improved_model.pth"), map_location="cpu", weights_only=False)
+    synth.save_golden_checkpoint(ck, "best_improved_model.pth")
     P = ck["model_state_dict"]
     out = {"eval": [], "known_answers": {
         "scores_T8": [0.13723799586296082, 0.13770483434200287, 0.13747946918010712, 0.13792464137077332],
@@ -609,7 +611,9 @@ def make_ma_traj():
                      "oracle_losses": o_losses, "n_tracks": [n.clone() for n in ntrs],
                      "final_summary": {k: synth.summarize(v) for k, v in final.items()},
                      "moved_l2": {k: float((v - P0[k]).double().norm()) for k, v in final.items() if v.is_floating_point()},
-                     "final_sample": {k: synth.strided_sample(v) for k, v in final.items() if v.is_floating_point()}}
+                     "sample_cap": TRAJ_SAMPLE_CAP,
+                     "final_sample": {k: synth.strided_sample(synth.strided_sample(v), TRAJ_SAMPLE_CAP)
+                                      for k, v in final.items() if v.is_floating_point()}}
     torch.save(out, os.path.join(GOLD, "ma_traj.pt"))
     print("   wrote ma_traj.pt", os.path.getsize(os.path.join(GOLD, "ma_traj.pt")) // 1024, "KiB")
 
