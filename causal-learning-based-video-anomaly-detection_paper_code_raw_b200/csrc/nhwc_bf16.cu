@@ -572,13 +572,13 @@ __global__ void avgpool_pad_bwd_frame_kernel(const float* __restrict__ dout, int
   }
 }
 
-// development knobs for the apply kernels: rows per CTA iteration (1, 2 or 4) and CTAs per SM
+// development knobs for the apply kernels: rows per CTA iteration (2 or 4; anything else runs 2) and CTAs per SM
 inline int bn_rows_per_iter() {
   static int v = -1;
   if (v < 0) {
     const char* e = getenv("CVAD_BN_ROWS");
     v = e ? atoi(e) : 2;
-    if (v != 1 && v != 2 && v != 4) v = 2;
+    if (v != 2 && v != 4) v = 2;
   }
   return v;
 }
@@ -657,7 +657,7 @@ int launch_apply(const __nv_bfloat16* r, __nv_bfloat16* a, const PadGeo& g, int 
   BnFin fin = fin_in;
   fin.reverse = bn_apply_reverse();
   const int rows = phase_out ? 2 * N * g.Hq : N * (H + 2);
-  const int R = bn_rows_per_iter() == 4 ? 4 : 2;
+  const int R = bn_rows_per_iter();
   const int want = (rows + R - 1) / R;
 #define CVAD_APPLY(PH, RR, FI) \
   pad_bn_apply_relu_kernel<PH, RR, FI><<<apply_grid(pad_bn_apply_relu_kernel<PH, RR, FI>, want), 256, 0, st>>>(r, a, g, mean, invstd, gamma, beta, fin)
@@ -687,7 +687,7 @@ int launch_bwd_apply(const __nv_bfloat16* r, const __nv_bfloat16* d, __nv_bfloat
                      const float* mean, const float* invstd, const float* gamma, const float* beta, double* ws, int training, bool fold,
                      float* dgamma, float* dbeta, cudaStream_t st) {
   const int rows = N * (H + 2);
-  const int R = bn_rows_per_iter() == 4 ? 4 : 2;
+  const int R = bn_rows_per_iter();
   const int want = (rows + R - 1) / R;
   const double count = (double)N * H * W;
   static int occ3 = -1;

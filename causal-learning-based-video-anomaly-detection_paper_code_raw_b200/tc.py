@@ -45,7 +45,7 @@ FUSED_STATS = os.environ.get("CVAD_FUSED_BN_STATS", "1") != "0"     # BatchNorm 
 # the next layer down instead of in front of it (a parallel branch of the captured step graph)
 WGRAD_OVERLAP = os.environ.get("CVAD_WGRAD_OVERLAP", "0") == "1"
 # BatchNorm-backward reductions of layer i-1 taken in the data-gradient epilogue of layer i (one pass over raw / dact instead of two).
-# Correct (tests/test_flat_gpu.py) but OFF: measured on a B200 it lengthens the data-gradients (8 epilogue warps become the bottleneck:
+# Correct (the epilogue's sums: tests/test_flat_gpu.py; the apply entry that consumes them: tests/test_bn_flat_gpu.py) but OFF: measured on a B200 it lengthens the data-gradients (8 epilogue warps become the bottleneck:
 # 0.62 -> 1.20 ms, 1.0 ms with the raw rows prefetched before the accumulator wait) by more than the reduce pass it removes (0.27 ms).
 FUSED_BN_BWD = os.environ.get("CVAD_FUSED_BN_BWD", "0") == "1"
 
