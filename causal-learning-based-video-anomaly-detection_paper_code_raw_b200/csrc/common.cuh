@@ -152,3 +152,45 @@ static inline cudaError_t cvad_ensure_dyn_smem(Kernel kernel, size_t smem, size_
   if (e == cudaSuccess) configured[dev] = smem;
   return e;
 }
+
+// ---- BatchNorm statistics.  Every BatchNorm reduction leaves per-channel fp64 sums in a 2*C workspace: ws[c] = sum y, ws[C + c] = sum y^2
+// in the forward pass, ws[c] = sum g, ws[C + c] = sum g*xhat in the backward pass.  The helpers below are the one place that turns those
+// sums into batch statistics and parameter gradients; whoever calls them re-zeroes ws afterwards.
+
+// Batch mean and biased variance of channel c over `count` values.  shift (nullptr = none): the sums were taken over y - shift[c] (the
+// stems sum their raw accumulator, before the conv bias), which moves the mean and leaves the variance.
+struct BnBatchStat { double mean, var; };
+__device__ __forceinline__ BnBatchStat bn_batch_stat(const double* ws, int C, int c, double count, const float* shift) {
+  const double m = ws[c] / count;
+  double var = ws[C + c] / count - m * m;
+  if (var < 0.0) var = 0.0;
+  return {shift ? m + (double)shift[c] : m, var};
+}
+__device__ __forceinline__ float bn_invstd(const BnBatchStat& s, float eps) { return (float)(1.0 / sqrt(s.var + (double)eps)); }
+
+// Forward finalize of channel c: mean / invstd for the apply and backward passes, the momentum update of the running statistics (with the
+// unbiased variance, as torch) when running_mean is non-null, and num_batches_tracked += 1 by channel 0 when nbt is non-null.
+__device__ __forceinline__ void bn_finalize_channel(const double* ws, int C, int c, double count, const float* shift, float eps, float momentum,
+                                                    float* mean, float* invstd, float* running_mean, float* running_var, long long* nbt) {
+  const BnBatchStat s = bn_batch_stat(ws, C, c, count, shift);
+  mean[c] = (float)s.mean;
+  invstd[c] = bn_invstd(s, eps);
+  if (running_mean) {
+    const double unbiased = count > 1.0 ? s.var * count / (count - 1.0) : s.var;
+    running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)s.mean;
+    running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
+  }
+  if (c == 0 && nbt) *nbt += 1;
+}
+
+// Backward parameter update of channel c: dgamma += sum g*xhat, dbeta += sum g, each only when non-null.
+__device__ __forceinline__ void bn_params_channel(const double* ws, int C, int c, float* dgamma, float* dbeta) {
+  if (dgamma) dgamma[c] += (float)ws[C + c];
+  if (dbeta) dbeta[c] += (float)ws[c];
+}
+
+// One launch of the finalize / parameter-update kernel over channels [0, C), which then re-zeroes ws[0, 2C) (norm_pool_f32.cu; library
+// internal, not exported).  Return 0 or the launch error.
+int bn_finalize_launch(double* ws, int C, double count, const float* shift, float eps, float momentum, float* mean, float* invstd,
+                       float* running_mean, float* running_var, long long* nbt, cudaStream_t st);
+int bn_params_launch(double* ws, int C, float* dgamma, float* dbeta, cudaStream_t st);

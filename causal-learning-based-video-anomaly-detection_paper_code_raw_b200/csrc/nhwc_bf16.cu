@@ -26,37 +26,6 @@ __device__ __forceinline__ uint4 pack8(const float (&f)[8]) {
   return v;
 }
 
-__global__ void bn_finalize_nhwc_kernel(double* __restrict__ ws, int C, double count, float eps, float momentum, float* __restrict__ mean,
-                                        float* __restrict__ invstd, float* __restrict__ running_mean, float* __restrict__ running_var,
-                                        long long* __restrict__ nbt) {
-  int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c < C) {
-    double m = ws[c] / count;
-    double var = ws[C + c] / count - m * m;
-    if (var < 0.0) var = 0.0;
-    mean[c] = (float)m;
-    invstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-    if (running_mean) {
-      double unbiased = count > 1.0 ? var * count / (count - 1.0) : var;
-      running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)m;
-      running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
-    }
-    ws[c] = 0.0;
-    ws[C + c] = 0.0;
-  }
-  if (c == 0 && nbt) *nbt += 1;
-}
-
-__global__ void bn_bwd_params_nhwc_kernel(double* __restrict__ ws, int C, float* __restrict__ dgamma, float* __restrict__ dbeta) {
-  int c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c < C) {
-    if (dgamma) dgamma[c] += (float)ws[C + c];
-    if (dbeta) dbeta[c] += (float)ws[c];
-    ws[c] = 0.0;
-    ws[C + c] = 0.0;
-  }
-}
-
 // ------------------------------------------------------------------------------------------------ adaptive average pool
 // adaptive-pool bin bounds; 32-bit arithmetic (frame dimensions are far below 2^15: the 64-bit divisions these used to be cost the
 // per-frame backward kernel more than its memory traffic)
@@ -97,9 +66,9 @@ __device__ __forceinline__ long long phase_row(const PadGeo& g, int n, int hp, i
 // (368..448 vectors) is one pass with all loads issued before the first use.  PHASE=1 handles the two column-phase planes
 // (a,0) and (a,1) of one plane row in the same block, so the raw row both of them sample is fetched from HBM once.
 // FIN: the batch statistics are still the raw fp64 sums in fin.ws (left there by the convolution's epilogue): every thread finalises its own
-// eight channels (the arithmetic of bn_finalize_nhwc_kernel, so the result is bit-identical), block 0 also publishes mean / invstd for
-// the backward and updates the running statistics, and the last block past this prologue re-zeroes the sums -- one launch instead of
-// two on the critical path of every layer.
+// eight channels (common.cuh's BatchNorm helpers, as the separate finalize kernel, so the result is bit-identical), block 0 also publishes
+// mean / invstd for the backward and updates the running statistics, and the last block past this prologue re-zeroes the sums -- one
+// launch instead of two on the critical path of every layer.
 struct BnFin {
   int reverse;            // walk the rows back to front (L2 reuse, see the kernel)
   double* ws;
@@ -134,11 +103,9 @@ __global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloa
     const int c = cg * 8 + i;
     float mu, is;
     if (FIN) {
-      const double m = fin.ws[c] / fin.count;
-      double var = fin.ws[g.C + c] / fin.count - m * m;
-      if (var < 0.0) var = 0.0;
-      mu = (float)m;
-      is = (float)(1.0 / sqrt(var + (double)fin.eps));
+      const BnBatchStat s = bn_batch_stat(fin.ws, g.C, c, fin.count, nullptr);
+      mu = (float)s.mean;
+      is = bn_invstd(s, fin.eps);
     } else {
       mu = mean[c];
       is = invstd[c];
@@ -148,19 +115,9 @@ __global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloa
   }
   if (FIN) {
     if (blockIdx.x == 0)
-      for (int c = threadIdx.x; c < g.C; c += blockDim.x) {
-        const double m = fin.ws[c] / fin.count;
-        double var = fin.ws[g.C + c] / fin.count - m * m;
-        if (var < 0.0) var = 0.0;
-        fin.mean_out[c] = (float)m;
-        fin.invstd_out[c] = (float)(1.0 / sqrt(var + (double)fin.eps));
-        if (fin.running_mean) {
-          const double unbiased = fin.count > 1.0 ? var * fin.count / (fin.count - 1.0) : var;
-          fin.running_mean[c] = (1.f - fin.momentum) * fin.running_mean[c] + fin.momentum * (float)m;
-          fin.running_var[c] = (1.f - fin.momentum) * fin.running_var[c] + fin.momentum * (float)unbiased;
-        }
-        if (c == 0 && fin.nbt) *fin.nbt += 1;
-      }
+      for (int c = threadIdx.x; c < g.C; c += blockDim.x)
+        bn_finalize_channel(fin.ws, g.C, c, fin.count, nullptr, fin.eps, fin.momentum, fin.mean_out, fin.invstd_out, fin.running_mean,
+                            fin.running_var, fin.nbt);
     bn_fold_release(fin.ws, g.C);
   }
   const int Hp = g.H + 2, Wp = g.W + 2;
@@ -343,7 +300,7 @@ __global__ void __launch_bounds__(256, 3) pad_reduce_kernel(const __nv_bfloat16*
 }
 
 // ReLU + BatchNorm backward: draw (plain padded, ZERO border) from raw and dact (plain or phase planes)
-// FOLD: block 0 also adds the two sums into dgamma / dbeta and the last block past the prologue re-zeroes ws (bn_bwd_params_nhwc_kernel's
+// FOLD: block 0 also adds the two sums into dgamma / dbeta and the last block past the prologue re-zeroes ws (the parameter-update kernel's
 // work): no third launch.
 // OCC: resident CTAs per SM the register allocation is held to (98 registers = 2 CTAs when left alone; 3 CTAs cost ~20 spilled registers)
 template <int PHASE, int R, bool FOLD, int OCC>
@@ -370,10 +327,7 @@ __global__ void __launch_bounds__(256, OCC) pad_bn_relu_bwd_apply_kernel(const _
   }
   if (FOLD) {
     if (blockIdx.x == 0)
-      for (int c = threadIdx.x; c < g.C; c += blockDim.x) {
-        if (dgamma) dgamma[c] += (float)ws[g.C + c];
-        if (dbeta) dbeta[c] += (float)ws[c];
-      }
+      for (int c = threadIdx.x; c < g.C; c += blockDim.x) bn_params_channel(ws, g.C, c, dgamma, dbeta);
     bn_fold_release(ws, g.C);
   }
   const int Hp = g.H + 2, Wp = g.W + 2;
@@ -717,19 +671,14 @@ CVAD_API int cvad_pad_bn_stats_bf16(const void* raw, int N, int H, int W, int C,
   cudaStream_t st = (cudaStream_t)stream;
   launch_reduce<false>((const __nv_bfloat16*)raw, nullptr, g, N, H, 0, nullptr, nullptr, nullptr, nullptr, ws, st);
   CVAD_LAUNCH_CHECK();
-  bn_finalize_nhwc_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, (double)N * H * W, eps, momentum, mean, invstd, running_mean, running_var,
-                                                           num_batches_tracked);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  return bn_finalize_launch(ws, C, (double)N * H * W, nullptr, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked, st);
 }
 
 CVAD_API int cvad_bn_finalize_f64(double* ws, int C, double count, float eps, float momentum, float* mean, float* invstd, float* running_mean,
                                   float* running_var, long long* num_batches_tracked, void* stream) {
   if (C <= 0 || count <= 0) return (int)cudaErrorInvalidValue;
-  bn_finalize_nhwc_kernel<<<(C + 127) / 128, 128, 0, (cudaStream_t)stream>>>(ws, C, count, eps, momentum, mean, invstd, running_mean, running_var,
-                                                                            num_batches_tracked);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  return bn_finalize_launch(ws, C, count, nullptr, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked,
+                            (cudaStream_t)stream);
 }
 
 CVAD_API int cvad_pad_bn_apply_relu_bf16(const void* raw, void* act, int N, int H, int W, int C, int phase_out, const float* mean,
@@ -750,9 +699,8 @@ CVAD_API int cvad_pad_bn_finalize_apply_relu_bf16(const void* raw, void* act, in
   cudaStream_t st = (cudaStream_t)stream;
   const double count = (double)N * H * W;
   if (!bn_fold()) {
-    bn_finalize_nhwc_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, count, eps, momentum, mean, invstd, running_mean, running_var,
-                                                             num_batches_tracked);
-    CVAD_LAUNCH_CHECK();
+    const int e = bn_finalize_launch(ws, C, count, nullptr, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked, st);
+    if (e) return e;
     BnFin none;
     memset(&none, 0, sizeof(none));
     return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, g, N, H, phase_out, mean, invstd, gamma, beta, false, none, st);
@@ -775,9 +723,7 @@ CVAD_API int cvad_pad_bn_relu_bwd_bf16(const void* raw, const void* dact, void* 
     int e = launch_bwd_apply(r, d, (__nv_bfloat16*)draw, g, N, H, W, phase_in, mean, invstd, gamma, beta, ws, training, fold, dgamma, dbeta, st);
     if (e || fold) return e;
   }
-  bn_bwd_params_nhwc_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, dgamma, dbeta);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  return bn_params_launch(ws, C, dgamma, dbeta, st);
 }
 
 // The same with the two per-channel sums already in ws (taken by the data-gradient epilogue of the layer above,
@@ -792,9 +738,7 @@ CVAD_API int cvad_pad_bn_relu_bwd_apply_bf16(const void* raw, const void* dact, 
   const bool fold = bn_fold() != 0;
   int e = launch_bwd_apply(r, d, (__nv_bfloat16*)draw, g, N, H, W, phase_in, mean, invstd, gamma, beta, ws, training, fold, dgamma, dbeta, st);
   if (e || fold) return e;
-  bn_bwd_params_nhwc_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, dgamma, dbeta);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  return bn_params_launch(ws, C, dgamma, dbeta, st);
 }
 
 CVAD_API int cvad_pad_avgpool_bf16_fwd(const void* x, int N, int H, int W, int C, int OH, int OW, float* out, void* stream) {

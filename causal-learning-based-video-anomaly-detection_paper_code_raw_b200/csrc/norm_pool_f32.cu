@@ -34,26 +34,16 @@ __global__ void bn_stats_kernel(const float* __restrict__ x, int N, int C, long 
   }
 }
 
-// One thread per channel: batch mean / biased var -> mean, invstd; running-stat update (momentum, unbiased var); ws re-zeroed.
-__global__ void bn_finalize_kernel(double* __restrict__ ws, int C, double count, float eps, float momentum, float* __restrict__ mean,
-                                   float* __restrict__ invstd, float* __restrict__ running_mean, float* __restrict__ running_var,
-                                   long long* __restrict__ num_batches_tracked) {
-  int c = blockIdx.x * blockDim.x + threadIdx.x;
+// One thread per channel: the forward finalize of every BatchNorm of the library (fp32, bf16 backbone, stems); ws re-zeroed.
+__global__ void bn_finalize_kernel(double* __restrict__ ws, int C, double count, const float* __restrict__ shift, float eps, float momentum,
+                                   float* __restrict__ mean, float* __restrict__ invstd, float* __restrict__ running_mean,
+                                   float* __restrict__ running_var, long long* __restrict__ num_batches_tracked) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c < C) {
-    double m = ws[c] / count;
-    double var = ws[C + c] / count - m * m;
-    if (var < 0.0) var = 0.0;
-    mean[c] = (float)m;
-    invstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-    if (running_mean) {
-      double unbiased = count > 1.0 ? var * count / (count - 1.0) : var;
-      running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)m;
-      running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
-    }
+    bn_finalize_channel(ws, C, c, count, shift, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked);
     ws[c] = 0.0;
     ws[C + c] = 0.0;
   }
-  if (c == 0 && num_batches_tracked) *num_batches_tracked += 1;
 }
 
 __global__ void bn_eval_prepare_kernel(int C, float eps, const float* __restrict__ running_mean, const float* __restrict__ running_var,
@@ -156,11 +146,11 @@ __global__ void bn_bwd_apply_kernel(const float* __restrict__ dy, const float* _
   }
 }
 
+// the backward's parameter-gradient update, for the fp32 and the bf16 backbone BatchNorms alike; ws re-zeroed
 __global__ void bn_bwd_params_kernel(double* __restrict__ ws, int C, float* __restrict__ dgamma, float* __restrict__ dbeta) {
-  int c = blockIdx.x * blockDim.x + threadIdx.x;
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c < C) {
-    if (dgamma) dgamma[c] += (float)ws[C + c];
-    if (dbeta) dbeta[c] += (float)ws[c];
+    bn_params_channel(ws, C, c, dgamma, dbeta);
     ws[c] = 0.0;
     ws[C + c] = 0.0;
   }
@@ -356,6 +346,19 @@ inline int ew_blocks(long long n) {
 
 }  // namespace
 
+int bn_finalize_launch(double* ws, int C, double count, const float* shift, float eps, float momentum, float* mean, float* invstd,
+                       float* running_mean, float* running_var, long long* nbt, cudaStream_t st) {
+  bn_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, count, shift, eps, momentum, mean, invstd, running_mean, running_var, nbt);
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
+int bn_params_launch(double* ws, int C, float* dgamma, float* dbeta, cudaStream_t st) {
+  bn_bwd_params_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, dgamma, dbeta);
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
 CVAD_API int cvad_bn_train_stats_f32(const float* x, int N, int C, long long S, double* ws, float eps, float momentum, float* mean,
                                      float* invstd, float* running_mean, float* running_var, long long* num_batches_tracked,
                                      void* stream) {
@@ -367,10 +370,7 @@ CVAD_API int cvad_bn_train_stats_f32(const float* x, int N, int C, long long S, 
   if (chunks < 1) chunks = 1;
   bn_stats_kernel<<<dim3(chunks, C), 256, 0, st>>>(x, N, C, S, ws);
   CVAD_LAUNCH_CHECK();
-  bn_finalize_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, (double)total, eps, momentum, mean, invstd, running_mean, running_var,
-                                                      num_batches_tracked);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  return bn_finalize_launch(ws, C, (double)total, nullptr, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked, st);
 }
 
 CVAD_API int cvad_bn_eval_prepare_f32(int C, float eps, const float* running_mean, const float* running_var, float* mean, float* invstd,
@@ -411,9 +411,7 @@ CVAD_API int cvad_bn_bwd_f32(const float* dy, const float* x, float* dx, int N, 
                                                                                                act, ws, (double)total, training);
     CVAD_LAUNCH_CHECK();
   }
-  bn_bwd_params_kernel<<<(C + 127) / 128, 128, 0, st>>>(ws, C, dgamma, dbeta);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  return bn_params_launch(ws, C, dgamma, dbeta, st);
 }
 
 // Eval-mode BatchNorm folded into the convolution in front of it (SURVEY K5): w'[co][...] = w[co][...] * s, b' = (b - running_mean) * s + beta

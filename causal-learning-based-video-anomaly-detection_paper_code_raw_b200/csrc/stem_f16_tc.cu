@@ -495,29 +495,6 @@ __global__ void __launch_bounds__(128 + 128 * S8_EG, 1) stem8_pool_kernel(const 
   if (warp == 2) tmem_dealloc<512>(tmem_base);
 }
 
-// ws holds sum / sum of squares of the RAW accumulator; y = acc + bias: mean_y = mean_acc + b, var_y = var_acc
-__global__ void stem8_finalize_kernel(double* __restrict__ ws, const float* __restrict__ bias, double count, float eps, float momentum,
-                                      float* __restrict__ mean, float* __restrict__ invstd, float* __restrict__ running_mean,
-                                      float* __restrict__ running_var, long long* __restrict__ nbt) {
-  const int c = threadIdx.x;
-  if (c < S8_C) {
-    const double ma = ws[c] / count;
-    double var = ws[S8_C + c] / count - ma * ma;
-    if (var < 0.0) var = 0.0;
-    const double m = ma + (double)bias[c];
-    mean[c] = (float)m;
-    invstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-    if (running_mean) {
-      const double unbiased = count > 1.0 ? var * count / (count - 1.0) : var;
-      running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)m;
-      running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
-    }
-    ws[c] = 0.0;
-    ws[S8_C + c] = 0.0;
-  }
-  if (c == 0 && nbt) *nbt += 1;
-}
-
 int geo8(Geo8& g, int N, int H, int W) {
   if (N <= 0 || H <= 0 || W <= 0 || (W & 3)) return 1;
   g.N = N; g.H = H; g.W = W;
@@ -615,10 +592,9 @@ CVAD_API int cvad_stem8_f16_stats(const void* x8, const float* w, const float* b
   if (grid > g.n_tiles) grid = g.n_tiles;
   stem8_stats_kernel<<<(unsigned)grid, 384, smem, st>>>(mx, w, g, ws);
   CVAD_LAUNCH_CHECK();
-  stem8_finalize_kernel<<<1, 32, 0, st>>>(ws, bias, (double)N * g.Ho * g.Wo, eps, momentum, mean, invstd, running_mean, running_var,
-                                          num_batches_tracked);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  // ws holds the sums of the RAW accumulator; y = acc + bias: the bias moves the mean, not the variance
+  return bn_finalize_launch(ws, S8_C, (double)N * g.Ho * g.Wo, bias, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked,
+                            st);
 }
 
 CVAD_API int cvad_stem8_f16_bn_relu_maxpool(const void* x8, const float* w, const float* bias, int N, int H, int W, const float* mean,

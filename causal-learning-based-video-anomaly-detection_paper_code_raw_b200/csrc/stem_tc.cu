@@ -531,29 +531,6 @@ __global__ void __launch_bounds__(384, 1) stem_pool_kernel(const __grid_constant
   if (warp == 2) tmem_dealloc<512>(tmem_base);
 }
 
-// ws holds sum / sum of squares of the RAW accumulator; y = acc + bias: mean_y = mean_acc + b, var_y = var_acc
-__global__ void stem_finalize_kernel(double* __restrict__ ws, const float* __restrict__ bias, double count, float eps, float momentum,
-                                     float* __restrict__ mean, float* __restrict__ invstd, float* __restrict__ running_mean,
-                                     float* __restrict__ running_var, long long* __restrict__ nbt) {
-  const int c = threadIdx.x;
-  if (c < ST_C) {
-    const double ma = ws[c] / count;
-    double var = ws[ST_C + c] / count - ma * ma;
-    if (var < 0.0) var = 0.0;
-    const double m = ma + (double)bias[c];
-    mean[c] = (float)m;
-    invstd[c] = (float)(1.0 / sqrt(var + (double)eps));
-    if (running_mean) {
-      const double unbiased = count > 1.0 ? var * count / (count - 1.0) : var;
-      running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * (float)m;
-      running_var[c] = (1.f - momentum) * running_var[c] + momentum * (float)unbiased;
-    }
-    ws[c] = 0.0;
-    ws[ST_C + c] = 0.0;
-  }
-  if (c == 0 && nbt) *nbt += 1;
-}
-
 // MaxPool2d(3,2,1) over relu'd bf16 NHWC (N,H,W,C) -> padded-flat (N,PH+2,PW+2,C) with zero border; 8 channels per thread
 __global__ void maxpool3x3s2_pad_kernel(const __nv_bfloat16* __restrict__ y, int N, int H, int W, int C, int PH, int PW,
                                         __nv_bfloat16* __restrict__ out) {
@@ -724,10 +701,9 @@ CVAD_API int cvad_stem_tf32_stats(const float* x4, const float* w, const float* 
   if (stem_geo(g, N, H, W)) return (int)cudaErrorInvalidValue;
   int e = stem_launch(0, x4, w, bias, g, nullptr, nullptr, nullptr, nullptr, ws, nullptr, st);
   if (e) return e;
-  stem_finalize_kernel<<<1, 32, 0, st>>>(ws, bias, (double)N * g.Ho * g.Wo, eps, momentum, mean, invstd, running_mean, running_var,
-                                         num_batches_tracked);
-  CVAD_LAUNCH_CHECK();
-  return 0;
+  // ws holds the sums of the RAW accumulator; y = acc + bias: the bias moves the mean, not the variance
+  return bn_finalize_launch(ws, ST_C, (double)N * g.Ho * g.Wo, bias, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked,
+                            st);
 }
 
 CVAD_API int cvad_stem_tf32_bn_relu(const float* x4, const float* w, const float* bias, int N, int H, int W, const float* mean,

@@ -7,7 +7,7 @@ non-finite loss or gradient -- decided on the device instead of through per-para
 
 Differences in execution, not in results:
 * the frame encoder runs once over all B*T frames (time-major) instead of T Python iterations; its BatchNorms keep the
-  reference's per-time-step batch statistics and T sequential running-statistics updates (``ops.grouped_batchnorm_act``);
+  reference's per-time-step batch statistics and T sequential running-statistics updates (``ops.batchnorm_act``);
 * the decoder, which the reference runs T times on the SAME sequence feature (cad1:254-257), runs once; ``reconstructed``
   is that frame viewed T times, the loss kernel sums the T targets' gradients, and the decoder BatchNorms' running
   statistics receive their T-1 further (identical) updates in closed form.
@@ -36,6 +36,11 @@ def init_weights(m):
     elif isinstance(m, nn.BatchNorm2d):
         nn.init.constant_(m.weight, 1)
         nn.init.constant_(m.bias, 0)
+
+
+def _bn(h, bn, groups=1):
+    return ops.batchnorm_act(h, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.num_batches_tracked,
+                             ops.bn_workspace(h.device, bn.num_features), bn.training, ACT_LEAKY01, bn.eps, bn.momentum, groups)
 
 
 class VideoAutoEncoder(nn.Module):
@@ -101,7 +106,7 @@ class VideoAutoEncoder(nn.Module):
         for ci in (0, 3, 6, 9):
             conv, bn = e[ci], e[ci + 1]
             h = ops.conv_act(h, conv.weight, conv.bias, 2, 1, ACT_NONE)
-            h = ops.grouped_batchnorm_act(h, bn, ACT_LEAKY01, groups)
+            h = _bn(h, bn, groups)
         lat = ops.linear_act(h.reshape(T * B, -1), e[13].weight, e[13].bias, ACT_TANH)           # (T*B, 64)
         frame_features = lat.reshape(T, B, -1).transpose(0, 1)                                    # (B, T, 64) view
         lstm = self.temporal_encoder
@@ -117,7 +122,7 @@ class VideoAutoEncoder(nn.Module):
             h = ops.channel_bias_act(ops.conv_transpose2d(h, ct.weight, 2, 1), ct.bias, ACT_NONE)
             if bn.training and repeats > 1:
                 rm0, rv0 = bn.running_mean.clone(), bn.running_var.clone()
-            h = ops.grouped_batchnorm_act(h, bn, ACT_LEAKY01, 1)
+            h = _bn(h, bn)
             if bn.training and repeats > 1:
                 # the reference calls this BatchNorm `repeats` times on identical input: apply the remaining updates
                 with torch.no_grad():

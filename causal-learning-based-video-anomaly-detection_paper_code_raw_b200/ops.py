@@ -432,47 +432,57 @@ def chainable(layers, din) -> bool:
 
 # ------------------------------------------------------------------------------------------------ batch norm
 class _BatchNormAct(torch.autograd.Function):
+    """BatchNorm + activation applied to ``groups`` consecutive slices of the batch axis as separate calls, in order: what the
+    reference does when it runs the frame encoder once per time step (cad1:227-231): per-step batch statistics and ``groups``
+    sequential running-statistics updates.  groups = 1 is the ordinary op."""
+
     @staticmethod
-    def forward(ctx, x, gamma, beta, running_mean, running_var, nbt, ws, training, act, eps, momentum):
+    def forward(ctx, x, gamma, beta, running_mean, running_var, nbt, ws, training, act, eps, momentum, groups):
         _cuda(x, gamma, beta)
         x = _f32c(x)
-        N, C = x.shape[:2]
+        NT, C = x.shape[:2]
+        assert NT % groups == 0
+        N = NT // groups
         S = x[0, 0].numel()
-        mean = torch.empty(C, device=x.device, dtype=torch.float32)
+        mean = torch.empty((groups, C), device=x.device, dtype=torch.float32)
         invstd = torch.empty_like(mean)
-        if training:
-            _call("cvad_bn_train_stats_f32", _ptr(x), N, C, S, _ptr(ws), float(eps), float(momentum), _ptr(mean), _ptr(invstd),
-                  _ptr(running_mean), _ptr(running_var), _ptr(nbt), _st())
-        else:
-            _call("cvad_bn_eval_prepare_f32", C, float(eps), _ptr(running_mean), _ptr(running_var), _ptr(mean), _ptr(invstd), _st())
         y = torch.empty_like(x)
-        _call("cvad_bn_apply_f32", _ptr(x), _ptr(y), N, C, S, _ptr(mean), _ptr(invstd), _ptr(gamma), _ptr(beta), act, _st())
-        ctx.meta = (training, act)
+        for gi in range(groups):
+            xs, ys = x[gi * N:(gi + 1) * N], y[gi * N:(gi + 1) * N]
+            if training:
+                _call("cvad_bn_train_stats_f32", _ptr(xs), N, C, S, _ptr(ws), float(eps), float(momentum), _ptr(mean[gi]), _ptr(invstd[gi]),
+                      _ptr(running_mean), _ptr(running_var), _ptr(nbt), _st())
+            else:
+                _call("cvad_bn_eval_prepare_f32", C, float(eps), _ptr(running_mean), _ptr(running_var), _ptr(mean[gi]), _ptr(invstd[gi]), _st())
+            _call("cvad_bn_apply_f32", _ptr(xs), _ptr(ys), N, C, S, _ptr(mean[gi]), _ptr(invstd[gi]), _ptr(gamma), _ptr(beta), act, _st())
+        ctx.meta = (training, act, groups)
         ctx.gamma, ctx.beta, ctx.ws = gamma, beta, ws
         ctx.save_for_backward(x, mean, invstd)
-        ctx.mark_non_differentiable(*[t for t in () if t is not None])
         return y
 
     @staticmethod
     def backward(ctx, dy):
         x, mean, invstd = ctx.saved_tensors
-        training, act = ctx.meta
+        training, act, groups = ctx.meta
         gamma, beta, ws = ctx.gamma, ctx.beta, ctx.ws
         dy = _f32c(dy)
-        N, C = x.shape[:2]
+        NT, C = x.shape[:2]
+        N = NT // groups
         S = x[0, 0].numel()
         dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
         dg = grad_buffer(gamma) if _wants_grad(gamma) else None
         db = grad_buffer(beta) if _wants_grad(beta) else None
         if dx is None and dg is None and db is None:
-            return (None,) * 11
-        _call("cvad_bn_bwd_f32", _ptr(dy), _ptr(x), _ptr(dx), N, C, S, _ptr(mean), _ptr(invstd), _ptr(gamma), _ptr(beta), act,
-              int(training), _ptr(ws), _ptr(dg), _ptr(db), _st())
-        return (dx,) + (None,) * 10
+            return (None,) * 12
+        for gi in range(groups):
+            sl = slice(gi * N, (gi + 1) * N)
+            _call("cvad_bn_bwd_f32", _ptr(dy[sl]), _ptr(x[sl]), _ptr(dx[sl]) if dx is not None else None, N, C, S, _ptr(mean[gi]),
+                  _ptr(invstd[gi]), _ptr(gamma), _ptr(beta), act, int(training), _ptr(ws), _ptr(dg), _ptr(db), _st())
+        return (dx,) + (None,) * 11
 
 
-def batchnorm_act(x, gamma, beta, running_mean, running_var, nbt, ws, training, act=ACT_NONE, eps=1e-5, momentum=0.1):
-    return _BatchNormAct.apply(x, gamma, beta, running_mean, running_var, nbt, ws, training, act, eps, momentum)
+def batchnorm_act(x, gamma, beta, running_mean, running_var, nbt, ws, training, act=ACT_NONE, eps=1e-5, momentum=0.1, groups=1):
+    return _BatchNormAct.apply(x, gamma, beta, running_mean, running_var, nbt, ws, training, act, eps, momentum, groups)
 
 
 # ------------------------------------------------------------------------------------------------ pooling
@@ -806,59 +816,6 @@ class _ChannelBiasAct(torch.autograd.Function):
 
 def channel_bias_act(x, bias, act=ACT_NONE):
     return _ChannelBiasAct.apply(x, bias, act)
-
-
-class _GroupedBatchNormAct(torch.autograd.Function):
-    """BatchNorm + activation applied to ``groups`` consecutive slices of the batch axis as separate calls, in order: what the
-    reference does when it runs the frame encoder once per time step (cad1:227-231): per-step batch statistics and ``groups``
-    sequential running-statistics updates.  groups = 1 is the ordinary op."""
-
-    @staticmethod
-    def forward(ctx, x, gamma, beta, running_mean, running_var, nbt, ws, training, act, eps, momentum, groups):
-        _cuda(x, gamma, beta)
-        x = _f32c(x)
-        NT, C = x.shape[:2]
-        assert NT % groups == 0
-        N = NT // groups
-        S = x[0, 0].numel()
-        mean = torch.empty((groups, C), device=x.device, dtype=torch.float32)
-        invstd = torch.empty_like(mean)
-        y = torch.empty_like(x)
-        for gi in range(groups):
-            xs, ys = x[gi * N:(gi + 1) * N], y[gi * N:(gi + 1) * N]
-            if training:
-                _call("cvad_bn_train_stats_f32", _ptr(xs), N, C, S, _ptr(ws), float(eps), float(momentum), _ptr(mean[gi]), _ptr(invstd[gi]),
-                      _ptr(running_mean), _ptr(running_var), _ptr(nbt), _st())
-            else:
-                _call("cvad_bn_eval_prepare_f32", C, float(eps), _ptr(running_mean), _ptr(running_var), _ptr(mean[gi]), _ptr(invstd[gi]), _st())
-            _call("cvad_bn_apply_f32", _ptr(xs), _ptr(ys), N, C, S, _ptr(mean[gi]), _ptr(invstd[gi]), _ptr(gamma), _ptr(beta), act, _st())
-        ctx.meta = (training, act, groups)
-        ctx.gamma, ctx.beta, ctx.ws = gamma, beta, ws
-        ctx.save_for_backward(x, mean, invstd)
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        x, mean, invstd = ctx.saved_tensors
-        training, act, groups = ctx.meta
-        gamma, beta, ws = ctx.gamma, ctx.beta, ctx.ws
-        dy = _f32c(dy)
-        NT, C = x.shape[:2]
-        N = NT // groups
-        S = x[0, 0].numel()
-        dx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
-        dg = grad_buffer(gamma) if _wants_grad(gamma) else None
-        db = grad_buffer(beta) if _wants_grad(beta) else None
-        for gi in range(groups):
-            sl = slice(gi * N, (gi + 1) * N)
-            _call("cvad_bn_bwd_f32", _ptr(dy[sl]), _ptr(x[sl]), _ptr(dx[sl]) if dx is not None else None, N, C, S, _ptr(mean[gi]),
-                  _ptr(invstd[gi]), _ptr(gamma), _ptr(beta), act, int(training), _ptr(ws), _ptr(dg), _ptr(db), _st())
-        return (dx,) + (None,) * 11
-
-
-def grouped_batchnorm_act(x, bn, act, groups=1):
-    return _GroupedBatchNormAct.apply(x, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.num_batches_tracked,
-                                      bn_workspace(x.device, bn.num_features), bn.training, act, bn.eps, bn.momentum, groups)
 
 
 class _LstmLast(torch.autograd.Function):
