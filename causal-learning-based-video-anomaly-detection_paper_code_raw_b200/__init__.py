@@ -9,6 +9,7 @@ Public surface (mirrors the reference's Python seam, SURVEY.md 8b):
   ma.CausalAnomalyDetector / ma.train_model / ma.test_model                  causal_anomaly_detection.py
   ma0.CausalAnomalyDetector / ma0.train_model / ma0.test_model               video_anomaly_detection.py
   ma0.StreamingWindowScorer (sliding windows over a frame stream: each frame's backbone pass is computed once)
+  infer.GraphedStreamingScorer / infer.FrozenBackbone (the same windows, one CUDA graph replay per push; eval BatchNorm folded into the convolutions)
   md.VideoAutoEncoder / md.train_model / md.calculate_anomaly_scores         causal_anomaly_detection1.py
   me.CausalAnomalyDetector / me.predict_anomaly_for_clip / me.score_windows  avenue_training_script_bbox.py
   train.train_improved_minicausal_vad (s2:339-468 driver with real resume, async checkpoints, history JSON)
@@ -21,6 +22,6 @@ from . import _lib
 
 _lib.lib()   # fail loudly when the CUDA extension has not been built
 
-from . import arena, evaltail, frames, graphs, ma, ma0, ma_ops, mb, mc, md, me, noise, ops, parallel, tc, train  # noqa: E402,F401
+from . import arena, evaltail, frames, graphs, infer, ma, ma0, ma_ops, mb, mc, md, me, noise, ops, parallel, tc, train  # noqa: E402,F401
 
-__all__ = ["arena", "evaltail", "frames", "graphs", "ma", "ma0", "ma_ops", "mb", "mc", "md", "me", "noise", "ops", "parallel", "tc", "train"]
+__all__ = ["arena", "evaltail", "frames", "graphs", "infer", "ma", "ma0", "ma_ops", "mb", "mc", "md", "me", "noise", "ops", "parallel", "tc", "train"]

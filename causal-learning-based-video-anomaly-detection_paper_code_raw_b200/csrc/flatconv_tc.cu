@@ -81,11 +81,13 @@ struct FcParams {
   // fused BatchNorm-BACKWARD reductions (data-gradient only, n_blocks == 1): the rows this launch writes are the gradient dact w.r.t. the
   // output of relu(bn(raw)) of the layer below; with g = dact * (raw*ga + gb > 0) (ga = gamma*invstd, gb = beta - mean*ga) the epilogue adds
   // sum g and sum g*xhat over the interior pixels to st_out[0..N) / st_out[N..2N) -- the two per-channel sums of the BatchNorm backward,
-  // which otherwise cost a full read pass over raw and dact.  bw_planes: the rows are the four phase planes of a stride-2 input
+  // which otherwise cost a full read pass over raw and dact.  planes: the rows are the four phase planes of a stride-2 input
   // (geometry (st_h+2) x (st_w+2) per plane) and map to pixel (2(i-1)+a, 2(j-1)+b) of the bw_H x bw_W interior of raw.
+  // ReLU-output forward (EPI_RELU): the output interior is st_h x st_w; planes = 1 writes it as the four phase planes of the next
+  // stride-2 convolution, plane_out_stride rows apart, instead of padded-flat.
   const __nv_bfloat16* bw_raw;
   const float *bw_gamma, *bw_beta, *bw_mean, *bw_invstd;
-  int bw_H, bw_W, bw_planes;
+  int bw_H, bw_W, planes;
   FcUnit units[FC_MAX_UNITS];
 };
 
@@ -142,12 +144,18 @@ __device__ __forceinline__ void warp_colsum16_pair(const float (&a)[16], const f
   sum_b = vv + __shfl_xor_sync(0xffffffffu, vv, 1);
 }
 
-// BW: the instance that also takes the BatchNorm-backward reductions in its epilogue (FcParams::bw_raw).  A separate instantiation: the
-// epilogue of the plain kernels is timing-critical (8 warps against the MMA stream) and must not carry that code.
-template <int ROWB, int N, bool BW>
+// Epilogue kinds, each a separate instantiation: the epilogue of the plain kernels is timing-critical (8 warps against the MMA stream) and
+// must not carry optional code.
+//   EPI_PLAIN  out = conv + bias (junk on the border rows), optionally with the BatchNorm batch statistics (FcParams::st_out)
+//   EPI_BW     data-gradient that also takes the BatchNorm-backward reductions (FcParams::bw_raw)
+//   EPI_RELU   out = relu(conv + bias) on interior pixels and exact zeros on the border: the forward of an eval-mode BatchNorm + ReLU
+//              already folded into the weights and bias; padded-flat or phase planes (FcParams::planes)
+enum { EPI_PLAIN = 0, EPI_BW = 1, EPI_RELU = 2 };
+template <int ROWB, int N, int EPI>
 __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant__ CUtensorMap map_src, const __grid_constant__ CUtensorMap map_tail,
                                                           const __grid_constant__ CUtensorMap map_w, const FcParams p,
                                                           const float* __restrict__ bias, __nv_bfloat16* __restrict__ out) {
+  constexpr bool BW = EPI == EPI_BW, RELU = EPI == EPI_RELU;
   constexpr int NSLOT = (512 / N) > FC_MAX_SLOTS ? FC_MAX_SLOTS : (512 / N);
   constexpr uint32_t TMEM_COLS = NSLOT * N;
   constexpr int TPO = FC_BOX / N;                  // taps per weight box
@@ -390,14 +398,19 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
         bool keep = false;                    // interior pixel (the only ones BatchNorm statistics run over)
         constexpr bool bw = BW;
         const __nv_bfloat16* rrow = nullptr;  // bw: this row's pixel in raw
-        if (p.st_out && q < p.rows) {
+        if ((RELU || p.st_out) && q < p.rows) {
           const int qi = (int)q;
           const int n = fast_div(qi, p.st_mul_img, p.st_shr_img);
           const int r = qi - n * ((p.st_h + 2) * (p.st_w + 2));
           const int i = fast_div(r, p.st_mul_row, p.st_shr_row), j = r - i * (p.st_w + 2);
-          if (!BW || !p.bw_planes) {
+          if (!BW || !p.planes) {
             keep = i >= 1 && i <= p.st_h && j >= 1 && j <= p.st_w;
             if (bw) rrow = p.bw_raw + q * (long long)N;
+            if (RELU && p.planes) {           // padded pixel (i, j) -> plane (i&1, j&1) at (i>>1 + 1, j>>1 + 1): the inverse of tc.to_phase
+              const int hq = (p.st_h - 1) / 2 + 3, wq = (p.st_w - 1) / 2 + 3;
+              const long long prow = ((i & 1) * 2 + (j & 1)) * p.plane_out_stride + ((long long)n * hq + (i >> 1) + 1) * wq + (j >> 1) + 1;
+              orow = out + prow * (long long)p.ld_out + nb * N;
+            }
           } else {
             const int hp = 2 * (i - 1) + (pl >> 1), wp = 2 * (j - 1) + (pl & 1);
             keep = hp >= 1 && hp <= p.bw_H && wp >= 1 && wp <= p.bw_W;
@@ -437,6 +450,10 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
               a += s_bias[c0 + 2 * i];
               b += s_bias[c0 + 2 * i + 1];
             }
+            if (RELU) {
+              a = keep ? fmaxf(a, 0.f) : 0.f;
+              b = keep ? fmaxf(b, 0.f) : 0.f;
+            }
             __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
             pk[i] = *reinterpret_cast<uint32_t*>(&h);
           }
@@ -444,7 +461,7 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
             *reinterpret_cast<uint4*>(orow + c0) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
             *reinterpret_cast<uint4*>(orow + c0 + 8) = make_uint4(pk[4], pk[5], pk[6], pk[7]);
           }
-          if (p.st_out && !bw) {              // warp-uniform: statistics of exactly the values the BatchNorm kernels will read back
+          if (!RELU && p.st_out && !bw) {     // warp-uniform: statistics of exactly the values the BatchNorm kernels will read back
             float x[16];
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
@@ -489,7 +506,7 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
       }
       acc_cnt += item_slots;
     }
-    if (p.st_out && !(lane & 1)) {            // one shared-memory add per warp and column, once per kernel
+    if (!RELU && p.st_out && !(lane & 1)) {   // one shared-memory add per warp and column, once per kernel
       const int col = ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1);
 #pragma unroll
       for (int i = 0; i < N / 16; ++i) {
@@ -501,7 +518,7 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc<TMEM_COLS>(tmem_base);
-  if (p.st_out && !BW)
+  if (!RELU && p.st_out && !BW)
     for (int i = tid; i < 2 * N; i += blockDim.x) atomicAdd(p.st_out + i, (double)s_stat[i]);
   if (BW && p.st_out)                     // sum g*xhat = invstd * (sum g*x - mean * sum g), combined in fp64 (as pad_reduce_kernel does)
     for (int i = tid; i < N; i += blockDim.x) {
@@ -557,7 +574,7 @@ void finish_units(FcParams& p) {
   }
 }
 
-template <int ROWB, int N, bool BW>
+template <int ROWB, int N, int EPI>
 int launch_flatconv(const void* src, long long src_rows, int K, const void* wpk, long long w_rows, FcParams& p, const float* bias,
                     __nv_bfloat16* out, cudaStream_t st) {
   constexpr int TPO = FC_BOX / N;
@@ -610,19 +627,20 @@ int launch_flatconv(const void* src, long long src_rows, int K, const void* wpk,
   e = make_tmap_2d(&mw, wpk, w_rows, K, FC_BOX, ROWB / 2, ROWB);
   if (e) return e;
   static size_t configured[CVAD_MAX_DEVICES] = {};
-  const cudaError_t ce = cvad_ensure_dyn_smem(flatconv_kernel<ROWB, N, BW>, smem, configured);
+  const cudaError_t ce = cvad_ensure_dyn_smem(flatconv_kernel<ROWB, N, EPI>, smem, configured);
   if (ce != cudaSuccess) return (int)ce;
   const long long MT = 128LL * p.sub;
   const long long total = ((p.rows + MT - 1) / MT) * p.n_blocks * p.n_groups;
   int grid = (int)(total < cvad_num_sms() ? total : cvad_num_sms());
   if (grid < total) grid -= grid % p.n_groups;           // the kernel's group rotation needs whole tiles per round
-  flatconv_kernel<ROWB, N, BW><<<grid, 384, smem, st>>>(ms, mt, mw, p, bias, out);
+  flatconv_kernel<ROWB, N, EPI><<<grid, 384, smem, st>>>(ms, mt, mw, p, bias, out);
   CVAD_LAUNCH_CHECK();
   return 0;
 }
 
-// `K` reduction channels (the gathered tensor's channel count), `Nout` output channels.
-int run_flat(const void* src, long long src_rows, int K, const void* wpk, int Nout, const float* bias, void* out, FcParams& p, cudaStream_t st) {
+// `K` reduction channels (the gathered tensor's channel count), `Nout` output channels.  relu: the EPI_RELU epilogue (forward only).
+int run_flat(const void* src, long long src_rows, int K, const void* wpk, int Nout, const float* bias, void* out, FcParams& p, cudaStream_t st,
+             bool relu = false) {
   if (K % 32 || Nout % 32) return (int)cudaErrorInvalidValue;
   if (K >= 64 && K % 64) return (int)cudaErrorInvalidValue;
   const int rowb = K >= 64 ? 128 : 64;
@@ -631,8 +649,9 @@ int run_flat(const void* src, long long src_rows, int K, const void* wpk, int No
   p.ld_out = Nout;
   const long long w_rows = 9LL * Nout;
   __nv_bfloat16* o = (__nv_bfloat16*)out;
-#define CVAD_FC(R, NN) (p.bw_raw ? launch_flatconv<R, NN, true>(src, src_rows, K, wpk, w_rows, p, bias, o, st) \
-                                 : launch_flatconv<R, NN, false>(src, src_rows, K, wpk, w_rows, p, bias, o, st))
+#define CVAD_FC(R, NN) (relu ? launch_flatconv<R, NN, EPI_RELU>(src, src_rows, K, wpk, w_rows, p, bias, o, st)      \
+                        : p.bw_raw ? launch_flatconv<R, NN, EPI_BW>(src, src_rows, K, wpk, w_rows, p, bias, o, st) \
+                                   : launch_flatconv<R, NN, EPI_PLAIN>(src, src_rows, K, wpk, w_rows, p, bias, o, st))
   if (rowb == 64) {
     if (n == 32) return CVAD_FC(64, 32);
     if (n == 64) return CVAD_FC(64, 64);
@@ -700,23 +719,30 @@ CVAD_API int cvad_flat_pack_w3x3_bf16(const float* w, int Cout, int Cin, int str
 
 namespace {
 int flat_fwd(const void* x, const void* w_fwd, const float* bias, void* y, int N, int H, int W, int Cin, int Cout, int stride, double* stats,
-             void* stream);
+             int relu_phase, void* stream);
 }
 
 CVAD_API int cvad_flat_conv3x3_fwd_bf16(const void* x, const void* w_fwd, const float* bias, void* y, int N, int H, int W, int Cin, int Cout,
                                         int stride, void* stream) {
-  return flat_fwd(x, w_fwd, bias, y, N, H, W, Cin, Cout, stride, nullptr, stream);
+  return flat_fwd(x, w_fwd, bias, y, N, H, W, Cin, Cout, stride, nullptr, -1, stream);
 }
 
 CVAD_API int cvad_flat_conv3x3_fwd_stats_bf16(const void* x, const void* w_fwd, const float* bias, void* y, int N, int H, int W, int Cin,
                                               int Cout, int stride, double* stats, void* stream) {
   if (!stats || Cout != n_block_of(Cout)) return (int)cudaErrorInvalidValue;      // one output-channel block per CTA row tile
-  return flat_fwd(x, w_fwd, bias, y, N, H, W, Cin, Cout, stride, stats, stream);
+  return flat_fwd(x, w_fwd, bias, y, N, H, W, Cin, Cout, stride, stats, -1, stream);
+}
+
+CVAD_API int cvad_flat_conv3x3_fwd_relu_bf16(const void* x, const void* w_fwd, const float* bias, void* y, int N, int H, int W, int Cin,
+                                             int Cout, int stride, int phase_out, void* stream) {
+  if (phase_out != 0 && phase_out != 1) return (int)cudaErrorInvalidValue;
+  return flat_fwd(x, w_fwd, bias, y, N, H, W, Cin, Cout, stride, nullptr, phase_out, stream);
 }
 
 namespace {
+// relu_phase: -1 = plain epilogue; 0 / 1 = EPI_RELU writing padded-flat / phase planes
 int flat_fwd(const void* x, const void* w_fwd, const float* bias, void* y, int N, int H, int W, int Cin, int Cout, int stride, double* stats,
-             void* stream) {
+             int relu_phase, void* stream) {
   if (stride != 1 && stride != 2) return (int)cudaErrorInvalidValue;
   const int slab = Cin >= 64 ? 64 : 32;
   const int nslab = Cin / slab;
@@ -759,7 +785,7 @@ int flat_fwd(const void* x, const void* w_fwd, const float* bias, void* y, int N
         }
       }
   }
-  if (stats) {
+  if (stats || relu_phase >= 0) {      // the epilogue decodes (image, row, column) of its pixel
     if (p.rows > 0x7fffffffLL) return (int)cudaErrorInvalidValue;
     p.st_out = stats;
     p.st_h = stride == 1 ? H : (H - 1) / 2 + 1;
@@ -767,7 +793,11 @@ int flat_fwd(const void* x, const void* w_fwd, const float* bias, void* y, int N
     fast_div_init((unsigned)((p.st_h + 2) * (p.st_w + 2)), p.st_mul_img, p.st_shr_img);
     fast_div_init((unsigned)(p.st_w + 2), p.st_mul_row, p.st_shr_row);
   }
-  return run_flat(x, src_rows, Cin, w_fwd, Cout, bias, y, p, (cudaStream_t)stream);
+  if (relu_phase == 1) {                // the next stride-2 convolution's planes: (N, (st_h-1)/2+3, (st_w-1)/2+3) rows each
+    p.planes = 1;
+    p.plane_out_stride = (long long)N * ((p.st_h - 1) / 2 + 3) * ((p.st_w - 1) / 2 + 3);
+  }
+  return run_flat(x, src_rows, Cin, w_fwd, Cout, bias, y, p, (cudaStream_t)stream, relu_phase >= 0);
 }
 }  // namespace
 
@@ -783,7 +813,7 @@ void set_bw(FcParams& p, const BwStats* bw, int H, int W, int planes) {
   p.bw_raw = (const __nv_bfloat16*)bw->raw;
   p.bw_gamma = bw->gamma; p.bw_beta = bw->beta; p.bw_mean = bw->mean; p.bw_invstd = bw->invstd;
   p.st_out = bw->ws;
-  p.bw_H = H; p.bw_W = W; p.bw_planes = planes;
+  p.bw_H = H; p.bw_W = W; p.planes = planes;
   // the rows of this launch live in the geometry (st_h+2) x (st_w+2): the padded input itself (stride 1) or one phase plane (stride 2)
   p.st_h = planes ? (H - 1) / 2 + 1 : H;
   p.st_w = planes ? (W - 1) / 2 + 1 : W;

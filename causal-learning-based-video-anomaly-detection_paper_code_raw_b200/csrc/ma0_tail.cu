@@ -6,6 +6,8 @@
 //   masked_mean      vad:398-399  score.mean() over the clip's tracks
 //   ma0_loss         vad:516-531  MSE(scores, labels) + 0.001 * (sum of finite KL terms / number of finite KL terms), with gradients
 //   window_features  streaming sliding-window inference: gathers (n_windows, T, F) clips out of a ring of per-frame features
+//   stream cursor    the same ring driven by a device-side cursor {frames pushed, next window}, so that one captured CUDA graph serves
+//                    every push of a given size: ring_write, window_features_cursor, then cursor_advance (stream-ordered after both)
 #include "common.cuh"
 #include "cvad_b200.h"
 
@@ -178,6 +180,40 @@ __global__ void window_features_kernel(const float4* __restrict__ ring, long lon
   }
 }
 
+// ring[(cursor[0] + r) % cap][:] = feats[r][:] for r < n
+__global__ void ring_write_kernel(const float4* __restrict__ feats, long long n, int F4, float4* __restrict__ ring, long long cap,
+                                  const long long* __restrict__ cursor) {
+  cvad_pdl_enter();
+  const long long pos = cursor[0] % cap, total = n * F4;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long r = i / F4;
+    const long long fr = (pos + r) % cap;
+    ring[fr * F4 + (i - r * F4)] = __ldg(feats + i);
+  }
+}
+
+// window_features_kernel with first = cursor[1] * stride
+__global__ void window_features_cursor_kernel(const float4* __restrict__ ring, long long cap, int stride, int T, int F4, long long n_win,
+                                              const long long* __restrict__ cursor, float4* __restrict__ out) {
+  cvad_pdl_enter();
+  const long long first = cursor[1] * stride;
+  const long long total = n_win * T * F4;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const int v = (int)(i % F4);
+    const long long wt = i / F4;
+    const int t = (int)(wt % T);
+    const long long w = wt / T;
+    const long long fr = (first + w * stride + t) % cap;
+    out[i] = __ldg(ring + fr * F4 + v);
+  }
+}
+
+__global__ void stream_cursor_advance_kernel(long long* cursor, long long n, long long n_win) {
+  cvad_pdl_enter();
+  cursor[0] += n;
+  cursor[1] += n_win;
+}
+
 inline int blocks_of(long long n) {
   long long b = (n + 255) / 256;
   const long long cap = 8LL * cvad_num_sms();
@@ -244,6 +280,32 @@ CVAD_API int cvad_window_features_f32(const float* ring, long long capacity, lon
   if (F % 4 || capacity <= 0 || stride <= 0 || T <= 0 || first_frame < 0) return (int)cudaErrorInvalidValue;
   cvad_launch_pdl(window_features_kernel, dim3(blocks_of(n_windows * T * (F / 4))), dim3(256), 0, (cudaStream_t)stream, 
       reinterpret_cast<const float4*>(ring), capacity, first_frame, stride, T, F / 4, n_windows, reinterpret_cast<float4*>(out));
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
+CVAD_API int cvad_ring_write_f32(const float* feats, long long n, int F, float* ring, long long capacity, const long long* cursor, void* stream) {
+  if (n <= 0) return 0;
+  if (F % 4 || capacity <= 0 || n > capacity || !cursor) return (int)cudaErrorInvalidValue;
+  cvad_launch_pdl(ring_write_kernel, dim3(blocks_of(n * (F / 4))), dim3(256), 0, (cudaStream_t)stream, reinterpret_cast<const float4*>(feats), n,
+                  F / 4, reinterpret_cast<float4*>(ring), capacity, cursor);
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
+CVAD_API int cvad_window_features_cursor_f32(const float* ring, long long capacity, int stride, int T, int F, long long n_windows,
+                                             const long long* cursor, float* out, void* stream) {
+  if (n_windows <= 0) return 0;
+  if (F % 4 || capacity <= 0 || stride <= 0 || T <= 0 || !cursor) return (int)cudaErrorInvalidValue;
+  cvad_launch_pdl(window_features_cursor_kernel, dim3(blocks_of(n_windows * T * (F / 4))), dim3(256), 0, (cudaStream_t)stream,
+                  reinterpret_cast<const float4*>(ring), capacity, stride, T, F / 4, n_windows, cursor, reinterpret_cast<float4*>(out));
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
+CVAD_API int cvad_stream_cursor_advance(long long* cursor, long long n, long long n_windows, void* stream) {
+  if (!cursor || n < 0 || n_windows < 0) return (int)cudaErrorInvalidValue;
+  cvad_launch_pdl(stream_cursor_advance_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, cursor, n, n_windows);
   CVAD_LAUNCH_CHECK();
   return 0;
 }

@@ -23,14 +23,18 @@ class GraphedStep:
     ``__call__(*inputs)`` copies the inputs into the static buffers (an H2D copy when they live in pinned host memory),
     replays the graph and returns the static output tensors (valid until the next replay)."""
 
-    def __init__(self, step_fn, example_inputs, mutated=(), warmup: int = 3, pre_replay=None, between=None, tail_fn=None, stages=None):
+    def __init__(self, step_fn, example_inputs, mutated=(), warmup: int = 3, pre_replay=None, between=None, tail_fn=None, stages=None,
+                 pool=None):
         """``between`` / ``tail_fn`` split the step in two graphs around an eagerly issued call: graph(step_fn) ->
         between() -> graph(tail_fn).  The data-parallel trainer uses it to keep the NCCL gradient all-reduce OUT of the
         captured graphs (``between``) while forward/backward and the fused optimizer are each one graph launch.
 
         ``stages``: the general form, a list ``[(eager_fn or None, graph_fn), ...]`` run after ``step_fn``'s graph: for every entry
         the eager callable is issued on the current stream (e.g. an asynchronous collective), then the graph of ``graph_fn()`` is
-        replayed.  All graphs share one memory pool, so later stages may use tensors that earlier stages produced."""
+        replayed.  All graphs share one memory pool, so later stages may use tensors that earlier stages produced.
+
+        ``pool``: a memory pool handle (``torch.cuda.graph_pool_handle()``) to capture into, shared with other steps that are never
+        replayed concurrently with this one (default: a private pool)."""
         self.pre_replay = pre_replay
         if stages is None:
             stages = [(between, tail_fn)] if (between is not None or tail_fn is not None) else []
@@ -58,7 +62,7 @@ class GraphedStep:
         del snap
         self.graph = torch.cuda.CUDAGraph()
         n0 = ops.LAUNCHES[0]
-        with torch.cuda.graph(self.graph):
+        with torch.cuda.graph(self.graph, pool=pool):
             out = step_fn(*self.static_inputs)
         pool = self.graph.pool()
         captured = []

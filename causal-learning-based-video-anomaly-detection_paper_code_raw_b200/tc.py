@@ -117,42 +117,7 @@ class _BackboneBF16(torch.autograd.Function):
             else:
                 _call("cvad_bn_eval_prepare_f32", C1, float(bn1.eps), _ptr(bn1.running_mean), _ptr(bn1.running_var), _ptr(mean), _ptr(invstd), st)
 
-        done = False
-        n8 = int(ops.L().cvad_stem8_bytes(N, H, W)) if (STEM_F16 and STEM_FUSED_POOL) else -1
-        if n8 >= 0:
-            # fp16 stem over a 2x4 space-to-depth (frame width a multiple of 4): 6 MMAs of N = 64 per 256 outputs, pass 2 fused with the pool
-            x8 = torch.empty(n8, device=dev, dtype=torch.uint8)
-            if x.dtype == torch.uint8:  # raw frames: Normalize(mean, std) of cad:1177-1179 applied on the fly
-                _call("cvad_stem8_space_to_depth_u8", _ptr(x), N, H, W, float(bb.input_mean), float(bb.input_std), _ptr(x8), st)
-            else:
-                _call("cvad_stem8_space_to_depth_f32", _ptr(x), N, H, W, _ptr(x8), st)
-            bn1_statistics("cvad_stem8_f16_stats", x8)
-            _call("cvad_stem8_f16_bn_relu_maxpool", _ptr(x8), _ptr(w1), _ptr(b1), N, H, W, _ptr(mean), _ptr(invstd), _ptr(bn1.weight),
-                  _ptr(bn1.bias), _ptr(a), st)
-            done = True
-            del x8
-        if not done:
-            n4 = int(ops.L().cvad_stem_x4_floats(N, H, W))
-            if n4 < 0:
-                raise RuntimeError(f"frame size {H}x{W} is outside the tensor-core stem's range")
-            x4 = torch.empty(n4, device=dev, dtype=torch.float32)       # 2x2 space-to-depth of the batch: 16-byte pixels
-            if x.dtype == torch.uint8:
-                _call("cvad_stem_space_to_depth_u8", _ptr(x), N, H, W, float(bb.input_mean), float(bb.input_std), _ptr(x4), st)
-            else:
-                _call("cvad_stem_space_to_depth_f32", _ptr(x), N, H, W, _ptr(x4), st)
-            bn1_statistics("cvad_stem_tf32_stats", x4)
-            fused = 801
-            if STEM_FUSED_POOL:
-                # pass 2 and MaxPool(3,2,1) in one kernel: the 708 MB tensor between them stays in shared memory (801 = a band does not fit)
-                fused = _call("cvad_stem_tf32_bn_relu_maxpool", _ptr(x4), _ptr(w1), _ptr(b1), N, H, W, _ptr(mean), _ptr(invstd), _ptr(bn1.weight),
-                              _ptr(bn1.bias), _ptr(a), st, accept=(801,))
-            if fused == 801:
-                y1 = torch.empty((N, H1, W1, C1), device=dev, dtype=BF16)
-                _call("cvad_stem_tf32_bn_relu", _ptr(x4), _ptr(w1), _ptr(b1), N, H, W, _ptr(mean), _ptr(invstd), _ptr(bn1.weight), _ptr(bn1.bias),
-                      _ptr(y1), st)
-                _call("cvad_pad_maxpool3x3s2_bf16", _ptr(y1), N, H1, W1, C1, _ptr(a), st)
-                del y1
-            del x4
+        stem_forward(bb, x, a, mean, invstd, bn1_statistics)
         del x
         cur.wait_stream(side)
         saved = []
@@ -253,6 +218,53 @@ class _BackboneBF16(torch.autograd.Function):
             cur.wait_stream(side)
             keep.clear()
         return (None, None) + (None,) * (len(ctx.needs_input_grad) - 2)
+
+
+def stem_forward(bb, x, a, mean, invstd, bn1_statistics=None):
+    """The stem conv1 -> bn1 -> ReLU -> MaxPool(3,2,1) of x (N,1,H,W) (uint8 raw frames or normalised fp32, contiguous) into ``a``, the
+    padded-flat (N, h+2, w+2, 32) bf16 input of layer1.  Takes the fp16 stem over a 2x4 space-to-depth when the frame width allows it,
+    else the tf32 stem with pass 2 fused with the pool, else the unfused tf32 stem and a separate pool.  ``bn1_statistics(entry, xs)``
+    fills (mean, invstd) between the space-to-depth and pass 2 (``entry``: the batch-statistics entry point of the chosen stem over
+    its space-to-depth ``xs``); None: they already hold bn1's."""
+    N, _, H, W = x.shape
+    dev, st = x.device, _st()
+    bn1, conv1 = bb.bn1, bb.conv1
+    C1 = conv1.out_channels
+    H1, W1 = out_hw(H, W, 2)
+    w1, b1 = conv1.weight.detach(), conv1.bias.detach()
+    n8 = int(ops.L().cvad_stem8_bytes(N, H, W)) if (STEM_F16 and STEM_FUSED_POOL) else -1
+    if n8 >= 0:
+        # fp16 stem over a 2x4 space-to-depth (frame width a multiple of 4): 6 MMAs of N = 64 per 256 outputs, pass 2 fused with the pool
+        x8 = torch.empty(n8, device=dev, dtype=torch.uint8)
+        if x.dtype == torch.uint8:  # raw frames: Normalize(mean, std) of cad:1177-1179 applied on the fly
+            _call("cvad_stem8_space_to_depth_u8", _ptr(x), N, H, W, float(bb.input_mean), float(bb.input_std), _ptr(x8), st)
+        else:
+            _call("cvad_stem8_space_to_depth_f32", _ptr(x), N, H, W, _ptr(x8), st)
+        if bn1_statistics is not None:
+            bn1_statistics("cvad_stem8_f16_stats", x8)
+        _call("cvad_stem8_f16_bn_relu_maxpool", _ptr(x8), _ptr(w1), _ptr(b1), N, H, W, _ptr(mean), _ptr(invstd), _ptr(bn1.weight),
+              _ptr(bn1.bias), _ptr(a), st)
+        return
+    n4 = int(ops.L().cvad_stem_x4_floats(N, H, W))
+    if n4 < 0:
+        raise RuntimeError(f"frame size {H}x{W} is outside the tensor-core stem's range")
+    x4 = torch.empty(n4, device=dev, dtype=torch.float32)       # 2x2 space-to-depth of the batch: 16-byte pixels
+    if x.dtype == torch.uint8:
+        _call("cvad_stem_space_to_depth_u8", _ptr(x), N, H, W, float(bb.input_mean), float(bb.input_std), _ptr(x4), st)
+    else:
+        _call("cvad_stem_space_to_depth_f32", _ptr(x), N, H, W, _ptr(x4), st)
+    if bn1_statistics is not None:
+        bn1_statistics("cvad_stem_tf32_stats", x4)
+    fused = 801
+    if STEM_FUSED_POOL:
+        # pass 2 and MaxPool(3,2,1) in one kernel: the 708 MB tensor between them stays in shared memory (801 = a band does not fit)
+        fused = _call("cvad_stem_tf32_bn_relu_maxpool", _ptr(x4), _ptr(w1), _ptr(b1), N, H, W, _ptr(mean), _ptr(invstd), _ptr(bn1.weight),
+                      _ptr(bn1.bias), _ptr(a), st, accept=(801,))
+    if fused == 801:
+        y1 = torch.empty((N, H1, W1, C1), device=dev, dtype=BF16)
+        _call("cvad_stem_tf32_bn_relu", _ptr(x4), _ptr(w1), _ptr(b1), N, H, W, _ptr(mean), _ptr(invstd), _ptr(bn1.weight), _ptr(bn1.bias),
+              _ptr(y1), st)
+        _call("cvad_pad_maxpool3x3s2_bf16", _ptr(y1), N, H1, W1, C1, _ptr(a), st)
 
 
 def backbone_forward_bf16(bb, x):

@@ -145,6 +145,13 @@ int cvad_ma0_loss_f32(const float* scores, const float* kl, const long long* lab
  * `capacity` frames x F floats; out (n_windows, T, F) gathers window w = frames first_frame + w*stride + [0,T) (indices modulo capacity) */
 int cvad_window_features_f32(const float* ring, long long capacity, long long first_frame, int stride, int T, int F, long long n_windows,
                              float* out, void* stream);
+/* The same ring driven by a device-side cursor[2] = {frames pushed, next window}, so that a captured CUDA graph serves every push of one
+ * size: ring_write puts feats (n, F) at ring rows (cursor[0] + [0,n)) % capacity; window_features_cursor is cvad_window_features_f32 with
+ * first_frame = cursor[1] * stride; cursor_advance adds (n, n_windows) to the cursor (issue it after the other two, on the same stream). */
+int cvad_ring_write_f32(const float* feats, long long n, int F, float* ring, long long capacity, const long long* cursor, void* stream);
+int cvad_window_features_cursor_f32(const float* ring, long long capacity, int stride, int T, int F, long long n_windows,
+                                    const long long* cursor, float* out, void* stream);
+int cvad_stream_cursor_advance(long long* cursor, long long n, long long n_windows, void* stream);
 
 /* ---- M-A causal branch, dense masked batched form (ma_tail.cu) -------------------------------------------------------
  * Every clip carries 5 padded track slots (the detector emits <= 5 boxes per frame, cad:178,198) and a per-clip track
@@ -209,6 +216,12 @@ int cvad_flat_conv3x3_fwd_bf16(const void* x, const void* w_fwd, const float* bi
  * Cout must be 32, 64, 128 or 256. */
 int cvad_flat_conv3x3_fwd_stats_bf16(const void* x, const void* w_fwd, const float* bias, void* y, int N, int H, int W, int Cin, int Cout,
                                      int stride, double* stats, void* stream);
+/* y = relu(conv3x3(x) + bias) in bf16, for an eval-mode BatchNorm already folded into w_fwd / bias (cvad_bn_fold_conv_f32 then
+ * cvad_flat_pack_w3x3_bf16).  phase_out = 0: y padded-flat (N,Ho+2,Wo+2,Cout), border written as exact zeros.
+ * phase_out = 1: y = the four phase planes (4,N,Ho2+2,Wo2+2,Cout) the next stride-2 convolution reads; every plane position that
+ * corresponds to a padded pixel is written (0 on the border), positions with no source pixel must be zero on entry and are not touched. */
+int cvad_flat_conv3x3_fwd_relu_bf16(const void* x, const void* w_fwd, const float* bias, void* y, int N, int H, int W, int Cin, int Cout,
+                                    int stride, int phase_out, void* stream);
 /* mean = ws[c]/count, var = ws[C+c]/count - mean^2 (biased) -> invstd; running stats with momentum and the unbiased variance
  * (nn.BatchNorm2d train mode); running_mean / running_var / num_batches_tracked may be NULL.  Re-zeroes ws. */
 int cvad_bn_finalize_f64(double* ws, int C, double count, float eps, float momentum, float* mean, float* invstd, float* running_mean,
