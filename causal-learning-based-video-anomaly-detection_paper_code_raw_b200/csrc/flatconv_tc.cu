@@ -670,11 +670,65 @@ __host__ __device__ inline int packed_tap(int stride, int i) {
   const int s2[9] = {0, 2, 6, 8, 1, 7, 3, 5, 4};
   return stride == 2 ? s2[i] : i;
 }
-// index of the first packed tap of phase plane pl and the number of taps in it (stride 2)
-inline void plane_taps(int pl, int& first, int& count) {
+// index of the first packed tap of source plane pl and the number of taps in it: stride 1 has one plane holding all nine taps,
+// stride 2 the four phase planes
+inline void plane_taps(int stride, int pl, int& first, int& count) {
   static const int f[4] = {0, 4, 6, 8}, c[4] = {4, 2, 2, 1};
-  first = f[pl];
-  count = c[pl];
+  first = stride == 2 ? f[pl] : 0;
+  count = stride == 2 ? c[pl] : 9;
+}
+
+// Geometry of a 3x3 convolution with input (N, H, W): the output interior h x w, its padded-flat rows (N, h+2, w+2) and their pitch
+// wrow, and the number of source planes in that geometry (stride 1: the padded input itself; stride 2: its four phase planes).
+struct FlatGeom {
+  int stride, h, w, wrow, planes;
+  long long rows;
+};
+inline FlatGeom flat_geom(int N, int H, int W, int stride) {
+  const int h = stride == 1 ? H : (H - 1) / 2 + 1, w = stride == 1 ? W : (W - 1) / 2 + 1;
+  return {stride, h, w, w + 2, stride == 1 ? 1 : 4, (long long)N * (h + 2) * (w + 2)};
+}
+
+// The epilogue's (image, row, column) decode of its output row over the geometry g (ReLU output, fused statistics): the row index is
+// decoded in 32 bits.
+int set_pixel_decode(FcParams& p, const FlatGeom& g) {
+  if (g.rows > 0x7fffffffLL) return (int)cudaErrorInvalidValue;
+  p.st_h = g.h;
+  p.st_w = g.w;
+  fast_div_init((unsigned)((g.h + 2) * (g.w + 2)), p.st_mul_img, p.st_shr_img);
+  fast_div_init((unsigned)(g.w + 2), p.st_mul_row, p.st_shr_row);
+  return 0;
+}
+
+// Appends the units of one work item that reads source planes pl0 .. pl0+n-1: one unit per K slab, walking the packed taps of those
+// planes in order, the taps of plane pl0+a accumulating into set a.  Tap (kh, kw) lies shift = (kh/stride)*wrow + kw/stride rows into
+// its plane.  The forward reads it at +shift from the segment start (row_off: one row and column before the output for stride 1, the
+// plane's offset in the stacked phase planes for stride 2); the data-gradient, the transposed sum, at shift(2,2) - shift.
+// group >= 0: the units form that group of p, whose set a writes output plane pl0+a.
+void add_units(FcParams& p, const FlatGeom& g, bool dgrad, int slab, int nslab, int nblk, int pl0, int n, int group) {
+  auto shift = [&](int t) { return t / 3 / g.stride * g.wrow + t % 3 / g.stride; };
+  if (group >= 0) {
+    p.n_groups = group + 1;
+    p.acc_sets = n;
+    p.group_unit0[group] = p.n_units;
+    p.group_nunits[group] = nslab;
+    for (int a = 0; a < n; ++a) p.group_plane[group][a] = pl0 + a;
+  }
+  for (int s = 0; s < nslab; ++s) {
+    FcUnit& u = p.units[p.n_units++];
+    u.row_off = dgrad || g.stride == 1 ? -(g.wrow + 1) : (int)(pl0 * g.rows);
+    u.col = s * slab;
+    for (int a = 0; a < n; ++a) {
+      int first, count;
+      plane_taps(g.stride, pl0 + a, first, count);
+      if (a == 0) u.w_row0 = first * nblk;
+      for (int i = 0; i < count; ++i, ++u.ntaps) {
+        const int t = packed_tap(g.stride, first + i);
+        u.tap_delta[u.ntaps] = dgrad ? shift(8) - shift(t) : shift(t);
+        u.tap_acc[u.ntaps] = (unsigned char)a;
+      }
+    }
+  }
 }
 
 // OIHW fp32 (Co, Ci, 3, 3) -> fwd [n-block][packed tap][N][Ci] bf16 (N = block of Co) and dgrad [n-block][packed tap][Nd][Co] (Nd = block of Ci)
@@ -746,58 +800,21 @@ int flat_fwd(const void* x, const void* w_fwd, const float* bias, void* y, int N
   if (stride != 1 && stride != 2) return (int)cudaErrorInvalidValue;
   const int slab = Cin >= 64 ? 64 : 32;
   const int nslab = Cin / slab;
-  const int nblk = n_block_of(Cout);
+  const FlatGeom g = flat_geom(N, H, W, stride);
+  if (g.planes * nslab > FC_MAX_UNITS || (stride == 2 && 3 * g.rows > 0x7fffffffLL - (1 << 20))) return (int)cudaErrorInvalidValue;
   FcParams p;
   memset(&p, 0, sizeof(p));
-  long long src_rows;
-  if (stride == 1) {
-    const int Wp = W + 2;
-    p.rows = (long long)N * (H + 2) * Wp;
-    src_rows = p.rows;
-    if (nslab > FC_MAX_UNITS) return (int)cudaErrorInvalidValue;
-    p.n_units = nslab;
-    for (int s = 0; s < nslab; ++s) {
-      FcUnit& u = p.units[s];
-      u.row_off = -(Wp + 1);
-      u.col = s * slab;
-      u.ntaps = 9;
-      u.w_row0 = 0;
-      for (int t = 0; t < 9; ++t) u.tap_delta[t] = (t / 3) * Wp + (t % 3);
-    }
-  } else {
-    const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1, Wq = Wo + 2;
-    p.rows = (long long)N * (Ho + 2) * Wq;
-    src_rows = 4 * p.rows;
-    if (4 * nslab > FC_MAX_UNITS || 3 * p.rows > 0x7fffffffLL - (1 << 20)) return (int)cudaErrorInvalidValue;
-    p.n_units = 4 * nslab;
-    for (int pl = 0; pl < 4; ++pl)
-      for (int s = 0; s < nslab; ++s) {
-        FcUnit& u = p.units[pl * nslab + s];
-        int first, count;
-        plane_taps(pl, first, count);
-        u.row_off = (int)(pl * p.rows);
-        u.col = s * slab;
-        u.ntaps = count;
-        u.w_row0 = first * nblk;
-        for (int i = 0; i < count; ++i) {
-          const int t = packed_tap(2, first + i), kh = t / 3, kw = t % 3;
-          u.tap_delta[i] = (kh >> 1) * Wq + (kw >> 1);
-        }
-      }
-  }
-  if (stats || relu_phase >= 0) {      // the epilogue decodes (image, row, column) of its pixel
-    if (p.rows > 0x7fffffffLL) return (int)cudaErrorInvalidValue;
+  p.rows = g.rows;
+  for (int pl = 0; pl < g.planes; ++pl) add_units(p, g, false, slab, nslab, n_block_of(Cout), pl, 1, -1);
+  if (stats || relu_phase >= 0) {
+    if (int e = set_pixel_decode(p, g)) return e;
     p.st_out = stats;
-    p.st_h = stride == 1 ? H : (H - 1) / 2 + 1;
-    p.st_w = stride == 1 ? W : (W - 1) / 2 + 1;
-    fast_div_init((unsigned)((p.st_h + 2) * (p.st_w + 2)), p.st_mul_img, p.st_shr_img);
-    fast_div_init((unsigned)(p.st_w + 2), p.st_mul_row, p.st_shr_row);
   }
   if (relu_phase == 1) {                // the next stride-2 convolution's planes: (N, (st_h-1)/2+3, (st_w-1)/2+3) rows each
     p.planes = 1;
     p.plane_out_stride = (long long)N * ((p.st_h - 1) / 2 + 3) * ((p.st_w - 1) / 2 + 3);
   }
-  return run_flat(x, src_rows, Cin, w_fwd, Cout, bias, y, p, (cudaStream_t)stream, relu_phase >= 0);
+  return run_flat(x, g.planes * g.rows, Cin, w_fwd, Cout, bias, y, p, (cudaStream_t)stream, relu_phase >= 0);
 }
 }  // namespace
 
@@ -808,17 +825,14 @@ struct BwStats {           // BatchNorm-backward reductions fused into the data-
   double* ws;
 };
 
-void set_bw(FcParams& p, const BwStats* bw, int H, int W, int planes) {
-  if (!bw) return;
+// raw is H x W; the rows of the launch live in the geometry g: the padded input itself (stride 1) or one phase plane (stride 2)
+int set_bw(FcParams& p, const BwStats* bw, int H, int W, const FlatGeom& g) {
+  if (!bw) return 0;
   p.bw_raw = (const __nv_bfloat16*)bw->raw;
   p.bw_gamma = bw->gamma; p.bw_beta = bw->beta; p.bw_mean = bw->mean; p.bw_invstd = bw->invstd;
   p.st_out = bw->ws;
-  p.bw_H = H; p.bw_W = W; p.planes = planes;
-  // the rows of this launch live in the geometry (st_h+2) x (st_w+2): the padded input itself (stride 1) or one phase plane (stride 2)
-  p.st_h = planes ? (H - 1) / 2 + 1 : H;
-  p.st_w = planes ? (W - 1) / 2 + 1 : W;
-  fast_div_init((unsigned)((p.st_h + 2) * (p.st_w + 2)), p.st_mul_img, p.st_shr_img);
-  fast_div_init((unsigned)(p.st_w + 2), p.st_mul_row, p.st_shr_row);
+  p.bw_H = H; p.bw_W = W; p.planes = g.stride == 2;
+  return set_pixel_decode(p, g);
 }
 
 int flat_dgrad(const void* dy, const void* w_dgrad, void* dx, int N, int H, int W, int Cin, int Cout, int stride, const BwStats* bw,
@@ -831,125 +845,41 @@ int flat_dgrad(const void* dy, const void* w_dgrad, void* dx, int N, int H, int 
   const int nblk = n_block_of(Cin);
   if (nslab > FC_MAX_UNITS) return (int)cudaErrorInvalidValue;
   cudaStream_t st = (cudaStream_t)stream;
-  if (stride == 1) {
-    const int Wp = W + 2;
-    FcParams p;
-    memset(&p, 0, sizeof(p));
-    p.rows = (long long)N * (H + 2) * Wp;
-    p.n_units = nslab;
-    for (int s = 0; s < nslab; ++s) {
-      FcUnit& u = p.units[s];
-      u.row_off = -(Wp + 1);
-      u.col = s * slab;
-      u.ntaps = 9;
-      u.w_row0 = 0;
-      for (int t = 0; t < 9; ++t) u.tap_delta[t] = (2 - t / 3) * Wp + (2 - t % 3);
-    }
-    if (bw && p.rows > 0x7fffffffLL) return (int)cudaErrorInvalidValue;
-    set_bw(p, bw, H, W, 0);
-    return run_flat(dy, p.rows, Cout, w_dgrad, Cin, nullptr, dx, p, st);
-  }
-  const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1, Wq = Wo + 2;
-  const long long rows = (long long)N * (Ho + 2) * Wq;
+  const FlatGeom g = flat_geom(N, H, W, stride);
+  FcParams p;
+  memset(&p, 0, sizeof(p));
+  p.rows = g.rows;
   // (measured, profiles/r02c_conv_variants.md: the single fetch pays where the nine taps' weights stay resident in shared memory -- one
   // K slab, N = 32: 102 -> 92 us at 60x90 32->64 -- and loses where four accumulator sets shrink the work item to 128 rows and the weights
   // have to be streamed again for each of them: 70 -> 88 us at 30x45 64->128)
   const bool single_fetch = g_dgrad_mode == 2 && (g_fc_tune[2] ? true : (nslab == 1 && nblk == 32));
-  if (single_fetch && 2 * nslab <= FC_MAX_UNITS) {
+  if (stride == 1) {
+    add_units(p, g, true, slab, nslab, nblk, 0, 1, -1);
+  } else if (single_fetch && 2 * nslab <= FC_MAX_UNITS) {
     // One launch, and ONE fetch of each dy segment for all four phase planes of dx: a work item walks all nine taps (packed plane by
     // plane) and keeps one accumulator set per plane.  Four sets need 4 x N columns of TMEM per 128 rows: with N = 128 that is the whole
     // ring, so the planes are split into two groups of two sets whose packed taps are contiguous: {0,1} (4 + 2 taps), {2,3} (2 + 1).
     const int ngr = nblk >= 128 ? 2 : 1;
-    static const int grp_planes[2][2][4] = {{{0, 1, 2, 3}, {0, 0, 0, 0}}, {{0, 1, 0, 0}, {2, 3, 0, 0}}};
-    FcParams p;
-    memset(&p, 0, sizeof(p));
-    p.rows = rows;
-    p.n_groups = ngr;
-    p.acc_sets = 4 / ngr;
-    p.plane_out_stride = rows;
-    p.n_units = ngr * nslab;
-    for (int g = 0; g < ngr; ++g) {
-      p.group_unit0[g] = g * nslab;
-      p.group_nunits[g] = nslab;
-      for (int a = 0; a < p.acc_sets; ++a) p.group_plane[g][a] = grp_planes[ngr - 1][g][a];
-      for (int s = 0; s < nslab; ++s) {
-        FcUnit& u = p.units[g * nslab + s];
-        u.row_off = -(Wq + 1);
-        u.col = s * slab;
-        u.ntaps = 0;
-        for (int a = 0; a < p.acc_sets; ++a) {
-          int first, count;
-          plane_taps(p.group_plane[g][a], first, count);
-          if (a == 0) u.w_row0 = first * nblk;
-          for (int i = 0; i < count; ++i) {
-            const int t = packed_tap(2, first + i), kh = t / 3, kw = t % 3;
-            u.tap_delta[u.ntaps] = (Wq + 1) - ((kh >> 1) * Wq + (kw >> 1));
-            u.tap_acc[u.ntaps] = (unsigned char)a;
-            ++u.ntaps;
-          }
-        }
-      }
-    }
-    if (bw && rows > 0x7fffffffLL) return (int)cudaErrorInvalidValue;
-    set_bw(p, bw, H, W, 1);
-    return run_flat(dy, rows, Cout, w_dgrad, Cin, nullptr, dx, p, st);
-  }
-  if (g_dgrad_mode >= 1 && 4 * nslab <= FC_MAX_UNITS) {
+    p.plane_out_stride = g.rows;
+    for (int gi = 0; gi < ngr; ++gi) add_units(p, g, true, slab, nslab, nblk, gi * (4 / ngr), 4 / ngr, gi);
+  } else if (g_dgrad_mode >= 1 && 4 * nslab <= FC_MAX_UNITS) {
     // all four phase planes in one launch: plane pl is a set of work items with its own units (its 4 / 2 / 2 / 1 taps) and its own
     // output offset; one drain instead of four, but every plane fetches the dy segment again
-    FcParams p;
-    memset(&p, 0, sizeof(p));
-    p.rows = rows;
-    p.n_groups = 4;
-    p.acc_sets = 1;
-    p.plane_out_stride = rows;
-    p.n_units = 4 * nslab;
+    p.plane_out_stride = g.rows;
+    for (int pl = 0; pl < 4; ++pl) add_units(p, g, true, slab, nslab, nblk, pl, 1, pl);
+  } else {
+    if (bw) return (int)cudaErrorNotSupported;      // the fused reductions need the one-launch form (plane index per work item)
     for (int pl = 0; pl < 4; ++pl) {
-      int first, count;
-      plane_taps(pl, first, count);
-      p.group_unit0[pl] = pl * nslab;
-      p.group_nunits[pl] = nslab;
-      p.group_plane[pl][0] = pl;
-      for (int s = 0; s < nslab; ++s) {
-        FcUnit& u = p.units[pl * nslab + s];
-        u.row_off = -(Wq + 1);
-        u.col = s * slab;
-        u.ntaps = count;
-        u.w_row0 = first * nblk;
-        for (int i = 0; i < count; ++i) {
-          const int t = packed_tap(2, first + i), kh = t / 3, kw = t % 3;
-          u.tap_delta[i] = (Wq + 1) - ((kh >> 1) * Wq + (kw >> 1));
-        }
-      }
+      memset(&p, 0, sizeof(p));
+      p.rows = g.rows;
+      p.out_row_base = pl * g.rows;
+      add_units(p, g, true, slab, nslab, nblk, pl, 1, -1);
+      if (int e = run_flat(dy, g.rows, Cout, w_dgrad, Cin, nullptr, dx, p, st)) return e;
     }
-    if (bw && rows > 0x7fffffffLL) return (int)cudaErrorInvalidValue;
-    set_bw(p, bw, H, W, 1);
-    return run_flat(dy, rows, Cout, w_dgrad, Cin, nullptr, dx, p, st);
+    return 0;
   }
-  if (bw) return (int)cudaErrorNotSupported;      // the fused reductions need the one-launch form (plane index per work item)
-  for (int pl = 0; pl < 4; ++pl) {
-    FcParams p;
-    memset(&p, 0, sizeof(p));
-    p.rows = rows;
-    p.out_row_base = pl * rows;
-    p.n_units = nslab;
-    int first, count;
-    plane_taps(pl, first, count);
-    for (int s = 0; s < nslab; ++s) {
-      FcUnit& u = p.units[s];
-      u.row_off = -(Wq + 1);
-      u.col = s * slab;
-      u.ntaps = count;
-      u.w_row0 = first * nblk;
-      for (int i = 0; i < count; ++i) {
-        const int t = packed_tap(2, first + i), kh = t / 3, kw = t % 3;
-        u.tap_delta[i] = (Wq + 1) - ((kh >> 1) * Wq + (kw >> 1));
-      }
-    }
-    int e = run_flat(dy, rows, Cout, w_dgrad, Cin, nullptr, dx, p, st);
-    if (e) return e;
-  }
-  return 0;
+  if (int e = set_bw(p, bw, H, W, g)) return e;
+  return run_flat(dy, g.rows, Cout, w_dgrad, Cin, nullptr, dx, p, st);
 }
 }  // namespace
 
@@ -1272,17 +1202,17 @@ int flat_wgrad(const void* x, const void* dy, float* dw, float* scratch, int N, 
   if (stride != 1 && stride != 2) return (int)cudaErrorInvalidValue;
   cudaStream_t st = (cudaStream_t)stream;
   const int apm = Cin == 32 ? 4 : (Cin == 64 ? 2 : 1);     // taps one MMA can cover through pixel-shift atoms
+  const FlatGeom geo = flat_geom(N, H, W, stride);
   WgParams p;
   memset(&p, 0, sizeof(p));
   p.Cin = Cin; p.Cout = Cout;
   p.scratch = scratch;
+  p.rows = geo.rows;
   if (stride == 1 && g_wgrad_kh_stack && ((Cin == 32 && Cout == 32) || (Cin == 64 && Cout == 64))) {
     // dW[kh][kw] = sum_q' x[q' + kw - 1] * dy[q' - (kh - 1)*Wp]: the kw taps are pixel-shift atoms of M (as below), the kh taps are
     // atoms of N one padded image row apart, so one M128 x N(3*Cout) MMA per 16 pixels covers a 3 x apm block of taps.  The operand
     // stream per 16 pixels drops from 3 x 5 KB to 7 KB (32 channels) and from 6 x 6 KB to 2 x 10 KB (64 channels).
-    const int Wp = W + 2;
-    p.rows = (long long)N * (H + 2) * Wp;
-    p.b_halo = Wp;
+    p.b_halo = geo.wrow;
     p.n_variants = 1;
     WgVariant& v = p.v[0];
     v.n_seg = 1;
@@ -1296,8 +1226,7 @@ int flat_wgrad(const void* x, const void* dy, float* dw, float* scratch, int N, 
     return dispatch_wgrad(x, p.rows, dy, p, dw, st);
   }
   if (stride == 1) {
-    const int Wp = W + 2;
-    p.rows = (long long)N * (H + 2) * Wp;
+    const int Wp = geo.wrow;
     // wide layers: one variant per kernel row keeps 3 accumulators of 128 columns in TMEM; narrow layers: all nine taps at once
     p.n_variants = apm == 1 ? 3 : 1;
     for (int l = 0; l < p.n_variants; ++l) {
@@ -1315,8 +1244,7 @@ int flat_wgrad(const void* x, const void* dy, float* dw, float* scratch, int N, 
     }
     return dispatch_wgrad(x, p.rows, dy, p, dw, st);
   }
-  const int Ho = (H - 1) / 2 + 1, Wo = (W - 1) / 2 + 1, Wq = Wo + 2;
-  p.rows = (long long)N * (Ho + 2) * Wq;
+  const int Wq = geo.wrow;
   if (3 * p.rows > 0x7fffffffLL - (1 << 20)) return (int)cudaErrorInvalidValue;
   if (apm > 1 && g_fc_tune[3] == 0) {
     // Narrow layers: all four planes are resident per stage anyway.  A tap (kh,kw) lives in plane (kh&1, kw&1) at pixel shift
