@@ -320,7 +320,7 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
                 tc_fence_after();
                 if (elect_one()) {
 #pragma unroll
-                  for (int k = 0; k < K16; ++k) tc_mma_bf16(tmem_base + slot * N, da0 + (uint64_t)(s * (128 * ROWB / 16) + 2 * k), db0 + 2 * k, idesc, k != 0);
+                  for (int k = 0; k < K16; ++k) tc_mma_f16(tmem_base + slot * N, da0 + (uint64_t)(s * (128 * ROWB / 16) + 2 * k), db0 + 2 * k, idesc, k != 0);
                   if (last) tc_commit(&bar_acc_full[slot]);
                 }
                 __syncwarp();
@@ -331,7 +331,7 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
                 uint64_t da = da0;
                 for (int s = 0; s < sub; ++s) {
 #pragma unroll
-                  for (int k = 0; k < K16; ++k) tc_mma_bf16(tmem_base + slot * N, da + 2 * k, db0 + 2 * k, idesc, 1u);
+                  for (int k = 0; k < K16; ++k) tc_mma_f16(tmem_base + slot * N, da + 2 * k, db0 + 2 * k, idesc, 1u);
                   if (last) tc_commit(&bar_acc_full[slot]);
                   da += 128 * ROWB / 16;
                   slot = slot + 1 == NSLOT ? 0 : slot + 1;
@@ -620,11 +620,11 @@ int launch_flatconv(const void* src, long long src_rows, int K, const void* wpk,
   p.tail_rows = p.seg_rows % FC_BOX;
   const size_t smem = fixed + (size_t)p.wst * FC_BOX * ROWB;
   CUtensorMap ms, mt, mw;
-  int e = make_tmap_2d(&ms, src, src_rows, K, FC_BOX, ROWB / 2, ROWB);
+  int e = make_tmap_2d(&ms, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, src, src_rows, K, FC_BOX, ROWB / 2, ROWB);
   if (e) return e;
-  e = make_tmap_2d(&mt, src, src_rows, K, p.tail_rows ? p.tail_rows : 64, ROWB / 2, ROWB);
+  e = make_tmap_2d(&mt, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, src, src_rows, K, p.tail_rows ? p.tail_rows : 64, ROWB / 2, ROWB);
   if (e) return e;
-  e = make_tmap_2d(&mw, wpk, w_rows, K, FC_BOX, ROWB / 2, ROWB);
+  e = make_tmap_2d(&mw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, wpk, w_rows, K, FC_BOX, ROWB / 2, ROWB);
   if (e) return e;
   static size_t configured[CVAD_MAX_DEVICES] = {};
   const cudaError_t ce = cvad_ensure_dyn_smem(flatconv_kernel<ROWB, N, EPI>, smem, configured);
@@ -1038,7 +1038,7 @@ __global__ void __launch_bounds__(256, 1) flatwgrad_kernel(const __grid_constant
           for (int k = 0; k < ksteps; ++k) {
             const uint64_t da = da_hi | (uint64_t)(((a0 + k * 16 * ROWB_A) >> 4) & 0x3FFF);
             const uint64_t db = db_hi | (uint64_t)(((base + a_bytes_max + k * 16 * ROWB_B) >> 4) & 0x3FFF);
-            tc_mma_bf16(tacc, da, db, idesc, (it | k) != 0);
+            tc_mma_f16(tacc, da, db, idesc, (it | k) != 0);
           }
         }
         tc_commit(&bar_empty[st]);
@@ -1140,14 +1140,14 @@ int launch_wgrad(const void* src, long long src_rows, const void* dy, WgParams& 
   p.pix_per_cta = ((p.rows + chunks - 1) / chunks + qs - 1) / qs * qs;
   chunks = (p.rows + p.pix_per_cta - 1) / p.pix_per_cta;
   CUtensorMap ma, mat, mb;
-  int e = make_tmap_2d(&ma, src, src_rows, p.Cin, FC_BOX, ROWB_A / 2, ROWB_A);
+  int e = make_tmap_2d(&ma, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, src, src_rows, p.Cin, FC_BOX, ROWB_A / 2, ROWB_A);
   if (e) return e;
-  e = make_tmap_2d(&mat, src, src_rows, p.Cin, p.a_tail ? p.a_tail : 32, ROWB_A / 2, ROWB_A);
+  e = make_tmap_2d(&mat, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, src, src_rows, p.Cin, p.a_tail ? p.a_tail : 32, ROWB_A / 2, ROWB_A);
   if (e) return e;
   CUtensorMap mbt;
-  e = make_tmap_2d(&mb, dy, p.rows, p.Cout, KH == 3 ? FC_BOX : p.b_box, ROWB_B / 2, ROWB_B);
+  e = make_tmap_2d(&mb, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, dy, p.rows, p.Cout, KH == 3 ? FC_BOX : p.b_box, ROWB_B / 2, ROWB_B);
   if (e) return e;
-  e = make_tmap_2d(&mbt, dy, p.rows, p.Cout, p.b_tail ? p.b_tail : 32, ROWB_B / 2, ROWB_B);
+  e = make_tmap_2d(&mbt, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, dy, p.rows, p.Cout, p.b_tail ? p.b_tail : 32, ROWB_B / 2, ROWB_B);
   if (e) return e;
   static size_t configured[CVAD_MAX_DEVICES] = {};
   const cudaError_t ce = cvad_ensure_dyn_smem(flatwgrad_kernel<ROWB_A, ROWB_B, NB, A_SLABS, KH>, smem, configured);

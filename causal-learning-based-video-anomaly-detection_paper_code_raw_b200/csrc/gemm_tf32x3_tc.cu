@@ -32,15 +32,6 @@ constexpr int TG_TILE_BYTES = TG_BM * TG_BK * 4;             // 16 KiB per opera
 constexpr int TG_STAGE_BYTES = 4 * TG_TILE_BYTES;            // A, W, A_lo, W_lo
 constexpr size_t TG_SMEM = (size_t)TG_STAGES * TG_STAGE_BYTES + 1024;
 
-__device__ __forceinline__ void tg_mma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 __device__ __forceinline__ float to_tf32(float x) {
   uint32_t r;
   asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
@@ -108,9 +99,9 @@ __global__ void __launch_bounds__(256, 1) gemm_tf32x3_kernel(const __grid_consta
         const uint64_t dal = desc_hi | (uint64_t)((a_lo >> 4) & 0x3FFF), dwl = desc_hi | (uint64_t)((w_lo >> 4) & 0x3FFF);
 #pragma unroll
         for (int k = 0; k < TG_BK / 8; ++k) {                               // +32 bytes per K8 step
-          tg_mma_tf32(tmem_base, dal + 2 * k, dwh + 2 * k, idesc, (it | k) != 0);      // small terms first
-          tg_mma_tf32(tmem_base, dah + 2 * k, dwl + 2 * k, idesc, 1u);
-          tg_mma_tf32(tmem_base, dah + 2 * k, dwh + 2 * k, idesc, 1u);
+          tc_mma_tf32(tmem_base, dal + 2 * k, dwh + 2 * k, idesc, (it | k) != 0);      // small terms first
+          tc_mma_tf32(tmem_base, dah + 2 * k, dwl + 2 * k, idesc, 1u);
+          tc_mma_tf32(tmem_base, dah + 2 * k, dwh + 2 * k, idesc, 1u);
         }
         tc_commit(&bar_empty[st]);
       }
@@ -171,20 +162,6 @@ __global__ void __launch_bounds__(256, 1) gemm_tf32x3_kernel(const __grid_consta
   if (warp == 2) tmem_dealloc<128>(tmem_base);
 }
 
-// fp32 matrix [rows][cols] (row pitch = cols), box = 128 rows x 32 floats, SWIZZLE_128B; rows past the end read as zero
-int make_tmap_f32(CUtensorMap* m, const float* base, long long rows, int cols) {
-  EncodeTiledFn enc = encode_tiled_fn();
-  if (!enc) return (int)cudaErrorNotSupported;
-  memset(m, 0, sizeof(*m));
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)cols * 4};
-  cuuint32_t box[2] = {(cuuint32_t)TG_BK, (cuuint32_t)TG_BM};
-  cuuint32_t es[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
-}
-
 }  // namespace
 
 // y (M,N) fp32 must be ZERO on entry (split-K partial sums are added atomically); x (M,K), w (N,K) fp32 row-major, 16-byte aligned, K % 32 == 0.
@@ -192,9 +169,10 @@ CVAD_API int cvad_linear_fwd_tf32x3(const float* x, const float* w, float* y, in
   if (M <= 0 || N <= 0) return 0;
   if (K <= 0 || K % TG_BK || (((uintptr_t)x | (uintptr_t)w) & 15)) return (int)cudaErrorInvalidValue;
   CUtensorMap ma, mw;
-  int e = make_tmap_f32(&ma, x, M, K);
+  // 128 rows x 32 floats per box (one 128-byte swizzle row); rows past M / N read as zero
+  int e = make_tmap_2d(&ma, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, x, M, K, TG_BM, TG_BK, 128);
   if (e) return e;
-  e = make_tmap_f32(&mw, w, N, K);
+  e = make_tmap_2d(&mw, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, w, N, K, TG_BM, TG_BK, 128);
   if (e) return e;
   const int tiles = ((M + TG_BM - 1) / TG_BM) * ((N + TG_BN - 1) / TG_BN);
   const int k_chunks = K / TG_BK;

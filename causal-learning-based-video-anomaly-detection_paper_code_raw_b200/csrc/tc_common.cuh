@@ -75,11 +75,20 @@ __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::
 __device__ __forceinline__ void tc_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n" ::"r"(smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ void tc_mma_bf16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+// kind::f16 covers bf16 and fp16 operands: the instruction descriptor picks which
+__device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void tc_mma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
@@ -130,17 +139,19 @@ inline EncodeTiledFn encode_tiled_fn() {
   }
   return fn;
 }
-// bf16 matrix [rows][cols] (row pitch = cols), box = box_rows x box_cols, swizzle span = swizzle_bytes (64 or 128)
-inline int make_tmap_2d(CUtensorMap* m, const void* base, long long rows, int cols, int box_rows, int box_cols, int swizzle_bytes) {
+// matrix [rows][cols] of elem_bytes-byte elements of type dt (row pitch = cols), box = box_rows x box_cols, swizzle span =
+// swizzle_bytes (64 or 128; anything else: no swizzle); rows past the end read as zero
+inline int make_tmap_2d(CUtensorMap* m, CUtensorMapDataType dt, int elem_bytes, const void* base, long long rows, int cols, int box_rows,
+                        int box_cols, int swizzle_bytes) {
   EncodeTiledFn enc = encode_tiled_fn();
   if (!enc) return (int)cudaErrorNotSupported;
   memset(m, 0, sizeof(*m));
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)cols * 2};
+  cuuint64_t strides[1] = {(cuuint64_t)cols * elem_bytes};
   cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
   cuuint32_t es[2] = {1, 1};
   CUtensorMapSwizzle sw = swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE);
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
+  CUresult r = enc(m, dt, 2, const_cast<void*>(base), dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? 0 : (int)cudaErrorInvalidValue;
 }

@@ -274,7 +274,7 @@ int cvad_pad_bn_relu_bwd_bf16(const void* raw, const void* dact, void* draw, int
 int cvad_pad_avgpool_bf16_fwd(const void* x, int N, int H, int W, int C, int OH, int OW, float* out, void* stream);
 int cvad_pad_avgpool_bf16_bwd(const float* dout, int N, int H, int W, int C, int OH, int OW, void* dx, void* stream);
 
-/* ---- tensor-core stem (stem_tc.cu): conv 7x7 s2 p3, 1 -> 32 (cad:115,145) as a tcgen05 kind::tf32 implicit GEMM -----------
+/* ---- tensor-core stem (stem_tc.cu, both formulations): conv 7x7 s2 p3, 1 -> 32 (cad:115,145) as a tcgen05 kind::tf32 implicit GEMM
  * x (N,1,H,W) fp32, w (32,1,7,7) fp32 OIHW, bias (32).  First a 2x2 space-to-depth of x into X4 (N,Ho+3,Wo+3,4) fp32 -- 16-byte
  * pixels that TMA streams and the MMA descriptor turns into im2col rows; x4 must hold cvad_stem_x4_floats(N,H,W) floats.
  * Pass 1: bn1 batch statistics of conv(x)+bias without writing the convolution output (ws = 64 zeroed doubles, re-zeroed by
@@ -298,7 +298,7 @@ int cvad_stem_tf32_bn_relu(const float* x4, const float* w, const float* bias, i
 int cvad_stem_tf32_bn_relu_maxpool(const float* x4, const float* w, const float* bias, int N, int H, int W, const float* mean,
                                    const float* invstd, const float* gamma, const float* beta, void* out, void* stream);
 
-/* The stem's second formulation (stem_f16_tc.cu): tcgen05 kind::f16 over a 2x4 space-to-depth X8 of the frames (fp16, one 16-byte pixel =
+/* The stem's second formulation (also stem_tc.cu): tcgen05 kind::f16 over a 2x4 space-to-depth X8 of the frames (fp16, one 16-byte pixel =
  * a 2 x 4 patch = two adjacent outputs of the stride-2 convolution; accumulator rows carry N = 64 columns = (output parity, channel)):
  * 6 MMAs of M128 x N64 x K16 per 256 outputs instead of 16 of M128 x N32 x K8.  For frames whose width is a multiple of 4;
  * cvad_stem8_bytes returns the size of the X8 buffer or -1 when the shape is outside this path (callers then use the tf32 entries above).
