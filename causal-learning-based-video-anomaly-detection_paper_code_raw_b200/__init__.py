@@ -10,6 +10,7 @@ Public surface (mirrors the reference's Python seam, SURVEY.md 8b):
   ma0.CausalAnomalyDetector / ma0.train_model / ma0.test_model               video_anomaly_detection.py
   ma0.StreamingWindowScorer (sliding windows over a frame stream: each frame's backbone pass is computed once)
   infer.GraphedStreamingScorer / infer.FrozenBackbone (the same windows, one CUDA graph replay per push; eval BatchNorm folded into the convolutions)
+  infer.MultiStreamScorer (many cameras or the videos of a test set: one push and one CUDA graph replay per tick for all streams)
   md.VideoAutoEncoder / md.train_model / md.calculate_anomaly_scores         causal_anomaly_detection1.py
   me.CausalAnomalyDetector / me.predict_anomaly_for_clip / me.score_windows  avenue_training_script_bbox.py
   train.train_improved_minicausal_vad (s2:339-468 driver with real resume, async checkpoints, history JSON)

@@ -6,8 +6,9 @@
 //   masked_mean      vad:398-399  score.mean() over the clip's tracks
 //   ma0_loss         vad:516-531  MSE(scores, labels) + 0.001 * (sum of finite KL terms / number of finite KL terms), with gradients
 //   window_features  streaming sliding-window inference: gathers (n_windows, T, F) clips out of a ring of per-frame features
-//   stream cursor    the same ring driven by a device-side cursor {frames pushed, next window}, so that one captured CUDA graph serves
-//                    every push of a given size: ring_write, window_features_cursor, then cursor_advance (stream-ordered after both)
+//   streams          S rings driven by device-side cursors {frames pushed, next window} and a per-push descriptor {count, reset}, so
+//                    that one captured CUDA graph serves every push of a given size for all streams at once: ring_write,
+//                    window_features, then cursor_advance (stream-ordered after both)
 #include "common.cuh"
 #include "cvad_b200.h"
 
@@ -180,38 +181,69 @@ __global__ void window_features_kernel(const float4* __restrict__ ring, long lon
   }
 }
 
-// ring[(cursor[0] + r) % cap][:] = feats[r][:] for r < n
-__global__ void ring_write_kernel(const float4* __restrict__ feats, long long n, int F4, float4* __restrict__ ring, long long cap,
-                                  const long long* __restrict__ cursor) {
+// The window rule of S streams that share one push (bbox:392-430 as a service, one stream per camera or video).  Stream k's cursor
+// cursors[k] = {frames pushed, next window}; its entry of the push descriptor push[k] = {count, reset}:
+//   base   = reset ? 0 : cursors[k][0]        frames   = base + count
+//   next   = reset ? 0 : cursors[k][1]        n_win    = frames >= T ? (frames - T) / stride + 1 - next : 0
+// infer.window_count is the host's copy of this rule.
+struct StreamPush {
+  long long base, next, frames, n_win;
+};
+
+__device__ __forceinline__ StreamPush stream_push(const long long* __restrict__ cursors, const long long* __restrict__ push, int k, int T,
+                                                  int stride) {
+  const bool reset = push[2 * k + 1] != 0;
+  StreamPush p;
+  p.base = reset ? 0 : cursors[2 * k];
+  p.next = reset ? 0 : cursors[2 * k + 1];
+  p.frames = p.base + push[2 * k];
+  p.n_win = p.frames >= T ? (p.frames - T) / stride + 1 - p.next : 0;
+  return p;
+}
+
+// rings[k][(base_k + r) % cap][:] = feats[k*n + r][:] for r < count_k; rows r >= count_k are not read
+__global__ void streams_ring_write_kernel(const float4* __restrict__ feats, int S, long long n, int F4, float4* __restrict__ rings, long long cap,
+                                          int T, int stride, const long long* __restrict__ cursors, const long long* __restrict__ push) {
   cvad_pdl_enter();
-  const long long pos = cursor[0] % cap, total = n * F4;
+  const long long total = S * n * F4;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-    const long long r = i / F4;
-    const long long fr = (pos + r) % cap;
-    ring[fr * F4 + (i - r * F4)] = __ldg(feats + i);
+    const long long row = i / F4;
+    const int k = (int)(row / n);
+    const long long r = row - k * n;
+    if (r >= push[2 * k]) continue;
+    const StreamPush p = stream_push(cursors, push, k, T, stride);
+    const long long fr = (p.base + r) % cap;
+    rings[(k * cap + fr) * F4 + (i - row * F4)] = __ldg(feats + i);
   }
 }
 
-// window_features_kernel with first = cursor[1] * stride
-__global__ void window_features_cursor_kernel(const float4* __restrict__ ring, long long cap, int stride, int T, int F4, long long n_win,
-                                              const long long* __restrict__ cursor, float4* __restrict__ out) {
+// out[k*m + j][t][:] = rings[k][((next_k + j)*stride + t) % cap][:] for j < n_win_k, zeros for the unused slots j >= n_win_k
+__global__ void streams_window_features_kernel(const float4* __restrict__ rings, int S, long long cap, int stride, int T, int F4, long long m,
+                                               const long long* __restrict__ cursors, const long long* __restrict__ push, float4* __restrict__ out) {
   cvad_pdl_enter();
-  const long long first = cursor[1] * stride;
-  const long long total = n_win * T * F4;
+  const long long total = S * m * T * F4;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const int v = (int)(i % F4);
-    const long long wt = i / F4;
-    const int t = (int)(wt % T);
-    const long long w = wt / T;
-    const long long fr = (first + w * stride + t) % cap;
-    out[i] = __ldg(ring + fr * F4 + v);
+    const long long st = i / F4;
+    const int t = (int)(st % T);
+    const long long slot = st / T;
+    const int k = (int)(slot / m);
+    const long long j = slot - k * m;
+    const StreamPush p = stream_push(cursors, push, k, T, stride);
+    float4 x = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (j < p.n_win) x = __ldg(rings + (k * cap + ((p.next + j) * stride + t) % cap) * F4 + v);
+    out[i] = x;
   }
 }
 
-__global__ void stream_cursor_advance_kernel(long long* cursor, long long n, long long n_win) {
+// cursors[k] = {frames_k, next_k + n_win_k}
+__global__ void streams_cursor_advance_kernel(long long* __restrict__ cursors, int S, int T, int stride, const long long* __restrict__ push) {
   cvad_pdl_enter();
-  cursor[0] += n;
-  cursor[1] += n_win;
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < S; k += gridDim.x * blockDim.x) {
+    const StreamPush p = stream_push(cursors, push, k, T, stride);
+    cursors[2 * k] = p.frames;
+    cursors[2 * k + 1] = p.next + p.n_win;
+  }
 }
 
 inline int blocks_of(long long n) {
@@ -284,28 +316,31 @@ CVAD_API int cvad_window_features_f32(const float* ring, long long capacity, lon
   return 0;
 }
 
-CVAD_API int cvad_ring_write_f32(const float* feats, long long n, int F, float* ring, long long capacity, const long long* cursor, void* stream) {
-  if (n <= 0) return 0;
-  if (F % 4 || capacity <= 0 || n > capacity || !cursor) return (int)cudaErrorInvalidValue;
-  cvad_launch_pdl(ring_write_kernel, dim3(blocks_of(n * (F / 4))), dim3(256), 0, (cudaStream_t)stream, reinterpret_cast<const float4*>(feats), n,
-                  F / 4, reinterpret_cast<float4*>(ring), capacity, cursor);
+CVAD_API int cvad_streams_ring_write_f32(const float* feats, int S, long long n, int F, float* rings, long long capacity, int T, int stride,
+                                         const long long* cursors, const long long* push, void* stream) {
+  if (F % 4 || capacity <= 0 || S <= 0 || n < 0 || T <= 0 || stride <= 0 || !feats || !rings || !cursors || !push)
+    return (int)cudaErrorInvalidValue;
+  if (n == 0) return 0;
+  cvad_launch_pdl(streams_ring_write_kernel, dim3(blocks_of(S * n * (F / 4))), dim3(256), 0, (cudaStream_t)stream,
+                  reinterpret_cast<const float4*>(feats), S, n, F / 4, reinterpret_cast<float4*>(rings), capacity, T, stride, cursors, push);
   CVAD_LAUNCH_CHECK();
   return 0;
 }
 
-CVAD_API int cvad_window_features_cursor_f32(const float* ring, long long capacity, int stride, int T, int F, long long n_windows,
-                                             const long long* cursor, float* out, void* stream) {
-  if (n_windows <= 0) return 0;
-  if (F % 4 || capacity <= 0 || stride <= 0 || T <= 0 || !cursor) return (int)cudaErrorInvalidValue;
-  cvad_launch_pdl(window_features_cursor_kernel, dim3(blocks_of(n_windows * T * (F / 4))), dim3(256), 0, (cudaStream_t)stream,
-                  reinterpret_cast<const float4*>(ring), capacity, stride, T, F / 4, n_windows, cursor, reinterpret_cast<float4*>(out));
+CVAD_API int cvad_streams_window_features_f32(const float* rings, int S, long long capacity, int stride, int T, int F, long long m,
+                                              const long long* cursors, const long long* push, float* out, void* stream) {
+  if (F % 4 || capacity <= 0 || S <= 0 || m < 0 || T <= 0 || stride <= 0 || !rings || !cursors || !push || !out)
+    return (int)cudaErrorInvalidValue;
+  if (m == 0) return 0;
+  cvad_launch_pdl(streams_window_features_kernel, dim3(blocks_of(S * m * T * (F / 4))), dim3(256), 0, (cudaStream_t)stream,
+                  reinterpret_cast<const float4*>(rings), S, capacity, stride, T, F / 4, m, cursors, push, reinterpret_cast<float4*>(out));
   CVAD_LAUNCH_CHECK();
   return 0;
 }
 
-CVAD_API int cvad_stream_cursor_advance(long long* cursor, long long n, long long n_windows, void* stream) {
-  if (!cursor || n < 0 || n_windows < 0) return (int)cudaErrorInvalidValue;
-  cvad_launch_pdl(stream_cursor_advance_kernel, dim3(1), dim3(1), 0, (cudaStream_t)stream, cursor, n, n_windows);
+CVAD_API int cvad_streams_cursor_advance(long long* cursors, int S, int T, int stride, const long long* push, void* stream) {
+  if (S <= 0 || T <= 0 || stride <= 0 || !cursors || !push) return (int)cudaErrorInvalidValue;
+  cvad_launch_pdl(streams_cursor_advance_kernel, dim3(blocks_of(S)), dim3(256), 0, (cudaStream_t)stream, cursors, S, T, stride, push);
   CVAD_LAUNCH_CHECK();
   return 0;
 }

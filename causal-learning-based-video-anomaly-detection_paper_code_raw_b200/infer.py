@@ -11,8 +11,9 @@ layout the next layer reads.  Per call:
 reads every convolution output back from HBM).  The numbers differ from that path in the last bits of bf16: the folded weights are
 rounded as bf16(w*s) instead of bf16(w) followed by an fp32 affine map, and the pre-activation is not rounded to bf16 before the ReLU.
 
-``GraphedStreamingScorer`` is ``ma0.StreamingWindowScorer`` with every push of a given size replayed as one CUDA graph: the stream's
-position lives in a device-side cursor, so the same graph serves every push of that size.
+``MultiStreamScorer`` is ``ma0.StreamingWindowScorer`` for S streams at once with every push of a given size replayed as one CUDA graph:
+each stream's position lives in a device-side cursor and each push carries a small descriptor (frames kept, start over) per stream, so
+the same graph serves every push of that size whatever the streams' phases.  ``GraphedStreamingScorer`` is its one-stream case.
 """
 from __future__ import annotations
 
@@ -134,64 +135,105 @@ class FrozenBackbone:
         return feats.reshape(n, -1)
 
 
-class GraphedStreamingScorer:
-    """Sliding-window scoring of a frame stream, as ``ma0.StreamingWindowScorer`` (same constructor, ``push`` contract and errors), with
-    each push replayed as one CUDA graph.
+def window_count(n_frames, next_window, count, reset, clip_len, stride):
+    """The window rule of one stream for one push (the host's copy of ``stream_push`` in ma0_tail.cu): a stream that has seen
+    ``n_frames`` frames and scored windows [0, ``next_window``) receives ``count`` frames (after starting over at frame 0 when ``reset``).
+    Window w covers frames w*stride + [0, clip_len).  Returns (frames seen after the push, windows the push completes)."""
+    base, nxt = (0, 0) if reset else (n_frames, next_window)
+    frames = base + count
+    return frames, ((frames - clip_len) // stride + 1 - nxt if frames >= clip_len else 0)
 
-    A push of n frames that completes n_win windows runs: copy into a static input -> ``FrozenBackbone`` -> write the n feature rows into
-    the ring at the device cursor -> gather the n_win windows -> ``model.tail`` -> advance the cursor.  Each distinct
-    (n, n_win, H, W, dtype) is captured once (all graphs of one scorer share one memory pool); later pushes of it replay the graph.  The
-    graphs read the model's live tensors, so in-place weight updates need nothing; a model tensor replaced by a new one (a new
-    ``data_ptr``) drops the graphs, which are captured again.  Use it for a fixed chunk size and a model that is frozen or updated in
-    place; a stream of ever-changing chunk sizes pays one capture per new size."""
 
-    def __init__(self, model, clip_len=16, stride=4, capacity=256):
+class MultiStreamScorer:
+    """Sliding-window scoring of S frame streams (cameras, or the videos of a test set, bbox:392-430) with one CUDA graph replay per push
+    for all of them.  Each stream gets exactly the windows and scores it would get from its own ``GraphedStreamingScorer``.
+
+    ``push(frames, counts)`` takes n new frames per stream, of which stream k keeps the first ``counts[k]``, and runs: copy into static
+    inputs -> ``FrozenBackbone`` over all S*n frames -> write each stream's kept feature rows into its ring at its device cursor -> gather
+    the windows each stream completed (m slots per stream, m = the most any stream completed; unused slots are zeros) -> ``model.tail``
+    over the S*m slots -> advance the cursors.  The counts and the streams to start over (``reset``) travel in a small per-push descriptor
+    that is a static input of the graph, so raggedness does not capture again: the graph key is (n, m, H, W, dtype), and since a stream
+    completes at most ceil(n / stride) windows in a push, a scorer holds at most ceil(n / stride) + 1 graphs per push size.  The host
+    mirrors every cursor (``n_frames``, ``next_window``) with ``window_count``, so it knows m and each stream's part of the output
+    without a device sync.  Graphs share one memory pool, read the model's live tensors (in-place weight updates need nothing) and are
+    dropped when a model tensor is replaced by a new one."""
+
+    def __init__(self, model, streams, clip_len=16, stride=4, capacity=64):
         if model.training:
-            raise RuntimeError("GraphedStreamingScorer needs model.eval(): train-mode BatchNorm couples the frames of a batch")
+            raise RuntimeError(f"{type(self).__name__} needs model.eval(): train-mode BatchNorm couples the frames of a batch")
         if capacity < clip_len + stride:
             raise ValueError("ring capacity must hold at least one window plus one stride of new frames")
-        self.model, self.clip_len, self.stride, self.capacity = model, int(clip_len), int(stride), int(capacity)
+        if streams < 1:
+            raise ValueError("a scorer needs at least one stream")
+        self.model, self.streams = model, int(streams)
+        self.clip_len, self.stride, self.capacity = int(clip_len), int(stride), int(capacity)
         self.frozen = None
-        self.ring = None            # (capacity, F) fp32 on the model's device
-        self.cursor = None          # int64 {frames pushed, next window} on the device: what the graphs read
-        self.n_frames = 0           # host mirrors of the cursor: they decide n_win and the graph key
-        self.next_window = 0
-        self.graphs = {}            # (n, n_win, H, W, dtype) -> GraphedStep
+        self.rings = None           # (S, capacity, F) fp32 on the model's device
+        self.cursors = None         # (S, 2) int64 {frames pushed, next window} per stream on the device: what the graphs read
+        self._n_frames = [0] * self.streams          # host mirrors of the cursors: they decide m, the output slices and the graph key
+        self._next_window = [0] * self.streams
+        self._reset = [False] * self.streams         # streams the next push starts over
+        self.graphs = {}            # (n, m, H, W, dtype) -> GraphedStep
         self.pool = None
         self._ptrs = None
+
+    @property
+    def n_frames(self):
+        """Frames each stream has pushed since its last start."""
+        return list(self._n_frames)
+
+    @property
+    def next_window(self):
+        """Index of each stream's next window."""
+        return list(self._next_window)
+
+    def reset(self, k):
+        """Start stream k over (a new video on that camera): the next push writes its frames from frame 0 and window 0 on."""
+        if not 0 <= k < self.streams:
+            raise IndexError(f"stream {k} out of range for {self.streams} streams")
+        self._n_frames[k] = self._next_window[k] = 0
+        self._reset[k] = True
 
     def _model_ptrs(self):
         return [t.data_ptr() for t in list(self.model.parameters()) + list(self.model.buffers())]
 
-    def _step(self, n, n_win):
-        model, F = self.model, self.ring.shape[1]
+    def _step(self, n, m):
+        model, S, T, F = self.model, self.streams, self.clip_len, self.rings.shape[2]
 
-        def step(x):
-            feats = self.frozen(x)
+        def step(x, push):
+            feats = self.frozen(x.reshape(S * n, *x.shape[2:]))
             st = _st()
-            _call("cvad_ring_write_f32", _ptr(feats), n, F, _ptr(self.ring), self.capacity, _ptr(self.cursor), st)
-            if n_win > 0:
-                clips = torch.empty((n_win, self.clip_len, F), device=feats.device, dtype=torch.float32)
-                _call("cvad_window_features_cursor_f32", _ptr(self.ring), self.capacity, self.stride, self.clip_len, F, n_win, _ptr(self.cursor),
-                      _ptr(clips), st)
+            _call("cvad_streams_ring_write_f32", _ptr(feats), S, n, F, _ptr(self.rings), self.capacity, T, self.stride, _ptr(self.cursors),
+                  _ptr(push), st)
+            if m > 0:
+                clips = torch.empty((S * m, T, F), device=feats.device, dtype=torch.float32)
+                _call("cvad_streams_window_features_f32", _ptr(self.rings), S, self.capacity, self.stride, T, F, m, _ptr(self.cursors),
+                      _ptr(push), _ptr(clips), st)
                 scores = model.tail(clips)["anomaly_scores"]
             else:
                 scores = torch.empty(0, device=feats.device)
-            _call("cvad_stream_cursor_advance", _ptr(self.cursor), n, n_win, st)
+            _call("cvad_streams_cursor_advance", _ptr(self.cursors), S, T, self.stride, _ptr(push), st)
             return scores
         return step
 
     @torch.no_grad()
-    def push(self, frames):
-        """frames (n,1,H,W) float32 (normalised) or uint8 (the loader's raw frames) on the model's device -> (window scores, first window index)."""
-        if frames.dim() != 4:
-            raise ValueError("expected (n, 1, H, W) frames")
-        n = frames.shape[0]
-        if n > self.capacity - self.clip_len:
+    def push(self, frames, counts=None):
+        """frames (S,n,1,H,W) float32 (normalised) or uint8 (the loader's raw frames) on the model's device; counts: S ints in [0, n], the
+        frames each stream keeps (default n; the rows beyond a count are computed and discarded, so they must hold finite frames).
+        Returns one (window scores, first window index) pair per stream; a stream's scores may be empty."""
+        if frames.dim() != 5:
+            raise ValueError("expected (S, n, 1, H, W) frames")
+        S, n = self.streams, frames.shape[1]
+        if frames.shape[0] != S:
+            raise ValueError(f"expected frames of {S} streams, got {frames.shape[0]}")
+        counts = [n] * S if counts is None else [int(c) for c in counts]
+        if len(counts) != S or not all(0 <= c <= n for c in counts):
+            raise ValueError(f"counts must be {S} ints in [0, {n}]")
+        if max(counts) > self.capacity - self.clip_len:
             raise ValueError("more new frames than the ring can take while it still holds an open window")
         ops._cuda(frames)
         if self.model.training:
-            raise RuntimeError("GraphedStreamingScorer needs model.eval(): train-mode BatchNorm couples the frames of a batch")
+            raise RuntimeError(f"{type(self).__name__} needs model.eval(): train-mode BatchNorm couples the frames of a batch")
         bb = self.model.backbone
         if self.frozen is None or self.frozen.backbone is not bb:
             self.frozen = FrozenBackbone(bb)
@@ -202,25 +244,50 @@ class GraphedStreamingScorer:
             self.graphs.clear()
             self._ptrs = ptrs
         dev = frames.device
-        if self.ring is None:
+        if self.rings is None:
             F = bb.layer4[3].out_channels * 4 * 6
-            self.ring = torch.zeros((self.capacity, F), device=dev, dtype=torch.float32)
-            self.cursor = torch.zeros(2, device=dev, dtype=torch.int64)
+            self.rings = torch.zeros((S, self.capacity, F), device=dev, dtype=torch.float32)
+            self.cursors = torch.zeros((S, 2), device=dev, dtype=torch.int64)
             self.pool = torch.cuda.graph_pool_handle()
-        n_frames = self.n_frames + n
-        n_win = 0
-        if n_frames >= self.clip_len:
-            n_win = (n_frames - self.clip_len) // self.stride + 1 - self.next_window
-        w0 = self.next_window
-        if n == 0:
-            return torch.empty(0, device=dev), w0
-        key = (n, max(n_win, 0), frames.shape[2], frames.shape[3], frames.dtype)
+        w0 = list(self._next_window)
+        if not any(counts):         # nothing to write; pending resets reach the device with the next push
+            empty = torch.empty(0, device=dev)
+            return [(empty, w) for w in w0]
+        wins = [window_count(self._n_frames[k], self._next_window[k], counts[k], self._reset[k], self.clip_len, self.stride) for k in range(S)]
+        m = max(nw for _, nw in wins)
+        push = torch.tensor([[c, int(r)] for c, r in zip(counts, self._reset)], dtype=torch.int64)
+        key = (n, m, frames.shape[3], frames.shape[4], frames.dtype)
         g = self.graphs.get(key)
         if g is None:
-            self.frozen._buffers(n, frames.shape[2], frames.shape[3], dev)      # allocated and zeroed outside the capture
-            # warm-up runs the step for real: the ring and the cursor are restored after it, so capturing does not advance the stream
-            g = self.graphs[key] = GraphedStep(self._step(n, key[1]), (frames,), mutated=(self.ring, self.cursor), pool=self.pool)
-        (scores,) = g(frames)
-        self.n_frames = n_frames
-        self.next_window += key[1]
-        return scores.clone(), w0
+            self.frozen._buffers(S * n, frames.shape[3], frames.shape[4], dev)      # allocated and zeroed outside the capture
+            # warm-up runs the step for real: the rings and the cursors are restored after it, so capturing does not advance the streams
+            g = self.graphs[key] = GraphedStep(self._step(n, m), (frames, push), mutated=(self.rings, self.cursors), pool=self.pool)
+        (scores,) = g(frames, push)
+        for k, (fr, nw) in enumerate(wins):
+            self._n_frames[k] = fr
+            self._next_window[k] += nw
+        self._reset = [False] * S
+        out = scores.clone()
+        return [(out[k * m:k * m + nw], w0[k]) for k, (_, nw) in enumerate(wins)]
+
+
+class GraphedStreamingScorer(MultiStreamScorer):
+    """Sliding-window scoring of one frame stream, as ``ma0.StreamingWindowScorer`` (same constructor, ``push`` contract and errors), with
+    each push replayed as one CUDA graph: ``MultiStreamScorer`` with one stream.  Each distinct (n, n_win, H, W, dtype) is captured once.
+    Use it for a fixed chunk size and a model that is frozen or updated in place; a stream of ever-changing chunk sizes pays one capture
+    per new size."""
+
+    def __init__(self, model, clip_len=16, stride=4, capacity=256):
+        super().__init__(model, 1, clip_len, stride, capacity)
+
+    ring = property(lambda self: None if self.rings is None else self.rings[0], doc="(capacity, F) fp32 ring on the model's device")
+    cursor = property(lambda self: None if self.cursors is None else self.cursors[0], doc="int64 {frames pushed, next window} on the device")
+    n_frames = property(lambda self: self._n_frames[0], doc="frames pushed so far")
+    next_window = property(lambda self: self._next_window[0], doc="index of the next window")
+
+    def push(self, frames):
+        """frames (n,1,H,W) float32 (normalised) or uint8 (the loader's raw frames) on the model's device -> (window scores, first window index)."""
+        if frames.dim() != 4:
+            raise ValueError("expected (n, 1, H, W) frames")
+        [(scores, w0)] = super().push(frames.unsqueeze(0))
+        return scores, w0

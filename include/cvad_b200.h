@@ -145,13 +145,20 @@ int cvad_ma0_loss_f32(const float* scores, const float* kl, const long long* lab
  * `capacity` frames x F floats; out (n_windows, T, F) gathers window w = frames first_frame + w*stride + [0,T) (indices modulo capacity) */
 int cvad_window_features_f32(const float* ring, long long capacity, long long first_frame, int stride, int T, int F, long long n_windows,
                              float* out, void* stream);
-/* The same ring driven by a device-side cursor[2] = {frames pushed, next window}, so that a captured CUDA graph serves every push of one
- * size: ring_write puts feats (n, F) at ring rows (cursor[0] + [0,n)) % capacity; window_features_cursor is cvad_window_features_f32 with
- * first_frame = cursor[1] * stride; cursor_advance adds (n, n_windows) to the cursor (issue it after the other two, on the same stream). */
-int cvad_ring_write_f32(const float* feats, long long n, int F, float* ring, long long capacity, const long long* cursor, void* stream);
-int cvad_window_features_cursor_f32(const float* ring, long long capacity, int stride, int T, int F, long long n_windows,
-                                    const long long* cursor, float* out, void* stream);
-int cvad_stream_cursor_advance(long long* cursor, long long n, long long n_windows, void* stream);
+/* S frame streams sharing one push (bbox:392-430 scores a test set video by video; a deployment serves many cameras), so that one captured
+ * CUDA graph serves every push of a given size for all of them.  rings (S, capacity, F) fp32; cursors (S, 2) int64 on the device, row k =
+ * {frames pushed, next window} of stream k; push (S, 2) int64 on the device, row k = {count_k in [0, n], reset_k}.  Window rule, per stream:
+ *   base_k = reset_k ? 0 : cursors[k][0]     next_k = reset_k ? 0 : cursors[k][1]     frames_k = base_k + count_k
+ *   n_win_k = frames_k >= T ? (frames_k - T) / stride + 1 - next_k : 0
+ * ring_write: feats (S*n, F), stream-major; row r < count_k of stream k goes to rings[k][(base_k + r) % capacity], rows r >= count_k
+ * are not read.  window_features: out (S*m, T, F); slot (k, j) holds window next_k + j of stream k (frames (next_k + j)*stride + [0,T)
+ * modulo capacity) when j < n_win_k, zeros otherwise.  cursor_advance: cursors[k] = {frames_k, next_k + n_win_k}; issue it after the
+ * other two, on the same stream. */
+int cvad_streams_ring_write_f32(const float* feats, int S, long long n, int F, float* rings, long long capacity, int T, int stride,
+                                const long long* cursors, const long long* push, void* stream);
+int cvad_streams_window_features_f32(const float* rings, int S, long long capacity, int stride, int T, int F, long long m,
+                                     const long long* cursors, const long long* push, float* out, void* stream);
+int cvad_streams_cursor_advance(long long* cursors, int S, int T, int stride, const long long* push, void* stream);
 
 /* ---- M-A causal branch, dense masked batched form (ma_tail.cu) -------------------------------------------------------
  * Every clip carries 5 padded track slots (the detector emits <= 5 boxes per frame, cad:178,198) and a per-clip track
