@@ -89,6 +89,27 @@ static inline void fast_div_init(unsigned d, unsigned& mul, unsigned& shr) {
 }
 __device__ __forceinline__ int fast_div(int x, unsigned mul, unsigned shr) { return mul ? (int)(__umulhi((unsigned)x, mul) >> shr) : x; }
 
+// The window rule of S streams that share one push (bbox:392-430 as a service, one stream per camera or video), shared by the feature
+// rings of ma0_tail.cu and the frame rings of frames.cu.  Stream k's cursor cursors[k] = {frames pushed, next window}; its entry of the
+// push descriptor push[k] = {count, reset}:
+//   base   = reset ? 0 : cursors[k][0]        frames   = base + count
+//   next   = reset ? 0 : cursors[k][1]        n_win    = frames >= T ? (frames - T) / stride + 1 - next : 0
+// infer.window_count is the host's copy of this rule.
+struct StreamPush {
+  long long base, next, frames, n_win;
+};
+
+__device__ __forceinline__ StreamPush stream_push(const long long* __restrict__ cursors, const long long* __restrict__ push, int k, int T,
+                                                  int stride) {
+  const bool reset = push[2 * k + 1] != 0;
+  StreamPush p;
+  p.base = reset ? 0 : cursors[2 * k];
+  p.next = reset ? 0 : cursors[2 * k + 1];
+  p.frames = p.base + push[2 * k];
+  p.n_win = p.frames >= T ? (p.frames - T) / stride + 1 - p.next : 0;
+  return p;
+}
+
 static inline bool cvad_pdl_enabled() {
   static int on = -1;
   if (on < 0) {

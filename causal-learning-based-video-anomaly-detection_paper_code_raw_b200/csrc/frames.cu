@@ -33,6 +33,23 @@ __device__ __forceinline__ Tap make_tap(int d, int src, double scale, bool zero_
   return t;
 }
 
+// cv2.resize(INTER_LINEAR) of pixel (dx, dy) of frame `frame` of src (.., sh, sw, C) into pixel `pix` of dst (.., C): the taps, then the
+// fixed-point blend.
+__device__ __forceinline__ void resize_pixel_u8(const uint8_t* src, long long frame, int sh, int sw, int C, int dx, int dy, double scale_x,
+                                                double scale_y, uint8_t* dst, long long pix) {
+  const Tap tx = make_tap(dx, sw, scale_x, true), ty = make_tap(dy, sh, scale_y, false);
+  const uint8_t* f = src + frame * sh * sw * C;
+  const uint8_t* r0 = f + (long long)ty.i0 * sw * C;
+  const uint8_t* r1 = f + (long long)ty.i1 * sw * C;
+  uint8_t* o = dst + pix * C;
+  for (int c = 0; c < C; ++c) {
+    const int s0 = (int)__ldg(r0 + tx.i0 * C + c) * tx.w0 + (int)__ldg(r0 + tx.i1 * C + c) * tx.w1;
+    const int s1 = (int)__ldg(r1 + tx.i0 * C + c) * tx.w0 + (int)__ldg(r1 + tx.i1 * C + c) * tx.w1;
+    const int v = (((ty.w0 * (s0 >> 4)) >> 16) + ((ty.w1 * (s1 >> 4)) >> 16) + 2) >> 2;
+    o[c] = (uint8_t)min(max(v, 0), 255);
+  }
+}
+
 // src (N, sh, sw, C) uint8 interleaved -> dst (N, dh, dw, C) uint8
 __global__ void resize_bilinear_u8_kernel(const uint8_t* __restrict__ src, int N, int sh, int sw, int C, uint8_t* __restrict__ dst, int dh, int dw,
                                           double scale_x, double scale_y) {
@@ -41,17 +58,57 @@ __global__ void resize_bilinear_u8_kernel(const uint8_t* __restrict__ src, int N
     const int dx = (int)(t % dw);
     const long long r = t / dw;
     const int dy = (int)(r % dh), n = (int)(r / dh);
-    const Tap tx = make_tap(dx, sw, scale_x, true), ty = make_tap(dy, sh, scale_y, false);
-    const uint8_t* f = src + (long long)n * sh * sw * C;
-    const uint8_t* r0 = f + (long long)ty.i0 * sw * C;
-    const uint8_t* r1 = f + (long long)ty.i1 * sw * C;
-    uint8_t* o = dst + t * C;
-    for (int c = 0; c < C; ++c) {
-      const int s0 = (int)__ldg(r0 + tx.i0 * C + c) * tx.w0 + (int)__ldg(r0 + tx.i1 * C + c) * tx.w1;
-      const int s1 = (int)__ldg(r1 + tx.i0 * C + c) * tx.w0 + (int)__ldg(r1 + tx.i1 * C + c) * tx.w1;
-      const int v = (((ty.w0 * (s0 >> 4)) >> 16) + ((ty.w1 * (s1 >> 4)) >> 16) + 2) >> 2;
-      o[c] = (uint8_t)min(max(v, 0), 255);
+    resize_pixel_u8(src, n, sh, sw, C, dx, dy, scale_x, scale_y, dst, t);
+  }
+}
+
+// Frame rings of S streams (the window rule is stream_push, common.cuh).  src (S*n, sh, sw, C), stream-major: row r < count_k of stream k
+// is resized to (dh, dw) into rings[k][(base_k + r) % cap] (rings (S, cap, dh, dw, C)); rows r >= count_k are not read.  At the ring's
+// own size the resize rule is the identity and the frame is copied.
+__global__ void streams_frame_write_u8_kernel(const uint8_t* __restrict__ src, int S, long long n, int sh, int sw, int C, uint8_t* __restrict__ rings,
+                                              long long cap, int dh, int dw, int T, int stride, const long long* __restrict__ cursors,
+                                              const long long* __restrict__ push, double scale_x, double scale_y) {
+  const long long hw = (long long)dh * dw;
+  const long long total = S * n * hw;
+  const bool copy = sh == dh && sw == dw;
+  for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
+    const long long row = t / hw, p = t - row * hw;
+    const int k = (int)(row / n);
+    const long long r = row - k * n;
+    if (r >= push[2 * k]) continue;
+    const StreamPush sp = stream_push(cursors, push, k, T, stride);
+    const long long pix = (k * cap + (sp.base + r) % cap) * hw + p;
+    if (copy) {
+      for (int c = 0; c < C; ++c) rings[pix * C + c] = __ldg(src + t * C + c);
+    } else {
+      resize_pixel_u8(src, row, sh, sw, C, (int)(p % dw), (int)(p / dw), scale_x, scale_y, rings, pix);
     }
+  }
+}
+
+// out (S*m, C, T, H, W) fp32: slot (k, j) = window next_k + j of stream k, frames ((next_k + j)*stride + [0, T)) % cap of its ring, as
+// value * scale with channel C-1-c read for c when reverse_channels (the element rule of clips_from_frames_kernel); zeros for j >= n_win_k
+__global__ void streams_clips_f32_kernel(const uint8_t* __restrict__ rings, int S, long long cap, int H, int W, int C, int T, int stride, long long m,
+                                         const long long* __restrict__ cursors, const long long* __restrict__ push, float scale, int reverse_channels,
+                                         float* __restrict__ out) {
+  const long long hw = (long long)H * W;
+  const long long total = S * m * C * T * hw;
+  for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
+    const long long p = t % hw;
+    long long r = t / hw;
+    const int tt = (int)(r % T); r /= T;
+    const int c = (int)(r % C);
+    const long long slot = r / C;
+    const int k = (int)(slot / m);
+    const long long j = slot - k * m;
+    const StreamPush sp = stream_push(cursors, push, k, T, stride);
+    float v = 0.f;
+    if (j < sp.n_win) {
+      const long long fr = ((sp.next + j) * stride + tt) % cap;
+      const int cs = reverse_channels ? C - 1 - c : c;
+      v = (float)__ldg(rings + ((k * cap + fr) * hw + p) * C + cs) * scale;
+    }
+    out[t] = v;
   }
 }
 
@@ -95,15 +152,16 @@ inline unsigned frame_blocks(long long n) {
   return (unsigned)b;
 }
 
+// OpenCV: inv_scale = dsize / ssize (double); scale = 1. / inv_scale
+inline double cv2_scale(int dst, int src) { return 1.0 / ((double)dst / src); }
+
 }  // namespace
 
 CVAD_API int cvad_resize_bilinear_u8(const void* src, int N, int src_h, int src_w, int C, void* dst, int dst_h, int dst_w, void* stream) {
   if (N <= 0) return 0;
   if (src_h <= 0 || src_w <= 0 || dst_h <= 0 || dst_w <= 0 || C < 1 || C > 4) return (int)cudaErrorInvalidValue;
-  // OpenCV: inv_scale = dsize / ssize (double); scale = 1. / inv_scale
-  const double scale_x = 1.0 / ((double)dst_w / src_w), scale_y = 1.0 / ((double)dst_h / src_h);
-  resize_bilinear_u8_kernel<<<frame_blocks((long long)N * dst_h * dst_w), 256, 0, (cudaStream_t)stream>>>((const uint8_t*)src, N, src_h, src_w, C,
-                                                                                                         (uint8_t*)dst, dst_h, dst_w, scale_x, scale_y);
+  resize_bilinear_u8_kernel<<<frame_blocks((long long)N * dst_h * dst_w), 256, 0, (cudaStream_t)stream>>>(
+      (const uint8_t*)src, N, src_h, src_w, C, (uint8_t*)dst, dst_h, dst_w, cv2_scale(dst_w, src_w), cv2_scale(dst_h, src_h));
   CVAD_LAUNCH_CHECK();
   return 0;
 }
@@ -124,6 +182,30 @@ CVAD_API int cvad_clips_from_frames_u8(const void* frames, int F, int H, int W, 
   if (F <= 0 || H <= 0 || W <= 0) return (int)cudaErrorInvalidValue;
   clips_from_frames_u8_kernel<<<frame_blocks((long long)B * T * H * W), 256, 0, (cudaStream_t)stream>>>((const uint8_t*)frames, F, (long long)H * W, starts,
                                                                                                       B, T, frame_stride, (uint8_t*)out);
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
+CVAD_API int cvad_streams_frame_write_u8(const void* src, int S, long long n, int src_h, int src_w, int C, void* rings, long long capacity, int dst_h,
+                                         int dst_w, int T, int stride, const long long* cursors, const long long* push, void* stream) {
+  if (!src || !rings || !cursors || !push || S <= 0 || n < 0 || capacity <= 0 || T <= 0 || stride <= 0 || src_h <= 0 || src_w <= 0 || dst_h <= 0 ||
+      dst_w <= 0 || C < 1 || C > 4)
+    return (int)cudaErrorInvalidValue;
+  if (n == 0) return 0;
+  streams_frame_write_u8_kernel<<<frame_blocks(S * n * dst_h * dst_w), 256, 0, (cudaStream_t)stream>>>(
+      (const uint8_t*)src, S, n, src_h, src_w, C, (uint8_t*)rings, capacity, dst_h, dst_w, T, stride, cursors, push, cv2_scale(dst_w, src_w),
+      cv2_scale(dst_h, src_h));
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
+CVAD_API int cvad_streams_clips_f32(const void* rings, int S, long long capacity, int H, int W, int C, int T, int stride, long long m,
+                                    const long long* cursors, const long long* push, float scale, int reverse_channels, float* out, void* stream) {
+  if (!rings || !cursors || !push || !out || S <= 0 || m < 0 || capacity <= 0 || T <= 0 || stride <= 0 || H <= 0 || W <= 0 || C < 1 || C > 4)
+    return (int)cudaErrorInvalidValue;
+  if (m == 0) return 0;
+  streams_clips_f32_kernel<<<frame_blocks(S * m * C * T * H * W), 256, 0, (cudaStream_t)stream>>>(
+      (const uint8_t*)rings, S, capacity, H, W, C, T, stride, m, cursors, push, scale, reverse_channels, out);
   CVAD_LAUNCH_CHECK();
   return 0;
 }

@@ -8,7 +8,7 @@
 //   window_features  streaming sliding-window inference: gathers (n_windows, T, F) clips out of a ring of per-frame features
 //   streams          S rings driven by device-side cursors {frames pushed, next window} and a per-push descriptor {count, reset}, so
 //                    that one captured CUDA graph serves every push of a given size for all streams at once: ring_write,
-//                    window_features, then cursor_advance (stream-ordered after both)
+//                    window_features, then cursor_advance (stream-ordered after both); the window rule is stream_push (common.cuh)
 #include "common.cuh"
 #include "cvad_b200.h"
 
@@ -179,26 +179,6 @@ __global__ void window_features_kernel(const float4* __restrict__ ring, long lon
     const long long fr = (first + w * stride + t) % cap;
     out[i] = __ldg(ring + fr * F4 + v);
   }
-}
-
-// The window rule of S streams that share one push (bbox:392-430 as a service, one stream per camera or video).  Stream k's cursor
-// cursors[k] = {frames pushed, next window}; its entry of the push descriptor push[k] = {count, reset}:
-//   base   = reset ? 0 : cursors[k][0]        frames   = base + count
-//   next   = reset ? 0 : cursors[k][1]        n_win    = frames >= T ? (frames - T) / stride + 1 - next : 0
-// infer.window_count is the host's copy of this rule.
-struct StreamPush {
-  long long base, next, frames, n_win;
-};
-
-__device__ __forceinline__ StreamPush stream_push(const long long* __restrict__ cursors, const long long* __restrict__ push, int k, int T,
-                                                  int stride) {
-  const bool reset = push[2 * k + 1] != 0;
-  StreamPush p;
-  p.base = reset ? 0 : cursors[2 * k];
-  p.next = reset ? 0 : cursors[2 * k + 1];
-  p.frames = p.base + push[2 * k];
-  p.n_win = p.frames >= T ? (p.frames - T) / stride + 1 - p.next : 0;
-  return p;
 }
 
 // rings[k][(base_k + r) % cap][:] = feats[k*n + r][:] for r < count_k; rows r >= count_k are not read

@@ -1,4 +1,4 @@
-"""Low-latency inference for the per-frame (2-D backbone) models M-A and M-A0.
+"""Low-latency inference: the per-frame (2-D backbone) models M-A and M-A0, and many camera streams for the 3-D clip models.
 
 ``FrozenBackbone`` is the bf16 tensor-core backbone of tc.py specialised to eval mode.  An eval-mode BatchNorm is a constant per-channel
 affine map, so it is folded into the convolution in front of it once, at snapshot time (w' = w*s, b' = (b - running_mean)*s + beta,
@@ -14,6 +14,10 @@ rounded as bf16(w*s) instead of bf16(w) followed by an fp32 affine map, and the 
 ``MultiStreamScorer`` is ``ma0.StreamingWindowScorer`` for S streams at once with every push of a given size replayed as one CUDA graph:
 each stream's position lives in a device-side cursor and each push carries a small descriptor (frames kept, start over) per stream, so
 the same graph serves every push of that size whatever the streams' phases.  ``GraphedStreamingScorer`` is its one-stream case.
+
+``MultiStreamClipScorer`` is the same service for M-B, M-C and M-E from raw camera frames: the rings hold cv2-resized frames instead of
+features, and every completed window is gathered from them and scored by the model's batched forward.  Both multi-stream scorers share
+their host-side bookkeeping (``_StreamBookkeeping``) and the device window rule (``stream_push``, mirrored by ``window_count``).
 """
 from __future__ import annotations
 
@@ -144,21 +148,14 @@ def window_count(n_frames, next_window, count, reset, clip_len, stride):
     return frames, ((frames - clip_len) // stride + 1 - nxt if frames >= clip_len else 0)
 
 
-class MultiStreamScorer:
-    """Sliding-window scoring of S frame streams (cameras, or the videos of a test set, bbox:392-430) with one CUDA graph replay per push
-    for all of them.  Each stream gets exactly the windows and scores it would get from its own ``GraphedStreamingScorer``.
+class _StreamBookkeeping:
+    """The host side of S streams scored through device rings, shared by ``MultiStreamScorer`` (rings of backbone features) and
+    ``MultiStreamClipScorer`` (rings of frames): constructor checks, push validation, the host mirrors of the device cursors
+    (``window_count``), resets, the per-push descriptor, graph keys and capture, dropping the graphs when a model tensor is replaced, and
+    the per-stream split of the outputs.  A subclass supplies its ring (``_new_ring``), the graph of one push (``_capture``), the outputs of
+    a push that keeps no frame (``_empty``) and, optionally, its own check for replaced tensors (``_refresh``)."""
 
-    ``push(frames, counts)`` takes n new frames per stream, of which stream k keeps the first ``counts[k]``, and runs: copy into static
-    inputs -> ``FrozenBackbone`` over all S*n frames -> write each stream's kept feature rows into its ring at its device cursor -> gather
-    the windows each stream completed (m slots per stream, m = the most any stream completed; unused slots are zeros) -> ``model.tail``
-    over the S*m slots -> advance the cursors.  The counts and the streams to start over (``reset``) travel in a small per-push descriptor
-    that is a static input of the graph, so raggedness does not capture again: the graph key is (n, m, H, W, dtype), and since a stream
-    completes at most ceil(n / stride) windows in a push, a scorer holds at most ceil(n / stride) + 1 graphs per push size.  The host
-    mirrors every cursor (``n_frames``, ``next_window``) with ``window_count``, so it knows m and each stream's part of the output
-    without a device sync.  Graphs share one memory pool, read the model's live tensors (in-place weight updates need nothing) and are
-    dropped when a model tensor is replaced by a new one."""
-
-    def __init__(self, model, streams, clip_len=16, stride=4, capacity=64):
+    def __init__(self, model, streams, clip_len, stride, capacity):
         if model.training:
             raise RuntimeError(f"{type(self).__name__} needs model.eval(): train-mode BatchNorm couples the frames of a batch")
         if capacity < clip_len + stride:
@@ -167,13 +164,12 @@ class MultiStreamScorer:
             raise ValueError("a scorer needs at least one stream")
         self.model, self.streams = model, int(streams)
         self.clip_len, self.stride, self.capacity = int(clip_len), int(stride), int(capacity)
-        self.frozen = None
-        self.rings = None           # (S, capacity, F) fp32 on the model's device
+        self.rings = None           # (S, capacity, ...) on the model's device
         self.cursors = None         # (S, 2) int64 {frames pushed, next window} per stream on the device: what the graphs read
         self._n_frames = [0] * self.streams          # host mirrors of the cursors: they decide m, the output slices and the graph key
         self._next_window = [0] * self.streams
         self._reset = [False] * self.streams         # streams the next push starts over
-        self.graphs = {}            # (n, m, H, W, dtype) -> GraphedStep
+        self.graphs = {}            # (n, m, ...frame key) -> GraphedStep
         self.pool = None
         self._ptrs = None
 
@@ -197,6 +193,83 @@ class MultiStreamScorer:
     def _model_ptrs(self):
         return [t.data_ptr() for t in list(self.model.parameters()) + list(self.model.buffers())]
 
+    def _refresh(self):
+        """Bring derived model state up to date; True when the graphs read tensors that no longer exist."""
+        return False
+
+    def _push(self, frames, counts, frame_key):
+        """frames (S, n, ...) on the device -> per stream (tuple of its rows of every output, first window index)."""
+        S, n = self.streams, frames.shape[1]
+        if frames.shape[0] != S:
+            raise ValueError(f"expected frames of {S} streams, got {frames.shape[0]}")
+        counts = [n] * S if counts is None else [int(c) for c in counts]
+        if len(counts) != S or not all(0 <= c <= n for c in counts):
+            raise ValueError(f"counts must be {S} ints in [0, {n}]")
+        if max(counts) > self.capacity - self.clip_len:
+            raise ValueError("more new frames than the ring can take while it still holds an open window")
+        ops._cuda(frames)
+        if self.model.training:
+            raise RuntimeError(f"{type(self).__name__} needs model.eval(): train-mode BatchNorm couples the frames of a batch")
+        replaced = self._refresh()
+        ptrs = self._model_ptrs()
+        if replaced or ptrs != self._ptrs:
+            self.graphs.clear()
+            self._ptrs = ptrs
+        dev = frames.device
+        if self.rings is None:
+            self.rings = self._new_ring(dev)
+            self.cursors = torch.zeros((S, 2), device=dev, dtype=torch.int64)
+            self.pool = torch.cuda.graph_pool_handle()
+        w0 = list(self._next_window)
+        if not any(counts):         # nothing to write; pending resets reach the device with the next push
+            return [(self._empty(dev), w) for w in w0]
+        wins = [window_count(self._n_frames[k], self._next_window[k], counts[k], self._reset[k], self.clip_len, self.stride) for k in range(S)]
+        m = max(nw for _, nw in wins)
+        push = torch.tensor([[c, int(r)] for c, r in zip(counts, self._reset)], dtype=torch.int64)
+        key = (n, m) + frame_key
+        g = self.graphs.get(key)
+        if g is None:
+            g = self.graphs[key] = self._capture(n, m, frames, push)
+        outs = [o.clone() for o in g(frames, push)]
+        for k, (fr, nw) in enumerate(wins):
+            self._n_frames[k] = fr
+            self._next_window[k] += nw
+        self._reset = [False] * S
+        return [(tuple(o[k * m:k * m + nw] for o in outs), w0[k]) for k, (_, nw) in enumerate(wins)]
+
+
+class MultiStreamScorer(_StreamBookkeeping):
+    """Sliding-window scoring of S frame streams (cameras, or the videos of a test set, bbox:392-430) with one CUDA graph replay per push
+    for all of them.  Each stream gets exactly the windows and scores it would get from its own ``GraphedStreamingScorer``.
+
+    ``push(frames, counts)`` takes n new frames per stream, of which stream k keeps the first ``counts[k]``, and runs: copy into static
+    inputs -> ``FrozenBackbone`` over all S*n frames -> write each stream's kept feature rows into its ring at its device cursor -> gather
+    the windows each stream completed (m slots per stream, m = the most any stream completed; unused slots are zeros) -> ``model.tail``
+    over the S*m slots -> advance the cursors.  The counts and the streams to start over (``reset``) travel in a small per-push descriptor
+    that is a static input of the graph, so raggedness does not capture again: the graph key is (n, m, H, W, dtype), and since a stream
+    completes at most ceil(n / stride) windows in a push, a scorer holds at most ceil(n / stride) + 1 graphs per push size.  The host
+    mirrors every cursor (``n_frames``, ``next_window``) with ``window_count``, so it knows m and each stream's part of the output
+    without a device sync.  Graphs share one memory pool, read the model's live tensors (in-place weight updates need nothing) and are
+    dropped when a model tensor is replaced by a new one."""
+
+    def __init__(self, model, streams, clip_len=16, stride=4, capacity=64):
+        super().__init__(model, streams, clip_len, stride, capacity)
+        self.frozen = None
+
+    def _refresh(self):
+        bb = self.model.backbone
+        new = self.frozen is None or self.frozen.backbone is not bb
+        if new:
+            self.frozen = FrozenBackbone(bb)
+        return self.frozen.refresh() or new
+
+    def _new_ring(self, dev):
+        F = self.model.backbone.layer4[3].out_channels * 4 * 6
+        return torch.zeros((self.streams, self.capacity, F), device=dev, dtype=torch.float32)
+
+    def _empty(self, dev):
+        return (torch.empty(0, device=dev),)
+
     def _step(self, n, m):
         model, S, T, F = self.model, self.streams, self.clip_len, self.rings.shape[2]
 
@@ -216,6 +289,11 @@ class MultiStreamScorer:
             return scores
         return step
 
+    def _capture(self, n, m, frames, push):
+        self.frozen._buffers(self.streams * n, frames.shape[3], frames.shape[4], frames.device)      # allocated and zeroed outside the capture
+        # warm-up runs the step for real: the rings and the cursors are restored after it, so capturing does not advance the streams
+        return GraphedStep(self._step(n, m), (frames, push), mutated=(self.rings, self.cursors), pool=self.pool)
+
     @torch.no_grad()
     def push(self, frames, counts=None):
         """frames (S,n,1,H,W) float32 (normalised) or uint8 (the loader's raw frames) on the model's device; counts: S ints in [0, n], the
@@ -223,52 +301,7 @@ class MultiStreamScorer:
         Returns one (window scores, first window index) pair per stream; a stream's scores may be empty."""
         if frames.dim() != 5:
             raise ValueError("expected (S, n, 1, H, W) frames")
-        S, n = self.streams, frames.shape[1]
-        if frames.shape[0] != S:
-            raise ValueError(f"expected frames of {S} streams, got {frames.shape[0]}")
-        counts = [n] * S if counts is None else [int(c) for c in counts]
-        if len(counts) != S or not all(0 <= c <= n for c in counts):
-            raise ValueError(f"counts must be {S} ints in [0, {n}]")
-        if max(counts) > self.capacity - self.clip_len:
-            raise ValueError("more new frames than the ring can take while it still holds an open window")
-        ops._cuda(frames)
-        if self.model.training:
-            raise RuntimeError(f"{type(self).__name__} needs model.eval(): train-mode BatchNorm couples the frames of a batch")
-        bb = self.model.backbone
-        if self.frozen is None or self.frozen.backbone is not bb:
-            self.frozen = FrozenBackbone(bb)
-            self.graphs.clear()
-        replaced = self.frozen.refresh()
-        ptrs = self._model_ptrs()
-        if replaced or ptrs != self._ptrs:
-            self.graphs.clear()
-            self._ptrs = ptrs
-        dev = frames.device
-        if self.rings is None:
-            F = bb.layer4[3].out_channels * 4 * 6
-            self.rings = torch.zeros((S, self.capacity, F), device=dev, dtype=torch.float32)
-            self.cursors = torch.zeros((S, 2), device=dev, dtype=torch.int64)
-            self.pool = torch.cuda.graph_pool_handle()
-        w0 = list(self._next_window)
-        if not any(counts):         # nothing to write; pending resets reach the device with the next push
-            empty = torch.empty(0, device=dev)
-            return [(empty, w) for w in w0]
-        wins = [window_count(self._n_frames[k], self._next_window[k], counts[k], self._reset[k], self.clip_len, self.stride) for k in range(S)]
-        m = max(nw for _, nw in wins)
-        push = torch.tensor([[c, int(r)] for c, r in zip(counts, self._reset)], dtype=torch.int64)
-        key = (n, m, frames.shape[3], frames.shape[4], frames.dtype)
-        g = self.graphs.get(key)
-        if g is None:
-            self.frozen._buffers(S * n, frames.shape[3], frames.shape[4], dev)      # allocated and zeroed outside the capture
-            # warm-up runs the step for real: the rings and the cursors are restored after it, so capturing does not advance the streams
-            g = self.graphs[key] = GraphedStep(self._step(n, m), (frames, push), mutated=(self.rings, self.cursors), pool=self.pool)
-        (scores,) = g(frames, push)
-        for k, (fr, nw) in enumerate(wins):
-            self._n_frames[k] = fr
-            self._next_window[k] += nw
-        self._reset = [False] * S
-        out = scores.clone()
-        return [(out[k * m:k * m + nw], w0[k]) for k, (_, nw) in enumerate(wins)]
+        return [(scores, w0) for (scores,), w0 in self._push(frames, counts, (frames.shape[3], frames.shape[4], frames.dtype))]
 
 
 class GraphedStreamingScorer(MultiStreamScorer):
@@ -291,3 +324,101 @@ class GraphedStreamingScorer(MultiStreamScorer):
             raise ValueError("expected (n, 1, H, W) frames")
         [(scores, w0)] = super().push(frames.unsqueeze(0))
         return scores, w0
+
+
+class MultiStreamClipScorer(_StreamBookkeeping):
+    """Sliding-window scoring of S camera streams for the 3-D clip models -- M-B (``mb.CausalAnomalyDetector``, the model
+    best_improved_model.pth loads into), M-E (``me.CausalAnomalyDetector``, bbox:392-430's window service) and M-C
+    (``mc.SimpleVideoAnomalyDetector``) -- from raw uint8 frames, with one CUDA graph replay per push for all streams.
+
+    Their temporal zero padding makes every window's activations depend on where the window starts (DESIGN.md section 5), so the rings hold
+    resized FRAMES, and each completed window is gathered from its ring and scored by the model's own batched forward: the scores are
+    those of ``model(clips)`` on the clips the reference builds per window.  ``push(frames, counts)`` runs: copy into static inputs ->
+    resize each stream's kept frames into its ring at its device cursor (``cvad_streams_frame_write_u8``: cv2.resize INTER_LINEAR, bit
+    for bit) -> gather the windows each stream completed into m fp32 clip slots per stream, unused slots zeros (``cvad_streams_clips_f32``)
+    -> ``model`` over the S*m slots -> advance the cursors.  M-B and M-E take C = 3 frames in BGR order, as cv2 and video decoders deliver
+    them, and see RGB clips in [0, 1] (the Avenue / bbox loader rule, bbox:397-411); M-C takes C = 1 grayscale frames, scaled by 1/255.
+    M-C's reference loader resizes with PIL (mc3:104-216), not cv2: push M-C frames already at the model's size, where the ring write is
+    a copy.
+
+    Window w of a stream covers its frames w*stride + [0, clip_len) and is scored as soon as they have arrived, the rule of
+    ``MultiStreamScorer`` (``window_count``).  bbox's loop over a finished video, ``range(0, F - window, stride)``, stops one window earlier
+    when (F - clip_len) % stride == 0: such a video gets one window more here, its last one.
+
+    Counts, ``reset``, ``n_frames``, ``next_window`` and the errors are those of ``MultiStreamScorer``.  The graph key is
+    (n, m, H, W, C): at most ceil(n / stride) + 1 graphs per push size and camera frame size.  Graphs share one memory pool and read the
+    model's live tensors, so an in-place weight or BatchNorm-statistic update needs no capture (M-C's eval BatchNorm fold runs inside the
+    graph); a replaced tensor drops them."""
+
+    def __init__(self, model, streams, clip_len=8, stride=4, capacity=32, size=(64, 64)):
+        from . import mb, mc, me
+        if isinstance(model, (mb.CausalAnomalyDetector, me.CausalAnomalyDetector)):
+            self.channels, self.reverse_channels = 3, 1
+            v = 16 if isinstance(model, me.CausalAnomalyDetector) else model.causal_discovery.num_variables
+            feat = model.feature_dim if isinstance(model, me.CausalAnomalyDetector) else model.feature_extractor.fc.out_features
+            self._out_shapes = ((), (v, v), (feat,))
+        elif isinstance(model, mc.SimpleVideoAnomalyDetector):
+            self.channels, self.reverse_channels = 1, 0
+            self._out_shapes = ((),)
+        else:
+            raise TypeError(f"MultiStreamClipScorer scores mb.CausalAnomalyDetector, me.CausalAnomalyDetector or mc.SimpleVideoAnomalyDetector, "
+                            f"not {type(model).__name__}")
+        super().__init__(model, streams, clip_len, stride, capacity)
+        self.size = (int(size[0]), int(size[1]))          # (width, height), as cv2.resize takes it
+
+    def _new_ring(self, dev):
+        w, h = self.size
+        return torch.zeros((self.streams, self.capacity, h, w, self.channels), device=dev, dtype=torch.uint8)
+
+    def _empty(self, dev):
+        return tuple(torch.empty((0,) + s, device=dev) for s in self._out_shapes)
+
+    def _step(self, n, m, H, W):
+        model, S, T, C = self.model, self.streams, self.clip_len, self.channels
+        w, h = self.size
+
+        def step(x, push):
+            x = x.contiguous()
+            st = _st()
+            _call("cvad_streams_frame_write_u8", _ptr(x), S, n, H, W, C, _ptr(self.rings), self.capacity, h, w, T, self.stride,
+                  _ptr(self.cursors), _ptr(push), st)
+            if m > 0:
+                clips = torch.empty((S * m, C, T, h, w), device=x.device, dtype=torch.float32)
+                _call("cvad_streams_clips_f32", _ptr(self.rings), S, self.capacity, h, w, C, T, self.stride, m, _ptr(self.cursors), _ptr(push),
+                      1.0 / 255.0, self.reverse_channels, _ptr(clips), st)
+                out = model(clips)
+                out = (out[0].reshape(-1), out[1], out[2]) if C == 3 else (out.reshape(-1),)      # M-E's s.squeeze() is 0-d at S*m = 1
+            else:
+                out = self._empty(x.device)
+            _call("cvad_streams_cursor_advance", _ptr(self.cursors), S, T, self.stride, _ptr(push), st)
+            return out
+        return step
+
+    def _capture(self, n, m, frames, push):
+        # warm-up runs the step for real: the rings and the cursors are restored after it, so capturing does not advance the streams
+        g = GraphedStep(self._step(n, m, frames.shape[2], frames.shape[3]), (frames, push), mutated=(self.rings, self.cursors), pool=self.pool)
+        cd = getattr(self.model, "causal_discovery", None)
+        if cd is not None:
+            # M-B's self-loop mask is cached for the latest batch size only: the next capture at another S*m replaces it, and the memory this
+            # graph reads would go back to the allocator.  The graph keeps the mask it captured alive.
+            g.held = list(cd._offdiag.values())
+        return g
+
+    @torch.no_grad()
+    def push(self, frames, counts=None):
+        """frames (S, n, H, W, C) uint8 on the model's device (C = 3, BGR, for M-B and M-E; C = 1 for M-C, which also takes (S, n, H, W)) at
+        any camera size H x W; counts: S ints in [0, n], the frames each stream keeps (default n; the rows beyond a count are not read).
+        Returns one (scores, first window index, adjacency, features) per stream, the records bbox:416-425 keeps per window: scores
+        (w,), adjacency (w, 16, 16) and features (w, F) of its w completed windows; adjacency and features are None for M-C."""
+        if frames.dim() == 4:
+            frames = frames.unsqueeze(-1)
+        if frames.dim() != 5:
+            raise ValueError("expected (S, n, H, W, C) frames")
+        if frames.dtype != torch.uint8:
+            raise TypeError(f"MultiStreamClipScorer takes raw uint8 frames, got {frames.dtype}")
+        if frames.shape[4] != self.channels:
+            raise ValueError(f"{type(self.model).__module__}.{type(self.model).__name__} takes {self.channels}-channel frames, got {frames.shape[4]}")
+        res = self._push(frames, counts, tuple(frames.shape[2:]))
+        if self.channels == 1:
+            return [(s, w0, None, None) for (s,), w0 in res]
+        return [(s, w0, a, f) for (s, a, f), w0 in res]

@@ -159,6 +159,21 @@ int cvad_streams_ring_write_f32(const float* feats, int S, long long n, int F, f
 int cvad_streams_window_features_f32(const float* rings, int S, long long capacity, int stride, int T, int F, long long m,
                                      const long long* cursors, const long long* push, float* out, void* stream);
 int cvad_streams_cursor_advance(long long* cursors, int S, int T, int stride, const long long* push, void* stream);
+/* The same streams with rings of FRAMES instead of features (frames.cu), for the 3-D clip models (M-B, M-C, M-E), whose temporal zero
+ * padding makes every window's activations depend on where it starts: each window is gathered from the ring and scored whole.  Same
+ * cursors, push descriptor and window rule as above; issue cvad_streams_cursor_advance after both, on the same stream.
+ * frame_write_u8: src (S*n, src_h, src_w, C) interleaved uint8, stream-major (BGR for C = 3, as cv2 and video decoders deliver it); row
+ *   r < count_k of stream k is resized to (dst_h, dst_w) with cvad_resize_bilinear_u8's rule (cv2.resize INTER_LINEAR, bit-exact; a copy
+ *   at the same size) into rings[k][(base_k + r) % capacity], rings (S, capacity, dst_h, dst_w, C) uint8; rows r >= count_k are not read.
+ * clips_f32: out (S*m, C, T, H, W) fp32 from rings (S, capacity, H, W, C); slot (k, j) holds window next_k + j of stream k (frames
+ *   (next_k + j)*stride + [0,T) modulo capacity) when j < n_win_k, zeros otherwise; each value is value * scale, and channel c reads
+ *   channel C-1-c when reverse_channels (BGR -> RGB): the values of cvad_clips_from_frames_f32 on the same frames.
+ * Both return cudaErrorInvalidValue for a NULL pointer, a non-positive S / capacity / T / stride / size, C outside [1, 4] or a negative
+ * n / m, and 0 without a launch for n = 0 / m = 0. */
+int cvad_streams_frame_write_u8(const void* src, int S, long long n, int src_h, int src_w, int C, void* rings, long long capacity, int dst_h,
+                                int dst_w, int T, int stride, const long long* cursors, const long long* push, void* stream);
+int cvad_streams_clips_f32(const void* rings, int S, long long capacity, int H, int W, int C, int T, int stride, long long m,
+                           const long long* cursors, const long long* push, float scale, int reverse_channels, float* out, void* stream);
 
 /* ---- M-A causal branch, dense masked batched form (ma_tail.cu) -------------------------------------------------------
  * Every clip carries 5 padded track slots (the detector emits <= 5 boxes per frame, cad:178,198) and a per-clip track
