@@ -88,6 +88,10 @@ struct FcParams {
   const __nv_bfloat16* bw_raw;
   const float *bw_gamma, *bw_beta, *bw_mean, *bw_invstd;
   int bw_H, bw_W, planes;
+  // masked column sums (EPI_MASK, data-gradient only, n_blocks == 1): sum_mask holds N bits per output row in the rows' own layout (bit c in
+  // 32-bit word c/32; the ReLU gate the BatchNorm apply of the layer below wrote, 0 on borders and empty plane positions); the epilogue adds
+  // sum over rows of bf16(out) * bit to st_out[0..N) -- the BatchNorm backward's sum g, with no pixel decode and no per-column constants
+  const uint32_t* sum_mask;
   FcUnit units[FC_MAX_UNITS];
 };
 
@@ -117,6 +121,20 @@ __device__ __forceinline__ void warp_colsum16_sq(const float (&x)[16], int lane,
   const float vv = (b1 ? ww[1] : ww[0]) + __shfl_xor_sync(0xffffffffu, b1 ? ww[0] : ww[1], 2);
   sum = v + __shfl_xor_sync(0xffffffffu, v, 1);
   sumsq = vv + __shfl_xor_sync(0xffffffffu, vv, 1);
+}
+
+// the same butterfly for one 32 x 16 tile
+__device__ __forceinline__ float warp_colsum16(const float (&x)[16], int lane) {
+  float y[8], z[4], w[2];
+  const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4, b1 = lane & 2;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) y[i] = (b4 ? x[i + 8] : x[i]) + __shfl_xor_sync(0xffffffffu, b4 ? x[i] : x[i + 8], 16);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) z[i] = (b3 ? y[i + 4] : y[i]) + __shfl_xor_sync(0xffffffffu, b3 ? y[i] : y[i + 4], 8);
+#pragma unroll
+  for (int i = 0; i < 2; ++i) w[i] = (b2 ? z[i + 2] : z[i]) + __shfl_xor_sync(0xffffffffu, b2 ? z[i] : z[i + 2], 4);
+  const float v = (b1 ? w[1] : w[0]) + __shfl_xor_sync(0xffffffffu, b1 ? w[0] : w[1], 2);
+  return v + __shfl_xor_sync(0xffffffffu, v, 1);
 }
 
 // the same butterfly for two independent 32 x 16 tiles (column sums of a and of b)
@@ -150,12 +168,14 @@ __device__ __forceinline__ void warp_colsum16_pair(const float (&a)[16], const f
 //   EPI_BW     data-gradient that also takes the BatchNorm-backward reductions (FcParams::bw_raw)
 //   EPI_RELU   out = relu(conv + bias) on interior pixels and exact zeros on the border: the forward of an eval-mode BatchNorm + ReLU
 //              already folded into the weights and bias; padded-flat or phase planes (FcParams::planes)
-enum { EPI_PLAIN = 0, EPI_BW = 1, EPI_RELU = 2 };
+//   EPI_MASK   data-gradient that also sums its bf16 output under a per-row bitmask (FcParams::sum_mask): the successor of EPI_BW, which
+//              loaded raw (as many bytes as it wrote) and formed xhat per element and slowed the MMAs; this one loads N bits per row
+enum { EPI_PLAIN = 0, EPI_BW = 1, EPI_RELU = 2, EPI_MASK = 3 };
 template <int ROWB, int N, int EPI>
 __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant__ CUtensorMap map_src, const __grid_constant__ CUtensorMap map_tail,
                                                           const __grid_constant__ CUtensorMap map_w, const FcParams p,
                                                           const float* __restrict__ bias, __nv_bfloat16* __restrict__ out) {
-  constexpr bool BW = EPI == EPI_BW, RELU = EPI == EPI_RELU;
+  constexpr bool BW = EPI == EPI_BW, RELU = EPI == EPI_RELU, MS = EPI == EPI_MASK;
   constexpr int NSLOT = (512 / N) > FC_MAX_SLOTS ? FC_MAX_SLOTS : (512 / N);
   constexpr uint32_t TMEM_COLS = NSLOT * N;
   constexpr int TPO = FC_BOX / N;                  // taps per weight box
@@ -398,7 +418,7 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
         bool keep = false;                    // interior pixel (the only ones BatchNorm statistics run over)
         constexpr bool bw = BW;
         const __nv_bfloat16* rrow = nullptr;  // bw: this row's pixel in raw
-        if ((RELU || p.st_out) && q < p.rows) {
+        if ((RELU || (p.st_out && !MS)) && q < p.rows) {
           const int qi = (int)q;
           const int n = fast_div(qi, p.st_mul_img, p.st_shr_img);
           const int r = qi - n * ((p.st_h + 2) * (p.st_w + 2));
@@ -432,6 +452,27 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
             }
           }
         }
+        constexpr int NW = MS ? N / 32 : 1;    // mask words of a row
+        uint32_t mw[NW];
+        if (MS) {
+          const uint32_t* mrow = p.sum_mask + (p.out_row_base + pl * p.plane_out_stride + q) * NW;
+#pragma unroll
+          for (int k = 0; k < NW; ++k) mw[k] = 0u;
+          if (q < p.rows) {
+            if (NW % 4 == 0) {
+#pragma unroll
+              for (int k = 0; k < NW; k += 4) {
+                const uint4 t = __ldg(reinterpret_cast<const uint4*>(mrow + k));
+                mw[k] = t.x; mw[k + 1 < NW ? k + 1 : 0] = t.y; mw[k + 2 < NW ? k + 2 : 0] = t.z; mw[k + 3 < NW ? k + 3 : 0] = t.w;
+              }
+            } else if (NW == 2) {
+              const uint2 t = __ldg(reinterpret_cast<const uint2*>(mrow));
+              mw[0] = t.x; mw[NW - 1] = t.y;
+            } else {
+              mw[0] = __ldg(mrow);
+            }
+          }
+        }
         mbar_wait(&bar_acc_full[slot], (use / NSLOT) & 1);
         tc_fence_after();
 #pragma unroll
@@ -461,7 +502,16 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
             *reinterpret_cast<uint4*>(orow + c0) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
             *reinterpret_cast<uint4*>(orow + c0 + 8) = make_uint4(pk[4], pk[5], pk[6], pk[7]);
           }
-          if (!RELU && p.st_out && !bw) {     // warp-uniform: statistics of exactly the values the BatchNorm kernels will read back
+          if (MS) {                           // sum of the bf16 values just stored, under the row's mask bits
+            const uint32_t bits = mw[(c0 / 32) % NW] >> (c0 & 16);
+            float x[16];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              x[2 * i] = (bits >> (2 * i)) & 1u ? __uint_as_float(pk[i] << 16) : 0.f;
+              x[2 * i + 1] = (bits >> (2 * i + 1)) & 1u ? __uint_as_float(pk[i] & 0xffff0000u) : 0.f;
+            }
+            st_s[c0 / 16] += warp_colsum16(x, lane);
+          } else if (EPI == EPI_PLAIN && p.st_out) {     // warp-uniform: statistics of exactly the values the BatchNorm kernels will read back
             float x[16];
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
@@ -511,15 +561,17 @@ __global__ void __launch_bounds__(384, 1) flatconv_kernel(const __grid_constant_
 #pragma unroll
       for (int i = 0; i < N / 16; ++i) {
         atomicAdd(&s_stat[i * 16 + col], st_s[i]);
-        atomicAdd(&s_stat[N + i * 16 + col], st_q[i]);
+        if (!MS) atomicAdd(&s_stat[N + i * 16 + col], st_q[i]);
       }
     }
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 2) tmem_dealloc<TMEM_COLS>(tmem_base);
-  if (!RELU && p.st_out && !BW)
+  if (EPI == EPI_PLAIN && p.st_out)
     for (int i = tid; i < 2 * N; i += blockDim.x) atomicAdd(p.st_out + i, (double)s_stat[i]);
+  if (MS)
+    for (int i = tid; i < N; i += blockDim.x) atomicAdd(p.st_out + i, (double)s_stat[i]);
   if (BW && p.st_out)                     // sum g*xhat = invstd * (sum g*x - mean * sum g), combined in fp64 (as pad_reduce_kernel does)
     for (int i = tid; i < N; i += blockDim.x) {
       const double a0 = (double)s_stat[i], a1 = (double)s_stat[N + i];
@@ -649,9 +701,10 @@ int run_flat(const void* src, long long src_rows, int K, const void* wpk, int No
   p.ld_out = Nout;
   const long long w_rows = 9LL * Nout;
   __nv_bfloat16* o = (__nv_bfloat16*)out;
-#define CVAD_FC(R, NN) (relu ? launch_flatconv<R, NN, EPI_RELU>(src, src_rows, K, wpk, w_rows, p, bias, o, st)      \
-                        : p.bw_raw ? launch_flatconv<R, NN, EPI_BW>(src, src_rows, K, wpk, w_rows, p, bias, o, st) \
-                                   : launch_flatconv<R, NN, EPI_PLAIN>(src, src_rows, K, wpk, w_rows, p, bias, o, st))
+#define CVAD_FC(R, NN) (relu ? launch_flatconv<R, NN, EPI_RELU>(src, src_rows, K, wpk, w_rows, p, bias, o, st)          \
+                        : p.bw_raw   ? launch_flatconv<R, NN, EPI_BW>(src, src_rows, K, wpk, w_rows, p, bias, o, st)   \
+                        : p.sum_mask ? launch_flatconv<R, NN, EPI_MASK>(src, src_rows, K, wpk, w_rows, p, bias, o, st) \
+                                     : launch_flatconv<R, NN, EPI_PLAIN>(src, src_rows, K, wpk, w_rows, p, bias, o, st))
   if (rowb == 64) {
     if (n == 32) return CVAD_FC(64, 32);
     if (n == 64) return CVAD_FC(64, 64);
@@ -835,8 +888,9 @@ int set_bw(FcParams& p, const BwStats* bw, int H, int W, const FlatGeom& g) {
   return set_pixel_decode(p, g);
 }
 
+// sum_mask / sum_ws: the EPI_MASK column sums of dx (FcParams::sum_mask) into sum_ws[0..Cin)
 int flat_dgrad(const void* dy, const void* w_dgrad, void* dx, int N, int H, int W, int Cin, int Cout, int stride, const BwStats* bw,
-               void* stream) {
+               const void* sum_mask, double* sum_ws, void* stream) {
   // (N,H,W,Cin) is the convolution INPUT geometry.  stride 1: dy, dx padded-flat (N,H+2,W+2,.).  stride 2: dy padded-flat
   // (N,Ho+2,Wo+2,Cout), dx = four phase planes in that same geometry.
   if (stride != 1 && stride != 2) return (int)cudaErrorInvalidValue;
@@ -873,19 +927,25 @@ int flat_dgrad(const void* dy, const void* w_dgrad, void* dx, int N, int H, int 
       memset(&p, 0, sizeof(p));
       p.rows = g.rows;
       p.out_row_base = pl * g.rows;
+      p.sum_mask = (const uint32_t*)sum_mask;
+      p.st_out = sum_ws;
       add_units(p, g, true, slab, nslab, nblk, pl, 1, -1);
       if (int e = run_flat(dy, g.rows, Cout, w_dgrad, Cin, nullptr, dx, p, st)) return e;
     }
     return 0;
   }
   if (int e = set_bw(p, bw, H, W, g)) return e;
+  if (sum_mask) {
+    p.sum_mask = (const uint32_t*)sum_mask;
+    p.st_out = sum_ws;
+  }
   return run_flat(dy, g.rows, Cout, w_dgrad, Cin, nullptr, dx, p, st);
 }
 }  // namespace
 
 CVAD_API int cvad_flat_conv3x3_dgrad_bf16(const void* dy, const void* w_dgrad, void* dx, int N, int H, int W, int Cin, int Cout, int stride,
                                           void* stream) {
-  return flat_dgrad(dy, w_dgrad, dx, N, H, W, Cin, Cout, stride, nullptr, stream);
+  return flat_dgrad(dy, w_dgrad, dx, N, H, W, Cin, Cout, stride, nullptr, nullptr, nullptr, stream);
 }
 
 CVAD_API int cvad_flat_conv3x3_dgrad_bnstats_bf16(const void* dy, const void* w_dgrad, void* dx, int N, int H, int W, int Cin, int Cout,
@@ -893,7 +953,13 @@ CVAD_API int cvad_flat_conv3x3_dgrad_bnstats_bf16(const void* dy, const void* w_
                                                   const float* invstd, double* ws, void* stream) {
   if (!raw_in || !ws || Cin != n_block_of(Cin)) return (int)cudaErrorInvalidValue;
   BwStats bw = {raw_in, gamma, beta, mean, invstd, ws};
-  return flat_dgrad(dy, w_dgrad, dx, N, H, W, Cin, Cout, stride, &bw, stream);
+  return flat_dgrad(dy, w_dgrad, dx, N, H, W, Cin, Cout, stride, &bw, nullptr, nullptr, stream);
+}
+
+CVAD_API int cvad_flat_conv3x3_dgrad_masksum_bf16(const void* dy, const void* w_dgrad, void* dx, int N, int H, int W, int Cin, int Cout, int stride,
+                                                  const void* mask, double* ws, void* stream) {
+  if (!mask || !ws || Cin != n_block_of(Cin)) return (int)cudaErrorInvalidValue;
+  return flat_dgrad(dy, w_dgrad, dx, N, H, W, Cin, Cout, stride, nullptr, mask, ws, stream);
 }
 
 // ================================================================================================ weight gradient
@@ -1087,15 +1153,31 @@ __global__ void __launch_bounds__(256, 1) flatwgrad_kernel(const __grid_constant
   if (warp == 2) tmem_dealloc<512>(tmem_base);
 }
 
-// dw (OIHW) += scratch ([tap][Cout][Cin]); scratch = 0
-__global__ void wgrad_fold_kernel(float* __restrict__ scratch, float* __restrict__ dw, int Cin, int Cout) {
+// dw (OIHW) += scratch ([tap][Cout][Cin]); scratch = 0.  w (OIHW fp32, optional; Cin <= 256): also t[ci] += sum_{co,tap} bf16(w) * scratch,
+// i.e. sum W*dW of this call's weight gradient with the weights the data-gradient multiplies by.  For every input channel that equals
+// sum act*dconv over the convolution's input buffer (dconv = d/d act, zero padding and phase planes included): the BatchNorm backward of the
+// layer below takes its T from here.  One element per thread in dw's order; the products gather in shared memory (a block's 256 elements
+// touch ~30 input channels) and each touched channel costs one fp64 atomic per block.
+__global__ void __launch_bounds__(256) wgrad_fold_kernel(float* __restrict__ scratch, float* __restrict__ dw, int Cin, int Cout,
+                                                         const float* __restrict__ w, double* __restrict__ t) {
+  __shared__ float s_t[256];
+  if (w) {
+    for (int c = threadIdx.x; c < Cin; c += blockDim.x) s_t[c] = 0.f;
+    __syncthreads();
+  }
   const int total = Cout * Cin * 9;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const int tap = i % 9, ci = (i / 9) % Cin, co = i / (9 * Cin);
     float* s = scratch + ((long long)tap * Cout + co) * Cin + ci;
-    dw[i] += *s;
+    const float v = *s;
+    dw[i] += v;
     *s = 0.f;
+    if (w) atomicAdd(&s_t[ci], __bfloat162float(__float2bfloat16(w[i])) * v);
   }
+  if (!w) return;
+  __syncthreads();
+  for (int c = threadIdx.x; c < Cin; c += blockDim.x)
+    if (s_t[c] != 0.f) atomicAdd(t + c, (double)s_t[c]);
 }
 
 template <int ROWB_A, int ROWB_B, int NB, int A_SLABS, int KH>
@@ -1186,15 +1268,28 @@ CVAD_API int cvad_flat_conv3x3_wgrad_bf16(const void* x, const void* dy, float* 
   return flat_wgrad(x, dy, dw, nullptr, N, H, W, Cin, Cout, stride, stream);
 }
 
-CVAD_API int cvad_flat_conv3x3_wgrad_staged_bf16(const void* x, const void* dy, float* dw, float* scratch, int N, int H, int W, int Cin,
-                                                 int Cout, int stride, void* stream) {
+namespace {
+int wgrad_staged(const void* x, const void* dy, float* dw, float* scratch, int N, int H, int W, int Cin, int Cout, int stride, const float* w,
+                 double* t, void* stream) {
   if (!scratch) return (int)cudaErrorInvalidValue;
   int e = flat_wgrad(x, dy, dw, scratch, N, H, W, Cin, Cout, stride, stream);
   if (e) return e;
   const int total = Cout * Cin * 9;
-  wgrad_fold_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(scratch, dw, Cin, Cout);
+  wgrad_fold_kernel<<<(total + 255) / 256, 256, 0, (cudaStream_t)stream>>>(scratch, dw, Cin, Cout, w, t);
   CVAD_LAUNCH_CHECK();
   return 0;
+}
+}  // namespace
+
+CVAD_API int cvad_flat_conv3x3_wgrad_staged_bf16(const void* x, const void* dy, float* dw, float* scratch, int N, int H, int W, int Cin,
+                                                 int Cout, int stride, void* stream) {
+  return wgrad_staged(x, dy, dw, scratch, N, H, W, Cin, Cout, stride, nullptr, nullptr, stream);
+}
+
+CVAD_API int cvad_flat_conv3x3_wgrad_staged_wdot_bf16(const void* x, const void* dy, float* dw, float* scratch, int N, int H, int W, int Cin,
+                                                      int Cout, int stride, const float* w, double* ws, void* stream) {
+  if (!w || !ws || Cin > 256) return (int)cudaErrorInvalidValue;
+  return wgrad_staged(x, dy, dw, scratch, N, H, W, Cin, Cout, stride, w, ws + Cin, stream);
 }
 
 namespace {

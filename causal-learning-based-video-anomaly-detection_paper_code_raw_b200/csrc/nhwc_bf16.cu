@@ -1,7 +1,8 @@
 // Bandwidth kernels of the bf16 (tensor-core) M-A backbone path on the padded-flat / phase-plane layouts of flatconv_tc.cu:
 //   bn_stats:  per-channel batch mean / biased variance (fp64 accumulation) + running-stat update (cad:131,136)
 //   bn_apply:  y = relu((x-mean)*invstd*gamma+beta), bf16 -> bf16, zero border / phase planes for the next convolution
-//   bn_bwd:    ReLU + BatchNorm backward (two passes: per-channel reductions, then dx), dgamma/dbeta accumulated in fp32
+//   bn_bwd:    ReLU + BatchNorm backward (two passes: per-channel reductions, then dx), dgamma/dbeta accumulated in fp32; or one pass when the
+//              reductions arrive from the convolution above (the "T" form, see pad_bn_relu_bwd_apply_kernel)
 //   avgpool:   AdaptiveAvgPool2d((4,6)) (cad:126,155) bf16 -> fp32 features in the reference's (c,h,w) flatten order
 // All loads/stores are 16-byte vectors over the channel axis (8 bf16), coalesced across threads.
 #include "common.cuh"
@@ -62,6 +63,9 @@ __device__ __forceinline__ long long phase_row(const PadGeo& g, int n, int hp, i
 }
 
 // relu(bn(raw)) -> act.  PHASE=0: plain padded act, zero border.  PHASE=1: four phase planes (zeros where no pixel maps).
+// mask (optional): the ReLU gate as one bit per element in act's row layout -- byte k holds the 8 channels of act's 16-byte vector k (bit c of
+// a pixel in 32-bit word c/32), 0 wherever act is zero by construction.  The data-gradient of the next convolution sums its output under
+// it (the BatchNorm backward's sum g, cvad_flat_conv3x3_dgrad_masksum_bf16), 1/16 of the bytes of re-reading raw.
 // Block = 256 threads, two 16-byte vectors per thread and pass (v = tid, tid + 256): every padded row of the backbone
 // (368..448 vectors) is one pass with all loads issued before the first use.  PHASE=1 handles the two column-phase planes
 // (a,0) and (a,1) of one plane row in the same block, so the raw row both of them sample is fetched from HBM once.
@@ -91,10 +95,13 @@ __device__ __forceinline__ void bn_fold_release(double* ws, int C) {
   }
 }
 
+// Output positions are 32-bit vector indices (make_geo bounds the buffers): with 64-bit ones the mask store took the phase-plane form from
+// 80 to 102 registers, i.e. from 3 to 2 resident CTAs per SM.
 template <int PHASE, int R, bool FIN>
-__global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloat16* __restrict__ raw, __nv_bfloat16* __restrict__ act, PadGeo g,
-                                                                const float* __restrict__ mean, const float* __restrict__ invstd,
-                                                                const float* __restrict__ gamma, const float* __restrict__ beta, BnFin fin) {
+__global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloat16* __restrict__ raw, __nv_bfloat16* __restrict__ act,
+                                                                uint8_t* __restrict__ mask, PadGeo g, const float* __restrict__ mean,
+                                                                const float* __restrict__ invstd, const float* __restrict__ gamma,
+                                                                const float* __restrict__ beta, BnFin fin) {
   const int groups = 1 << g.lg;
   const int cg = threadIdx.x & (groups - 1);
   float sc[8], sh[8];
@@ -130,7 +137,7 @@ __global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloa
     for (int v0 = threadIdx.x; v0 < span; v0 += 512) {
       uint4 x[R][2];
       bool in[R][2], ok[R][2];
-      long long dst[R][2];
+      unsigned dst[R][2];
 #pragma unroll
       for (int rr = 0; rr < R; ++rr) {
         // fin.reverse: rows are walked from the END of the tensor -- the convolution in front of this kernel wrote raw front to back, so
@@ -138,7 +145,7 @@ __global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloa
         // kernel then wrote last
         const int r = fin.reverse ? items - 1 - (r0 + rr) : r0 + rr;
         int n = 0, hp = -1, a = 0;
-        long long row0 = 0, row1 = 0;                              // first vector of the output row(s)
+        unsigned row0 = 0, row1 = 0;                              // first vector of the output row(s)
         if (r >= 0 && r < items) {
           if (PHASE) {
             const int t = fast_div(r, g.mulHq, g.shrHq);
@@ -146,12 +153,12 @@ __global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloa
             a = fast_div(t, g.mulN, g.shrN);
             n = t - a * g.N;
             hp = 2 * (i - 1) + a;
-            row0 = ((((long long)(2 * a) * g.N + n) * g.Hq) + i) * rowlen;
-            row1 = ((((long long)(2 * a + 1) * g.N + n) * g.Hq) + i) * rowlen;
+            row0 = (((unsigned)(2 * a) * g.N + n) * g.Hq + i) * rowlen;
+            row1 = (((unsigned)(2 * a + 1) * g.N + n) * g.Hq + i) * rowlen;
           } else {
             n = fast_div(r, g.mulHp, g.shrHp);
             hp = r - n * Hp;
-            row0 = (long long)r * rowlen;
+            row0 = (unsigned)r * rowlen;
           }
         }
         const bool row_ok = hp >= 1 && hp <= g.H;
@@ -174,14 +181,20 @@ __global__ void __launch_bounds__(256) pad_bn_apply_relu_kernel(const __nv_bfloa
         for (int u = 0; u < 2; ++u) {
           if (!in[rr][u]) continue;
           uint4 o = make_uint4(0, 0, 0, 0);
+          unsigned bits = 0u;
           if (ok[rr][u]) {
             float f[8];
             unpack8(x[rr][u], f);
 #pragma unroll
-            for (int i = 0; i < 8; ++i) f[i] = fmaxf(fmaf(f[i], sc[i], sh[i]), 0.f);
+            for (int i = 0; i < 8; ++i) {
+              const float y = fmaf(f[i], sc[i], sh[i]);
+              bits |= (y > 0.f ? 1u : 0u) << i;
+              f[i] = fmaxf(y, 0.f);
+            }
             o = pack8(f);
           }
           reinterpret_cast<uint4*>(act)[dst[rr][u]] = o;
+          if (mask) mask[dst[rr][u]] = (uint8_t)bits;
         }
     }
   }
@@ -303,7 +316,15 @@ __global__ void __launch_bounds__(256, 3) pad_reduce_kernel(const __nv_bfloat16*
 // FOLD: block 0 also adds the two sums into dgamma / dbeta and the last block past the prologue re-zeroes ws (the parameter-update kernel's
 // work): no third launch.
 // OCC: resident CTAs per SM the register allocation is held to (98 registers = 2 CTAs when left alone; 3 CTAs cost ~20 spilled registers)
-template <int PHASE, int R, bool FOLD, int OCC>
+// TS: no reduce pass in front.  ws[0, C) holds S1 = sum g (the masked-sum epilogue of the data-gradient above) and ws[C, 2C) holds
+// T = sum act*dact (from the weight gradient above: sum W*dW, cvad_flat_conv3x3_wgrad_staged_wdot_bf16).  Since act = relu(gamma*xhat + beta),
+// gamma * sum g*xhat = T - beta*S1, which is all the apply needs (no division by gamma).  dgamma / dbeta keep their definition: each thread
+// keeps its channel group, sums g and g*x in registers, and the block adds sum g and sum g*xhat into g_bn_tsum (the layout of a BatchNorm
+// workspace); the last block past the prologue re-zeroes ws, and the parameter-update launch behind the kernel consumes and re-zeroes
+// g_bn_tsum.
+__device__ double g_bn_tsum[2 * 256];      // zero-initialised; every TS backward leaves it zero again (stream-ordered, as ws)
+
+template <int PHASE, int R, bool FOLD, int OCC, bool TS = false>
 __global__ void __launch_bounds__(256, OCC) pad_bn_relu_bwd_apply_kernel(const __nv_bfloat16* __restrict__ raw, const __nv_bfloat16* __restrict__ dact,
                                                                     __nv_bfloat16* __restrict__ draw, PadGeo g, const float* __restrict__ mean,
                                                                     const float* __restrict__ invstd, const float* __restrict__ gamma,
@@ -313,7 +334,7 @@ __global__ void __launch_bounds__(256, OCC) pad_bn_relu_bwd_apply_kernel(const _
   const int cg = threadIdx.x & (groups - 1);
   // With a = gamma*invstd, b = beta - mean*a (the forward's scale/shift), g = dact*(x*a + b > 0), mg = mean(g), mgx = mean(g*xhat):
   //   draw = a*(g - mg - xhat*mgx) = a*g - k0 - k1*x,   k1 = a*mgx*invstd,  k0 = a*mg - k1*mean     (eval mode: k0 = k1 = 0)
-  float ca[8], cb[8], k0[8], k1[8];
+  float ca[8], cb[8], k0[8], k1[8], sg[8], sgx[8];
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     const int c = cg * 8 + i;
@@ -321,10 +342,18 @@ __global__ void __launch_bounds__(256, OCC) pad_bn_relu_bwd_apply_kernel(const _
     ca[i] = gamma[c] * is;
     cb[i] = beta[c] - mu * ca[i];
     const float mg = training ? (float)(ws[c] / count) : 0.f;
-    const float mgx = training ? (float)(ws[g.C + c] / count) : 0.f;
-    k1[i] = ca[i] * mgx * is;
+    if (TS) {
+      const float gmgx = training ? (float)((ws[g.C + c] - (double)beta[c] * ws[c]) / count) : 0.f;     // gamma * mean(g*xhat)
+      k1[i] = gmgx * is * is;
+    } else {
+      const float mgx = training ? (float)(ws[g.C + c] / count) : 0.f;
+      k1[i] = ca[i] * mgx * is;
+    }
     k0[i] = ca[i] * mg - k1[i] * mu;
+    sg[i] = 0.f;
+    sgx[i] = 0.f;
   }
+  if (TS) bn_fold_release(ws, g.C);
   if (FOLD) {
     if (blockIdx.x == 0)
       for (int c = threadIdx.x; c < g.C; c += blockDim.x) bn_params_channel(ws, g.C, c, dgamma, dbeta);
@@ -369,12 +398,33 @@ __global__ void __launch_bounds__(256, OCC) pad_bn_relu_bwd_apply_kernel(const _
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
               const float gg = fmaf(f[i], ca[i], cb[i]) > 0.f ? d[i] : 0.f;
+              if (TS) {
+                sg[i] += gg;
+                sgx[i] = fmaf(gg, f[i], sgx[i]);
+              }
               f[i] = fmaf(-k1[i], f[i], fmaf(ca[i], gg, -k0[i]));
             }
             o = pack8(f);
           }
           reinterpret_cast<uint4*>(draw)[(long long)(r0 + rr) * rowlen + v0 + u * 256] = o;
         }
+    }
+  }
+  if (TS) {      // block sums per channel (as pad_reduce_kernel: fp32 per thread, fp64 across the block's slots), then one atomic per channel
+    __shared__ float red[TS ? 256 * 16 : 1];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { red[threadIdx.x * 16 + i] = sg[i]; red[threadIdx.x * 16 + 8 + i] = sgx[i]; }
+    __syncthreads();
+    const int slots = blockDim.x >> g.lg;
+    for (int c = threadIdx.x; c < g.C; c += blockDim.x) {
+      const int g2 = c >> 3, i = c & 7;
+      double a0 = 0.0, a1 = 0.0;
+      for (int r = 0; r < slots; ++r) {
+        a0 += (double)red[(r * groups + g2) * 16 + i];
+        a1 += (double)red[(r * groups + g2) * 16 + 8 + i];
+      }
+      atomicAdd(g_bn_tsum + c, a0);
+      atomicAdd(g_bn_tsum + g.C + c, (a1 - (double)mean[c] * a0) * (double)invstd[c]);
     }
   }
 }
@@ -551,6 +601,8 @@ inline int make_geo(PadGeo& g, int N, int H, int W, int C, int phase) {
   g.N = N; g.H = H; g.W = W; g.C = C;
   g.Hq = phase ? (H - 1) / 2 + 3 : 0;
   g.Wq = phase ? (W - 1) / 2 + 3 : 0;
+  // the apply kernel addresses its output in 16-byte vectors with 32-bit indices
+  if ((long long)N * (H + 2) * (W + 2) * (C / 8) > 0xffffffffLL || 4LL * N * g.Hq * g.Wq * (C / 8) > 0xffffffffLL) return 1;
   g.lg = 0;
   while ((8 << g.lg) < C) ++g.lg;
   fast_div_init((unsigned)W, g.mulW, g.shrW);
@@ -606,15 +658,16 @@ inline int bn_apply_reverse() {
   return v;
 }
 
-int launch_apply(const __nv_bfloat16* r, __nv_bfloat16* a, const PadGeo& g, int N, int H, int phase_out, const float* mean, const float* invstd,
-                 const float* gamma, const float* beta, bool finalize, const BnFin& fin_in, cudaStream_t st) {
+int launch_apply(const __nv_bfloat16* r, __nv_bfloat16* a, uint8_t* mask, const PadGeo& g, int N, int H, int phase_out, const float* mean,
+                 const float* invstd, const float* gamma, const float* beta, bool finalize, const BnFin& fin_in, cudaStream_t st) {
   BnFin fin = fin_in;
   fin.reverse = bn_apply_reverse();
   const int rows = phase_out ? 2 * N * g.Hq : N * (H + 2);
   const int R = bn_rows_per_iter();
   const int want = (rows + R - 1) / R;
 #define CVAD_APPLY(PH, RR, FI) \
-  pad_bn_apply_relu_kernel<PH, RR, FI><<<apply_grid(pad_bn_apply_relu_kernel<PH, RR, FI>, want), 256, 0, st>>>(r, a, g, mean, invstd, gamma, beta, fin)
+  pad_bn_apply_relu_kernel<PH, RR, FI><<<apply_grid(pad_bn_apply_relu_kernel<PH, RR, FI>, want), 256, 0, st>>>(r, a, mask, g, mean, invstd, gamma, \
+                                                                                                                beta, fin)
 #define CVAD_APPLY2(PH, FI) { if (R == 2) CVAD_APPLY(PH, 2, FI); else CVAD_APPLY(PH, 4, FI); }
   if (phase_out) { if (finalize) CVAD_APPLY2(1, true) else CVAD_APPLY2(1, false) }
   else { if (finalize) CVAD_APPLY2(0, true) else CVAD_APPLY2(0, false) }
@@ -636,10 +689,11 @@ inline int bn_fold() {
   return v;
 }
 
-// apply pass of the backward; with dgamma / dbeta it also performs the parameter-gradient update and re-zeroes ws (FOLD)
+// apply pass of the backward; with dgamma / dbeta it also performs the parameter-gradient update and re-zeroes ws (FOLD).  ts: the
+// (S1, T) form (no FOLD), which also takes the parameter-gradient sums
 int launch_bwd_apply(const __nv_bfloat16* r, const __nv_bfloat16* d, __nv_bfloat16* draw, const PadGeo& g, int N, int H, int W, int phase_in,
                      const float* mean, const float* invstd, const float* gamma, const float* beta, double* ws, int training, bool fold,
-                     float* dgamma, float* dbeta, cudaStream_t st) {
+                     float* dgamma, float* dbeta, cudaStream_t st, bool ts = false) {
   const int rows = N * (H + 2);
   const int R = bn_rows_per_iter();
   const int want = (rows + R - 1) / R;
@@ -649,12 +703,14 @@ int launch_bwd_apply(const __nv_bfloat16* r, const __nv_bfloat16* d, __nv_bfloat
     const char* e = getenv("CVAD_BN_OCC");
     occ3 = e ? (atoi(e) >= 3) : 0;          // measured: 3 CTAs per SM (80 registers, ~20 spilled) is 75 us per step slower than 2 (98 registers)
   }
-#define CVAD_BAPPLY(PH, RR, FO, OC)                                                                                                         \
-  pad_bn_relu_bwd_apply_kernel<PH, RR, FO, OC><<<apply_grid(pad_bn_relu_bwd_apply_kernel<PH, RR, FO, OC>, want), 256, 0, st>>>(               \
+#define CVAD_BAPPLY(PH, RR, FO, OC, TS)                                                                                                     \
+  pad_bn_relu_bwd_apply_kernel<PH, RR, FO, OC, TS><<<apply_grid(pad_bn_relu_bwd_apply_kernel<PH, RR, FO, OC, TS>, want), 256, 0, st>>>(       \
       r, d, draw, g, mean, invstd, gamma, beta, ws, count, training, dgamma, dbeta)
-#define CVAD_BAPPLY2(PH, FO) { if (R == 2) { if (occ3) CVAD_BAPPLY(PH, 2, FO, 3); else CVAD_BAPPLY(PH, 2, FO, 2); } else CVAD_BAPPLY(PH, 4, FO, 1); }
-  if (phase_in) { if (fold) CVAD_BAPPLY2(1, true) else CVAD_BAPPLY2(1, false) }
-  else { if (fold) CVAD_BAPPLY2(0, true) else CVAD_BAPPLY2(0, false) }
+#define CVAD_BAPPLY2(PH, FO, TS) \
+  { if (R == 2) { if (occ3) CVAD_BAPPLY(PH, 2, FO, 3, TS); else CVAD_BAPPLY(PH, 2, FO, 2, TS); } else CVAD_BAPPLY(PH, 4, FO, 1, TS); }
+  if (ts) { if (phase_in) CVAD_BAPPLY2(1, false, true) else CVAD_BAPPLY2(0, false, true) }
+  else if (phase_in) { if (fold) CVAD_BAPPLY2(1, true, false) else CVAD_BAPPLY2(1, false, false) }
+  else { if (fold) CVAD_BAPPLY2(0, true, false) else CVAD_BAPPLY2(0, false, false) }
 #undef CVAD_BAPPLY2
 #undef CVAD_BAPPLY
   CVAD_LAUNCH_CHECK();
@@ -688,12 +744,13 @@ CVAD_API int cvad_pad_bn_apply_relu_bf16(const void* raw, void* act, int N, int 
   cudaStream_t st = (cudaStream_t)stream;
   BnFin fin;
   memset(&fin, 0, sizeof(fin));
-  return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, g, N, H, phase_out, mean, invstd, gamma, beta, false, fin, st);
+  return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, nullptr, g, N, H, phase_out, mean, invstd, gamma, beta, false, fin, st);
 }
 
-CVAD_API int cvad_pad_bn_finalize_apply_relu_bf16(const void* raw, void* act, int N, int H, int W, int C, int phase_out, double* ws, float eps,
-                                                  float momentum, const float* gamma, const float* beta, float* mean, float* invstd,
-                                                  float* running_mean, float* running_var, long long* num_batches_tracked, void* stream) {
+namespace {
+int finalize_apply(const void* raw, void* act, void* mask, int N, int H, int W, int C, int phase_out, double* ws, float eps, float momentum,
+                   const float* gamma, const float* beta, float* mean, float* invstd, float* running_mean, float* running_var,
+                   long long* num_batches_tracked, void* stream) {
   PadGeo g;
   if (make_geo(g, N, H, W, C, phase_out) || !ws || !mean || !invstd) return (int)cudaErrorInvalidValue;
   cudaStream_t st = (cudaStream_t)stream;
@@ -703,10 +760,39 @@ CVAD_API int cvad_pad_bn_finalize_apply_relu_bf16(const void* raw, void* act, in
     if (e) return e;
     BnFin none;
     memset(&none, 0, sizeof(none));
-    return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, g, N, H, phase_out, mean, invstd, gamma, beta, false, none, st);
+    return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, (uint8_t*)mask, g, N, H, phase_out, mean, invstd, gamma, beta, false,
+                        none, st);
   }
   BnFin fin = {0, ws, count, eps, momentum, mean, invstd, running_mean, running_var, num_batches_tracked};
-  return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, g, N, H, phase_out, nullptr, nullptr, gamma, beta, true, fin, st);
+  return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, (uint8_t*)mask, g, N, H, phase_out, nullptr, nullptr, gamma, beta, true,
+                      fin, st);
+}
+}  // namespace
+
+CVAD_API int cvad_pad_bn_finalize_apply_relu_bf16(const void* raw, void* act, int N, int H, int W, int C, int phase_out, double* ws, float eps,
+                                                  float momentum, const float* gamma, const float* beta, float* mean, float* invstd,
+                                                  float* running_mean, float* running_var, long long* num_batches_tracked, void* stream) {
+  return finalize_apply(raw, act, nullptr, N, H, W, C, phase_out, ws, eps, momentum, gamma, beta, mean, invstd, running_mean, running_var,
+                        num_batches_tracked, stream);
+}
+
+CVAD_API int cvad_pad_bn_finalize_apply_relu_mask_bf16(const void* raw, void* act, void* mask, int N, int H, int W, int C, int phase_out,
+                                                       double* ws, float eps, float momentum, const float* gamma, const float* beta, float* mean,
+                                                       float* invstd, float* running_mean, float* running_var, long long* num_batches_tracked,
+                                                       void* stream) {
+  if (!mask) return (int)cudaErrorInvalidValue;
+  return finalize_apply(raw, act, mask, N, H, W, C, phase_out, ws, eps, momentum, gamma, beta, mean, invstd, running_mean, running_var,
+                        num_batches_tracked, stream);
+}
+
+CVAD_API int cvad_pad_bn_apply_relu_mask_bf16(const void* raw, void* act, void* mask, int N, int H, int W, int C, int phase_out, const float* mean,
+                                              const float* invstd, const float* gamma, const float* beta, void* stream) {
+  PadGeo g;
+  if (!mask || make_geo(g, N, H, W, C, phase_out)) return (int)cudaErrorInvalidValue;
+  BnFin fin;
+  memset(&fin, 0, sizeof(fin));
+  return launch_apply((const __nv_bfloat16*)raw, (__nv_bfloat16*)act, (uint8_t*)mask, g, N, H, phase_out, mean, invstd, gamma, beta, false, fin,
+                      (cudaStream_t)stream);
 }
 
 CVAD_API int cvad_pad_bn_relu_bwd_bf16(const void* raw, const void* dact, void* draw, int N, int H, int W, int C, int phase_in,
@@ -739,6 +825,32 @@ CVAD_API int cvad_pad_bn_relu_bwd_apply_bf16(const void* raw, const void* dact, 
   int e = launch_bwd_apply(r, d, (__nv_bfloat16*)draw, g, N, H, W, phase_in, mean, invstd, gamma, beta, ws, training, fold, dgamma, dbeta, st);
   if (e || fold) return e;
   return bn_params_launch(ws, C, dgamma, dbeta, st);
+}
+
+// the parameter-gradient update of the TS backward, from g_bn_tsum (re-zeroed)
+static __global__ void bn_tsum_params_kernel(int C, float* __restrict__ dgamma, float* __restrict__ dbeta) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c < C) {
+    bn_params_channel(g_bn_tsum, C, c, dgamma, dbeta);
+    g_bn_tsum[c] = 0.0;
+    g_bn_tsum[C + c] = 0.0;
+  }
+}
+
+// Training-mode backward without the reduce pass: ws[0, C) = sum g and ws[C, 2C) = sum act*dact are already there (see the TS form of
+// pad_bn_relu_bwd_apply_kernel); one pass over raw and dact, then the parameter-gradient update.  ws is zero again afterwards.
+CVAD_API int cvad_pad_bn_relu_bwd_tsum_bf16(const void* raw, const void* dact, void* draw, int N, int H, int W, int C, int phase_in,
+                                            const float* mean, const float* invstd, const float* gamma, const float* beta, double* ws,
+                                            float* dgamma, float* dbeta, void* stream) {
+  PadGeo g;
+  if (make_geo(g, N, H, W, C, phase_in) || !draw || !ws) return (int)cudaErrorInvalidValue;
+  cudaStream_t st = (cudaStream_t)stream;
+  int e = launch_bwd_apply((const __nv_bfloat16*)raw, (const __nv_bfloat16*)dact, (__nv_bfloat16*)draw, g, N, H, W, phase_in, mean, invstd, gamma,
+                           beta, ws, 1, false, nullptr, nullptr, st, true);
+  if (e) return e;
+  bn_tsum_params_kernel<<<(C + 127) / 128, 128, 0, st>>>(C, dgamma, dbeta);
+  CVAD_LAUNCH_CHECK();
+  return 0;
 }
 
 CVAD_API int cvad_pad_avgpool_bf16_fwd(const void* x, int N, int H, int W, int C, int OH, int OW, float* out, void* stream) {

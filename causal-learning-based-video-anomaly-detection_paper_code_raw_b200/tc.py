@@ -10,8 +10,11 @@ straight into tcgen05.mma.  Statistics and parameter gradients are fp32.
   for the 8 layers: raw_i = flatconv(a_{i-1}) ; (mean, invstd) = stats(raw_i) ; a_i = relu(bn(raw_i)) [plain | phase planes]
   features = AdaptiveAvgPool(4,6)(a_8) -> fp32 (B*T, 6144) in the reference's (c,h,w) order
 
-Backward walks the same list in reverse: fused ReLU+BN backward (two passes), tcgen05 weight-gradient (fp32 atomics into
-the gradient arena) and tcgen05 data-gradient.  Convolution biases that feed a BatchNorm have an analytically zero
+Backward walks the same list in reverse: ReLU+BN backward, tcgen05 weight-gradient (fp32 atomics into the gradient arena) and
+tcgen05 data-gradient.  The BatchNorm backward of every training-mode layer below the top one is one pass over raw and dact: its two
+per-channel sums come from the convolution above -- sum g from the data-gradient's epilogue under the ReLU bitmask the forward apply
+wrote, sum act*dact = sum W*dW from the staged weight gradient (include/cvad_b200.h, cvad_pad_bn_relu_bwd_tsum_bf16).  The top layer
+(its dact comes from the average pool) and the configurations without a staged main-stream weight gradient take a reduce pass first.  Convolution biases that feed a BatchNorm have an analytically zero
 gradient (the reference only accumulates round-off there); they receive exactly zero here.
 """
 from __future__ import annotations
@@ -44,10 +47,6 @@ FUSED_STATS = os.environ.get("CVAD_FUSED_BN_STATS", "1") != "0"     # BatchNorm 
 # weight-gradient GEMMs on a side stream: wgrad_i needs only draw_i and a_{i-1}, so it can run beside the HBM-bound BatchNorm backward of
 # the next layer down instead of in front of it (a parallel branch of the captured step graph)
 WGRAD_OVERLAP = os.environ.get("CVAD_WGRAD_OVERLAP", "0") == "1"
-# BatchNorm-backward reductions of layer i-1 taken in the data-gradient epilogue of layer i (one pass over raw / dact instead of two).
-# Correct (the epilogue's sums: tests/test_flat_gpu.py; the apply entry that consumes them: tests/test_bn_flat_gpu.py) but OFF: measured on a B200 it lengthens the data-gradients (8 epilogue warps become the bottleneck:
-# 0.62 -> 1.20 ms, 1.0 ms with the raw rows prefetched before the accumulator wait) by more than the reduce pass it removes (0.27 ms).
-FUSED_BN_BWD = os.environ.get("CVAD_FUSED_BN_BWD", "0") == "1"
 
 
 def _layers(bb):
@@ -122,6 +121,9 @@ class _BackboneBF16(torch.autograd.Function):
         cur.wait_stream(side)
         saved = []
         cin = C1
+        # ReLU bitmask of layer i for its (S1, T) backward: a training-mode BatchNorm under a convolution whose weight gradient runs staged
+        # on this stream (T is read from its staging buffer, and it must be complete before layer i's backward)
+        ts_ok = need_bwd and STAGED_WGRAD and not WGRAD_OVERLAP
         for i, (conv, bn) in enumerate(layers):
             cout, stride = conv.out_channels, strides[i]
             wf, wd = packs[i]
@@ -143,15 +145,20 @@ class _BackboneBF16(torch.autograd.Function):
                 _call("cvad_bn_eval_prepare_f32", cout, float(bn.eps), _ptr(bn.running_mean), _ptr(bn.running_var), _ptr(mean), _ptr(invstd), st)
             phase_out = i + 1 < len(layers) and strides[i + 1] == 2
             act = torch.empty(act_shape(N, ho, wo, cout, phase_out), device=dev, dtype=BF16)
+            mask = None
+            if ts_ok and bn.training and i + 1 < len(layers) and _wants_grad(layers[i + 1][0].weight):
+                mask = torch.empty(act.numel() // 8, device=dev, dtype=torch.uint8)
             if fused:
-                _call("cvad_pad_bn_finalize_apply_relu_bf16", _ptr(raw), _ptr(act), N, ho, wo, cout, int(phase_out), _ptr(ws), float(bn.eps),
+                _call("cvad_pad_bn_finalize_apply_relu_mask_bf16" if mask is not None else "cvad_pad_bn_finalize_apply_relu_bf16", _ptr(raw),
+                      _ptr(act), *((_ptr(mask),) if mask is not None else ()), N, ho, wo, cout, int(phase_out), _ptr(ws), float(bn.eps),
                       float(bn.momentum), _ptr(bn.weight), _ptr(bn.bias), _ptr(mean), _ptr(invstd), _ptr(bn.running_mean), _ptr(bn.running_var),
                       _ptr(bn.num_batches_tracked), st)
             else:
-                _call("cvad_pad_bn_apply_relu_bf16", _ptr(raw), _ptr(act), N, ho, wo, cout, int(phase_out), _ptr(mean), _ptr(invstd),
-                      _ptr(bn.weight), _ptr(bn.bias), st)
+                _call("cvad_pad_bn_apply_relu_mask_bf16" if mask is not None else "cvad_pad_bn_apply_relu_bf16", _ptr(raw), _ptr(act),
+                      *((_ptr(mask),) if mask is not None else ()), N, ho, wo, cout, int(phase_out), _ptr(mean), _ptr(invstd), _ptr(bn.weight),
+                      _ptr(bn.bias), st)
             if need_bwd:
-                saved.append((a, raw, mean, invstd, wd, (h, w, cin, cout, stride, ho, wo), bn.training, phase_out))
+                saved.append((a, raw, mean, invstd, wd, (h, w, cin, cout, stride, ho, wo), bn.training, phase_out, mask))
             a, h, w, cin = act, ho, wo, cout
         feats = torch.empty((N, cin, 4, 6), device=dev, dtype=torch.float32)
         _call("cvad_pad_avgpool_bf16_fwd", _ptr(a), N, h, w, cin, 4, 6, _ptr(feats), st)
@@ -174,20 +181,19 @@ class _BackboneBF16(torch.autograd.Function):
         cur = torch.cuda.current_stream()
         side = ops.aux_stream(dev, 1) if WGRAD_OVERLAP else None
         keep = []                     # operands of side-stream launches stay referenced until the join (the allocator tracks one stream)
-        sums_ready = False            # the BatchNorm-backward sums of layer idx were taken by the data-gradient of layer idx + 1
         for idx in range(len(layers) - 1, -1, -1):
             conv, bn = layers[idx]
-            a_in, raw, mean, invstd, wd, (hi, wi, cin, cout, stride, ho, wo), bn_training, phase_out = saved[idx]
+            a_in, raw, mean, invstd, wd, (hi, wi, cin, cout, stride, ho, wo), bn_training, phase_out, mask = saved[idx]
             draw = torch.empty_like(raw)
             dg = grad_buffer(bn.weight) if _wants_grad(bn.weight) else None
             db = grad_buffer(bn.bias) if _wants_grad(bn.bias) else None
-            if sums_ready:      # the two per-channel sums are already in the workspace (taken by the data-gradient above)
-                _call("cvad_pad_bn_relu_bwd_apply_bf16", _ptr(raw), _ptr(dact), _ptr(draw), N, ho, wo, cout, int(phase_out), _ptr(mean), _ptr(invstd),
-                      _ptr(bn.weight), _ptr(bn.bias), int(bn_training), _ptr(ops.bn_workspace(dev, cout)), _ptr(dg), _ptr(db), st)
+            if mask is not None:    # sum g and sum act*dact are already in the workspace (taken by the convolution above)
+                _call("cvad_pad_bn_relu_bwd_tsum_bf16", _ptr(raw), _ptr(dact), _ptr(draw), N, ho, wo, cout, int(phase_out), _ptr(mean), _ptr(invstd),
+                      _ptr(bn.weight), _ptr(bn.bias), _ptr(ops.bn_workspace(dev, cout)), _ptr(dg), _ptr(db), st)
             else:
                 _call("cvad_pad_bn_relu_bwd_bf16", _ptr(raw), _ptr(dact), _ptr(draw), N, ho, wo, cout, int(phase_out), _ptr(mean), _ptr(invstd),
                       _ptr(bn.weight), _ptr(bn.bias), int(bn_training), _ptr(ops.bn_workspace(dev, cout)), _ptr(dg), _ptr(db), st)
-            sums_ready = False
+            mask_lo = saved[idx - 1][8] if idx > 0 else None      # the layer below takes its sums from this layer's convolution
             if _wants_grad(conv.weight):
                 wst = st
                 if side is not None:
@@ -195,7 +201,11 @@ class _BackboneBF16(torch.autograd.Function):
                     keep.append((a_in, draw))
                     wst = side.cuda_stream
                 with torch.cuda.stream(side) if side is not None else contextlib.nullcontext():
-                    if STAGED_WGRAD:
+                    if mask_lo is not None:
+                        _call("cvad_flat_conv3x3_wgrad_staged_wdot_bf16", _ptr(a_in), _ptr(draw), _ptr(grad_buffer(conv.weight)),
+                              _ptr(_wgrad_scratch(dev, cin, cout)), N, hi, wi, cin, cout, stride, _ptr(conv.weight), _ptr(ops.bn_workspace(dev, cin)),
+                              wst)
+                    elif STAGED_WGRAD:
                         _call("cvad_flat_conv3x3_wgrad_staged_bf16", _ptr(a_in), _ptr(draw), _ptr(grad_buffer(conv.weight)),
                               _ptr(_wgrad_scratch(dev, cin, cout)), N, hi, wi, cin, cout, stride, wst)
                     else:
@@ -204,13 +214,10 @@ class _BackboneBF16(torch.autograd.Function):
                 grad_buffer(conv.bias)          # analytically zero (BatchNorm removes the mean); keep the tensor "with grad"
             if idx > 0:
                 dact = torch.empty(a_in.shape, device=dev, dtype=BF16)
-                _, raw_lo, mean_lo, invstd_lo, _, _, lo_training, _ = saved[idx - 1]
-                bn_lo = layers[idx - 1][1]
-                if FUSED_BN_BWD and lo_training and cin in (32, 64, 128, 256):
-                    # dact is the gradient w.r.t. relu(bn(raw_lo)): its epilogue also takes sum g / sum g*xhat for that BatchNorm's backward
-                    _call("cvad_flat_conv3x3_dgrad_bnstats_bf16", _ptr(draw), _ptr(wd), _ptr(dact), N, hi, wi, cin, cout, stride, _ptr(raw_lo),
-                          _ptr(bn_lo.weight), _ptr(bn_lo.bias), _ptr(mean_lo), _ptr(invstd_lo), _ptr(ops.bn_workspace(dev, cin)), st)
-                    sums_ready = True
+                if mask_lo is not None:
+                    # dact is the gradient w.r.t. relu(bn(raw_lo)): its epilogue also takes sum g under the ReLU mask of that layer
+                    _call("cvad_flat_conv3x3_dgrad_masksum_bf16", _ptr(draw), _ptr(wd), _ptr(dact), N, hi, wi, cin, cout, stride, _ptr(mask_lo),
+                          _ptr(ops.bn_workspace(dev, cin)), st)
                 else:
                     _call("cvad_flat_conv3x3_dgrad_bf16", _ptr(draw), _ptr(wd), _ptr(dact), N, hi, wi, cin, cout, stride, st)
             saved[idx] = None

@@ -267,6 +267,26 @@ int cvad_flat_conv3x3_dgrad_bnstats_bf16(const void* dy, const void* w_dgrad, vo
 int cvad_pad_bn_relu_bwd_apply_bf16(const void* raw, const void* dact, void* draw, int N, int H, int W, int C, int phase_in, const float* mean,
                                     const float* invstd, const float* gamma, const float* beta, int training, double* ws, float* dgamma,
                                     float* dbeta, void* stream);
+/* The BatchNorm backward's reductions without a pass of their own (cad:131-136 backward, train mode).  With act = relu(bn(raw)) of the layer
+ * below, dact = dL/d act and g = dact * (act > 0):
+ *   S1 = sum g: the data-gradient that writes dact sums its output under the ReLU mask the forward apply wrote (masksum below);
+ *   T = sum act*dact = sum_{co,tap} W*dW for every input channel of the convolution above, taken from its staged weight gradient (wdot);
+ * and gamma * sum g*xhat = T - beta*S1, so cvad_pad_bn_relu_bwd_tsum_bf16 finishes the backward in one pass over raw and dact.
+ * ws: the lower layer's BatchNorm workspace, 2*C fp64 (zero on entry; S1 in [0,C), T in [C,2C); zero again after the tsum call).
+ *
+ * Data-gradient (as cvad_flat_conv3x3_dgrad_bf16, dx bit-identical) that also adds sum_rows bf16(dx)*bit to ws[0..Cin); mask: Cin bits per
+ * row of dx in dx's own layout (cvad_pad_bn_apply_relu_mask_bf16).  Cin = 32, 64, 128 or 256. */
+int cvad_flat_conv3x3_dgrad_masksum_bf16(const void* dy, const void* w_dgrad, void* dx, int N, int H, int W, int Cin, int Cout, int stride,
+                                         const void* mask, double* ws, void* stream);
+/* Staged weight gradient (as cvad_flat_conv3x3_wgrad_staged_bf16) that also adds T[ci] = sum_{co,tap} bf16(w)*dW of this call (w: the fp32
+ * OIHW weight the data-gradient's bf16 pack was made from) to ws[Cin..2Cin).  Cin = 32, 64, 128 or 256. */
+int cvad_flat_conv3x3_wgrad_staged_wdot_bf16(const void* x, const void* dy, float* dw, float* scratch, int N, int H, int W, int Cin, int Cout,
+                                             int stride, const float* w, double* ws, void* stream);
+/* ReLU+BN backward (training mode) from S1 / T in ws: draw padded-flat with ZERO border; dgamma += sum g*xhat, dbeta += sum g (taken in the
+ * same pass; either may be NULL); ws re-zeroed */
+int cvad_pad_bn_relu_bwd_tsum_bf16(const void* raw, const void* dact, void* draw, int N, int H, int W, int C, int phase_in, const float* mean,
+                                   const float* invstd, const float* gamma, const float* beta, double* ws, float* dgamma, float* dbeta,
+                                   void* stream);
 /* development switch for the stride-2 data-gradient: 2 (default) = one launch, one work item per row tile fills all four phase planes of dx
  * from ONE fetch of the dy segment; 1 = one launch, one work item per (tile, plane); 0 = four launches */
 int cvad_flat_dgrad_mode(int mode);
@@ -289,6 +309,14 @@ int cvad_pad_bn_finalize_apply_relu_bf16(const void* raw, void* act, int N, int 
 /* act = relu(bn(raw)) written padded-flat with zero border (phase_out = 0) or as the four phase planes (phase_out = 1) */
 int cvad_pad_bn_apply_relu_bf16(const void* raw, void* act, int N, int H, int W, int C, int phase_out, const float* mean, const float* invstd,
                                 const float* gamma, const float* beta, void* stream);
+/* The two apply entries above that also write the ReLU gate: mask = numel(act)/8 bytes in act's row layout, C bits per pixel (bit c in 32-bit
+ * word c/32), set where act > 0 -- the same test as the backward's -- and 0 wherever act is zero by construction (border, empty plane
+ * positions) */
+int cvad_pad_bn_finalize_apply_relu_mask_bf16(const void* raw, void* act, void* mask, int N, int H, int W, int C, int phase_out, double* ws,
+                                              float eps, float momentum, const float* gamma, const float* beta, float* mean, float* invstd,
+                                              float* running_mean, float* running_var, long long* num_batches_tracked, void* stream);
+int cvad_pad_bn_apply_relu_mask_bf16(const void* raw, void* act, void* mask, int N, int H, int W, int C, int phase_out, const float* mean,
+                                     const float* invstd, const float* gamma, const float* beta, void* stream);
 /* ReLU+BN backward; dact padded-flat (phase_in = 0) or phase planes (phase_in = 1); draw padded-flat with ZERO border (may be NULL) */
 int cvad_pad_bn_relu_bwd_bf16(const void* raw, const void* dact, void* draw, int N, int H, int W, int C, int phase_in, const float* mean,
                               const float* invstd, const float* gamma, const float* beta, int training, double* ws, float* dgamma,

@@ -29,7 +29,7 @@ def main():
             lib.cvad_flat_tune(k, int(os.environ[f"CVAD_FC_TUNE{k}"]))
     flush = torch.empty(256 << 20, device=dev, dtype=torch.uint8)
     bf = torch.bfloat16
-    tot = {"fwd+stats": 0.0, "fwd": 0.0, "dgrad": 0.0, "wgrad-staged": 0.0, "wgrad": 0.0}
+    tot = {"fwd+stats": 0.0, "fwd": 0.0, "dgrad": 0.0, "dgrad-masksum": 0.0, "wgrad-staged": 0.0, "wgrad-staged-wdot": 0.0, "wgrad": 0.0}
     for li, (H, W, Ci, Co, s) in enumerate(LAYERS):
         Ho, Wo = tc.out_hw(H, W, s)
         xin = torch.randn(tc.act_shape(N, H, W, Ci, s == 2), device=dev).to(bf)
@@ -43,12 +43,18 @@ def main():
         dx = torch.empty_like(xin)
         dw = torch.zeros(Co, Ci, 3, 3, device=dev)
         ws = torch.zeros(2 * Co, device=dev, dtype=torch.float64)
+        ws_in = torch.zeros(4 * Ci, device=dev, dtype=torch.float64)
+        mask = torch.randint(0, 256, (xin.numel() // 8,), device=dev, dtype=torch.uint8)        # the ReLU bitmask of the layer below
         scr = torch.zeros(9 * Co * Ci, device=dev)
         calls = {
             "fwd+stats": lambda: _call("cvad_flat_conv3x3_fwd_stats_bf16", _ptr(xin), _ptr(wf), _ptr(b), _ptr(y), N, H, W, Ci, Co, s, _ptr(ws), _st()),
             "fwd": lambda: _call("cvad_flat_conv3x3_fwd_bf16", _ptr(xin), _ptr(wf), _ptr(b), _ptr(y), N, H, W, Ci, Co, s, _st()),
             "dgrad": lambda: _call("cvad_flat_conv3x3_dgrad_bf16", _ptr(dy), _ptr(wd), _ptr(dx), N, H, W, Ci, Co, s, _st()),
+            "dgrad-masksum": lambda: _call("cvad_flat_conv3x3_dgrad_masksum_bf16", _ptr(dy), _ptr(wd), _ptr(dx), N, H, W, Ci, Co, s, _ptr(mask),
+                                           _ptr(ws_in), _st()),
             "wgrad-staged": lambda: _call("cvad_flat_conv3x3_wgrad_staged_bf16", _ptr(xin), _ptr(dy), _ptr(dw), _ptr(scr), N, H, W, Ci, Co, s, _st()),
+            "wgrad-staged-wdot": lambda: _call("cvad_flat_conv3x3_wgrad_staged_wdot_bf16", _ptr(xin), _ptr(dy), _ptr(dw), _ptr(scr), N, H, W, Ci, Co,
+                                               s, _ptr(w), _ptr(ws_in), _st()),
             "wgrad": lambda: _call("cvad_flat_conv3x3_wgrad_bf16", _ptr(xin), _ptr(dy), _ptr(dw), N, H, W, Ci, Co, s, _st()),
         }
         if os.environ.get("STEP_ONLY"):           # exactly the convolution launches of one train step, once each (for an ncu metrics pass)
