@@ -101,7 +101,7 @@ def gru_last(P, x):
     bi, bh = P["traj_encoder.gru.bias_ih_l0"], P["traj_encoder.gru.bias_hh_l0"]
     N, T, _ = x.shape
     Hd = Wh.shape[1]
-    h = torch.zeros(N, Hd)
+    h = torch.zeros(N, Hd, dtype=x.dtype)
     for t in range(T):
         gi = F.linear(x[:, t], Wi, bi)
         gh = F.linear(h, Wh, bh)
@@ -118,8 +118,14 @@ def ma_forward(P: dict, x: torch.Tensor, eps: torch.Tensor, train: bool = False,
     anomaly_scores (B,), causal_factors (B,5,6), adjacency_matrices (B,6,6), kl_losses (B,),
     detections (B,T,5,4) + det_counts (B,T), n_tracks (B,), direct_predictions (B,2),
     causal_anomaly_scores (B,)."""
-    keep = keep or {}
     feats = backbone(P, x, train, new_stats)
+    return ma_tail(P, feats, eps, train, keep)
+
+
+def ma_tail(P: dict, feats: torch.Tensor, eps: torch.Tensor, train: bool = False, keep: dict | None = None):
+    """Everything behind the backbone: feats (B,T,6144) -> the dict of ``ma_forward``.  Runs in the features' dtype (float64 included:
+    the fp64 reference of the causal branch's kernels)."""
+    keep = keep or {}
     B, T, _ = feats.shape
     box, cnt = detect(P, feats, train, keep)
     ntr = cnt.max(dim=1).values                                              # tracks per clip, cad:260
@@ -138,7 +144,7 @@ def ma_forward(P: dict, x: torch.Tensor, eps: torch.Tensor, train: bool = False,
     kl = (klrow * trk_ok).sum(dim=1) / ntr
     # structure learner: rows/cols index TRACKS (cad:382-387), matrix is num_factors x num_factors
     node = F.linear(z, P["structure_learner.node_encoder.weight"], P["structure_learner.node_encoder.bias"])
-    adj = torch.zeros(B, NF, NF)
+    adj = torch.zeros(B, NF, NF, dtype=feats.dtype)
     pair = torch.cat([node.unsqueeze(2).expand(B, MAXDET, MAXDET, -1), node.unsqueeze(1).expand(B, MAXDET, MAXDET, -1)], dim=-1)
     e = _mlp(P, "structure_learner.edge_predictor", (0, 2), pair, ("relu", "sigmoid")).squeeze(-1)   # (B,5,5)
     emask = trk_ok.unsqueeze(2) * trk_ok.unsqueeze(1) * (1 - torch.eye(MAXDET))
@@ -171,7 +177,7 @@ def ma_forward(P: dict, x: torch.Tensor, eps: torch.Tensor, train: bool = False,
 
 def ma_loss(out: dict, labels: torch.Tensor):
     """cad:649-662.  CrossEntropy is applied to the already-softmaxed probabilities (double softmax)."""
-    y = labels.float()
+    y = labels.to(out["anomaly_scores"].dtype)
     ce = F.cross_entropy(out["direct_predictions"], labels)
     mse_final = F.mse_loss(out["anomaly_scores"], y)
     kl = out["kl_losses"]
