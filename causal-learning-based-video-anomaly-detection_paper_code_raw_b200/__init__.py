@@ -11,7 +11,9 @@ Public surface (mirrors the reference's Python seam, SURVEY.md 8b):
   ma0.StreamingWindowScorer (sliding windows over a frame stream: each frame's backbone pass is computed once)
   infer.GraphedStreamingScorer / infer.FrozenBackbone (the same windows, one CUDA graph replay per push; eval BatchNorm folded into the convolutions)
   infer.MultiStreamScorer (many cameras or the videos of a test set: one push and one CUDA graph replay per tick for all streams)
+  infer.MultiStreamClipScorer (the same service for the 3-D clip models M-B, M-C and M-E from raw camera frames)
   md.VideoAutoEncoder / md.train_model / md.calculate_anomaly_scores         causal_anomaly_detection1.py
+  infer.MultiStreamAutoEncoderScorer (many camera streams for M-D, one replay per tick; each frame encoded once)
   me.CausalAnomalyDetector / me.predict_anomaly_for_clip / me.score_windows  avenue_training_script_bbox.py
   train.train_improved_minicausal_vad (s2:339-468 driver with real resume, async checkpoints, history JSON)
   frames.DeviceFrames (uint8 frame cache on the device: cv2-exact bilinear resize, clip / sliding-window gather)

@@ -1,6 +1,7 @@
 // M-D (causal_anomaly_detection1.py) specific kernels: the LSTM(64->64) recurrence over T (cad1:182-188, 238-239), the
-// cosine-distance-to-memory anomaly score (cad1:262-301) and the reconstruction MSE with its gradient and the per-clip
-// error used by calculate_anomaly_scores (cad1:323-344, 545-552).  Convolutions, BatchNorm and the linear layers of the
+// cosine-distance-to-memory anomaly score (cad1:262-301), the reconstruction MSE with its gradient and the per-clip
+// error used by calculate_anomaly_scores (cad1:323-344, 545-552), and the scores of every window slot of S streams read
+// from their frame rings (infer.MultiStreamAutoEncoderScorer).  Convolutions, BatchNorm and the linear layers of the
 // autoencoder reuse the generic fp32 kernels (conv_f32.cu: a ConvTranspose2d forward IS the data-gradient kernel).
 #include "common.cuh"
 #include "cvad_b200.h"
@@ -98,16 +99,15 @@ __global__ void __launch_bounds__(LG) lstm_bwd_kernel(const float* __restrict__ 
   if (db_hh) atomicAdd(db_hh + g, dbias);
 }
 
-// score[b] = clamp(min_m (1 - clamp(cos(seq_b, mem_m), -1, 1)), 0, 2) / 2 over the first n_filled memory rows (cad1:279-294)
-__global__ void __launch_bounds__(128) memory_score_kernel(const float* __restrict__ seq, const float* __restrict__ mem, int n_filled, int D,
-                                                           float eps, float* __restrict__ score) {
-  extern __shared__ float sq[];          // normalised query [D]
-  __shared__ float red[32];
-  const int b = blockIdx.x;
+// cad1:279-294 for one query row q (D floats) by the whole block: clamp(min_m (1 - clamp(cos(q, mem_m), -1, 1)), 0, 2) / 2 over the
+// first n_filled rows of mem, returned to thread 0.  sq: D floats of shared memory, red: 32.  Each row's dot product is one thread's
+// sequential loop and the minimum is exact, so the value is the same at any block size (the norm of q too while D <= blockDim.x).
+__device__ float memory_score_block(const float* __restrict__ q, const float* __restrict__ mem, int n_filled, int D, float eps,
+                                    float* __restrict__ sq, float* __restrict__ red) {
   float part = 0.f;
-  for (int i = threadIdx.x; i < D; i += blockDim.x) { const float v = seq[(long long)b * D + i]; part = fmaf(v, v, part); }
+  for (int i = threadIdx.x; i < D; i += blockDim.x) { const float v = q[i]; part = fmaf(v, v, part); }
   const float nrm = fmaxf(sqrtf(block_sum(part, red)), eps);
-  for (int i = threadIdx.x; i < D; i += blockDim.x) sq[i] = seq[(long long)b * D + i] / nrm;
+  for (int i = threadIdx.x; i < D; i += blockDim.x) sq[i] = q[i] / nrm;
   __syncthreads();
   float best = 3.f;
   for (int m = threadIdx.x; m < n_filled; m += blockDim.x) {
@@ -124,10 +124,71 @@ __global__ void __launch_bounds__(128) memory_score_kernel(const float* __restri
   for (int o = 16; o > 0; o >>= 1) best = fminf(best, __shfl_xor_sync(0xffffffffu, best, o));
   if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = best;
   __syncthreads();
-  if (threadIdx.x == 0) {
-    float v = red[0];
+  float v = red[0];
+  if (threadIdx.x == 0)
     for (int w = 1; w < (int)(blockDim.x >> 5); ++w) v = fminf(v, red[w]);
-    score[b] = fminf(fmaxf(v, 0.f), 2.f) * 0.5f;
+  return fminf(fmaxf(v, 0.f), 2.f) * 0.5f;
+}
+
+// score[b] = memory_score_block(seq_b) over the first n_filled memory rows (cad1:279-294)
+__global__ void __launch_bounds__(128) memory_score_kernel(const float* __restrict__ seq, const float* __restrict__ mem, int n_filled, int D,
+                                                           float eps, float* __restrict__ score) {
+  extern __shared__ float sq[];          // normalised query [D]
+  __shared__ float red[32];
+  const int b = blockIdx.x;
+  const float s = memory_score_block(seq + (long long)b * D, mem, n_filled, D, eps, sq, red);
+  if (threadIdx.x == 0) score[b] = s;
+}
+
+// calculate_anomaly_scores (cad1:526-564) for every window slot of S streams, one CTA per slot (k, j) (stream_push, common.cuh):
+// recon_err = mean over the window's T frames x E values of (recon - x_t)^2, x_t read from stream k's frame ring (fp32 per thread and
+// vector, fp64 across the block, as recon_mse_kernel); mem_score = memory_score_block(z) over the first clamp(*memory_ptr, 0, memory_rows)
+// rows, 0 below 10 rows; score = 0.7 recon_err + 0.3 mem_score, rounded as the two products and the sum are in torch.  Unused slots
+// (j >= n_win_k) get zeros.
+__global__ void __launch_bounds__(256) streams_md_scores_kernel(const float4* __restrict__ rings, long long cap, long long E4, int T, int stride,
+                                                                long long m, const long long* __restrict__ cursors,
+                                                                const long long* __restrict__ push, const float4* __restrict__ recon,
+                                                                const float* __restrict__ z, const float* __restrict__ memory, int memory_rows,
+                                                                const long long* __restrict__ memory_ptr, int D, float* __restrict__ score,
+                                                                float* __restrict__ recon_err, float* __restrict__ mem_score) {
+  extern __shared__ float sq[];          // normalised query [D]
+  __shared__ float red[32];
+  __shared__ double shd[32];
+  cvad_pdl_enter();
+  const long long slot = blockIdx.x;
+  const int k = (int)(slot / m);
+  const long long j = slot - k * m;
+  const StreamPush p = stream_push(cursors, push, k, T, stride);
+  if (j >= p.n_win) {
+    if (threadIdx.x == 0) score[slot] = recon_err[slot] = mem_score[slot] = 0.f;
+    return;
+  }
+  const float4* rb = recon + slot * E4;
+  const float4* ring = rings + (long long)k * cap * E4;
+  const long long first = (p.next + j) * stride;
+  double acc = 0.0;
+  for (long long e = threadIdx.x; e < E4; e += blockDim.x) {
+    const float4 r = __ldg(rb + e);
+    float part = 0.f;
+#pragma unroll 4
+    for (int t = 0; t < T; ++t) {
+      const float4 x = __ldg(ring + ((first + t) % cap) * E4 + e);
+      const float d0 = r.x - x.x, d1 = r.y - x.y, d2 = r.z - x.z, d3 = r.w - x.w;
+      part = fmaf(d0, d0, part);
+      part = fmaf(d1, d1, part);
+      part = fmaf(d2, d2, part);
+      part = fmaf(d3, d3, part);
+    }
+    acc += (double)part;
+  }
+  acc = block_sum_d(acc, shd);
+  const long long filled = min(max(*memory_ptr, 0LL), (long long)memory_rows);       // the same value in every thread
+  const float ms = filled >= 10 ? memory_score_block(z + slot * D, memory, (int)filled, D, 1e-8f, sq, red) : 0.f;
+  if (threadIdx.x == 0) {
+    const float re = (float)(acc / ((double)T * (double)(4 * E4)));
+    recon_err[slot] = re;
+    mem_score[slot] = ms;
+    score[slot] = __fadd_rn(__fmul_rn(0.7f, re), __fmul_rn(0.3f, ms));
   }
 }
 
@@ -237,6 +298,21 @@ CVAD_API int cvad_lstm_bwd_f32(const float* dhT, const float* saved, const float
 CVAD_API int cvad_memory_score_f32(const float* seq, const float* memory, int B, int n_filled, int D, float* score, void* stream) {
   if (B <= 0) return 0;
   memory_score_kernel<<<B, 128, D * sizeof(float), (cudaStream_t)stream>>>(seq, memory, n_filled, D, 1e-8f, score);
+  CVAD_LAUNCH_CHECK();
+  return 0;
+}
+
+CVAD_API int cvad_streams_md_scores_f32(const float* frame_rings, int S, long long capacity, long long E, int T, int stride, long long m,
+                                        const long long* cursors, const long long* push, const float* recon, const float* z, const float* memory,
+                                        int memory_rows, const long long* memory_ptr, int D, float* score, float* recon_err, float* mem_score,
+                                        void* stream) {
+  if (!frame_rings || !cursors || !push || !recon || !z || !memory || !memory_ptr || !score || !recon_err || !mem_score || E <= 0 || E % 4 ||
+      S <= 0 || T <= 0 || stride <= 0 || capacity <= 0 || D <= 0 || memory_rows <= 0 || m < 0 || (((uintptr_t)frame_rings | (uintptr_t)recon) & 15))
+    return (int)cudaErrorInvalidValue;
+  if (m == 0) return 0;
+  cvad_launch_pdl(streams_md_scores_kernel, dim3((unsigned)(S * m)), dim3(256), (size_t)D * sizeof(float), (cudaStream_t)stream,
+                  reinterpret_cast<const float4*>(frame_rings), capacity, E / 4, T, stride, m, cursors, push, reinterpret_cast<const float4*>(recon),
+                  z, memory, memory_rows, memory_ptr, D, score, recon_err, mem_score);
   CVAD_LAUNCH_CHECK();
   return 0;
 }

@@ -1,4 +1,4 @@
-"""Low-latency inference: the per-frame (2-D backbone) models M-A and M-A0, and many camera streams for the 3-D clip models.
+"""Low-latency inference: the per-frame (2-D backbone) models M-A and M-A0, and many camera streams for the 3-D clip models and M-D.
 
 ``FrozenBackbone`` is the bf16 tensor-core backbone of tc.py specialised to eval mode.  An eval-mode BatchNorm is a constant per-channel
 affine map, so it is folded into the convolution in front of it once, at snapshot time (w' = w*s, b' = (b - running_mean)*s + beta,
@@ -16,8 +16,12 @@ each stream's position lives in a device-side cursor and each push carries a sma
 the same graph serves every push of that size whatever the streams' phases.  ``GraphedStreamingScorer`` is its one-stream case.
 
 ``MultiStreamClipScorer`` is the same service for M-B, M-C and M-E from raw camera frames: the rings hold cv2-resized frames instead of
-features, and every completed window is gathered from them and scored by the model's batched forward.  Both multi-stream scorers share
-their host-side bookkeeping (``_StreamBookkeeping``) and the device window rule (``stream_push``, mirrored by ``window_count``).
+features, and every completed window is gathered from them and scored by the model's batched forward.
+
+``MultiStreamAutoEncoderScorer`` is the same service for M-D: its eval-mode encoder is per frame, so each frame is encoded once into a ring
+of LSTM input projections, and each completed window runs only the recurrence, the decoder and its score kernel.  The three multi-stream
+scorers share their host-side bookkeeping (``_StreamBookkeeping``) and the device window rule (``stream_push``, mirrored by
+``window_count``).
 """
 from __future__ import annotations
 
@@ -422,3 +426,88 @@ class MultiStreamClipScorer(_StreamBookkeeping):
         if self.channels == 1:
             return [(s, w0, None, None) for (s,), w0 in res]
         return [(s, w0, a, f) for (s, a, f), w0 in res]
+
+
+class MultiStreamAutoEncoderScorer(_StreamBookkeeping):
+    """Sliding-window scoring of S camera streams for M-D (``md.VideoAutoEncoder``) with one CUDA graph replay per push for all of them:
+    per window the (score, reconstruction error, memory score) of ``md.calculate_anomaly_scores`` on the window's clip.
+
+    In eval mode M-D's frame encoder and the LSTM input projection gi = W_ih latent + b_ih are per frame, so each frame is encoded once,
+    however many windows contain it: the rings hold each stream's gi rows (S, capacity, 256) next to its frames (S, capacity, 4096), which
+    the reconstruction error reads.  What a window needs of its own is the LSTM recurrence from a zero state at its first frame, the
+    decoder and its two score terms.  ``push(frames, counts)`` runs: copy into static inputs -> ``model.encode_frames`` and the input
+    projection over all S*n frames -> write each stream's kept gi rows and frames into its rings at its device cursor
+    (``cvad_streams_ring_write_f32``) -> gather the gi rows of the windows each stream completed (m slots per stream,
+    ``cvad_streams_window_features_f32``) -> ``ops.lstm_last`` and the eval decoder over the S*m slots -> score every slot against its
+    window's frames in the frame ring and against the memory bank (``cvad_streams_md_scores_f32``; unused slots are zeros) -> advance the
+    cursors.  The memory bank's fill count ``memory_ptr`` is read on the device, so ``update_memory`` and ``load_state_dict`` reach the next
+    replay without a capture.
+
+    The scores equal ``calculate_anomaly_scores`` on the window clips up to the last bits: the encoder's 2048 -> 64 layer splits its
+    reduction by batch size, and here the batch is the S*n frames of a push.  Window w of a stream covers its frames w*stride + [0, clip_len)
+    and is scored as soon as they have arrived (``window_count``); bbox's loop over a finished video, ``range(0, F - window, stride)``,
+    stops one window earlier when (F - clip_len) % stride == 0: such a video gets one window more here, its last one.
+
+    Counts, ``reset``, ``n_frames``, ``next_window`` and the errors are those of ``MultiStreamScorer``.  The graph key is (n, m): at most
+    ceil(n / stride) + 1 graphs per push size.  Graphs share one memory pool and read the model's live tensors, so an in-place weight or
+    BatchNorm-statistic update needs no capture; a replaced tensor drops them."""
+
+    def __init__(self, model, streams, clip_len=8, stride=4, capacity=32):
+        from . import md
+        if not isinstance(model, md.VideoAutoEncoder):
+            raise TypeError(f"MultiStreamAutoEncoderScorer scores md.VideoAutoEncoder, not {type(model).__name__}")
+        super().__init__(model, streams, clip_len, stride, capacity)
+        self.frame_rings = None     # (S, capacity, 64*64) fp32: the frames the reconstruction error reads
+
+    def _new_ring(self, dev):
+        self.frame_rings = torch.zeros((self.streams, self.capacity, 64 * 64), device=dev, dtype=torch.float32)
+        return torch.zeros((self.streams, self.capacity, 4 * self.model.temporal_encoder.hidden_size), device=dev, dtype=torch.float32)
+
+    def _empty(self, dev):
+        return tuple(torch.empty(0, device=dev) for _ in range(3))
+
+    def _step(self, n, m):
+        model, S, T = self.model, self.streams, self.clip_len
+        lstm, G, E = model.temporal_encoder, self.rings.shape[2], self.frame_rings.shape[2]
+
+        def step(x, push):
+            x = x.contiguous().reshape(S * n, 1, 64, 64)
+            gi = ops.linear_act(model.encode_frames(x), lstm.weight_ih_l0, lstm.bias_ih_l0)
+            st = _st()
+            for src, ring, F in ((gi, self.rings, G), (x, self.frame_rings, E)):
+                _call("cvad_streams_ring_write_f32", _ptr(src), S, n, F, _ptr(ring), self.capacity, T, self.stride, _ptr(self.cursors),
+                      _ptr(push), st)
+            if m > 0:
+                win = torch.empty((S * m, T, G), device=x.device, dtype=torch.float32)
+                _call("cvad_streams_window_features_f32", _ptr(self.rings), S, self.capacity, self.stride, T, G, m, _ptr(self.cursors),
+                      _ptr(push), _ptr(win), st)
+                z = ops.lstm_last(win, lstm.weight_hh_l0, lstm.bias_hh_l0)
+                recon = model._decode_once(z, 1)
+                out = tuple(torch.empty(S * m, device=x.device, dtype=torch.float32) for _ in range(3))
+                mem = model.normal_memory
+                _call("cvad_streams_md_scores_f32", _ptr(self.frame_rings), S, self.capacity, E, T, self.stride, m, _ptr(self.cursors),
+                      _ptr(push), _ptr(recon), _ptr(z), _ptr(mem), mem.shape[0], _ptr(model.memory_ptr), mem.shape[1], *map(_ptr, out), st)
+            else:
+                out = self._empty(x.device)
+            _call("cvad_streams_cursor_advance", _ptr(self.cursors), S, T, self.stride, _ptr(push), st)
+            return out
+        return step
+
+    def _capture(self, n, m, frames, push):
+        # warm-up runs the step for real: the rings and the cursors are restored after it, so capturing does not advance the streams
+        return GraphedStep(self._step(n, m), (frames, push), mutated=(self.rings, self.frame_rings, self.cursors), pool=self.pool)
+
+    @torch.no_grad()
+    def push(self, frames, counts=None):
+        """frames (S, n, 1, 64, 64) or (S, n, 64, 64) float32 on the model's device, in the model's input range (what
+        ``calculate_anomaly_scores`` receives per clip); counts: S ints in [0, n], the frames each stream keeps (default n; the rows beyond
+        a count are encoded and discarded, so they must hold finite frames).  Returns one (scores, first window index, reconstruction
+        errors, memory scores) per stream, each (w,) for its w completed windows: the (scores, ..., recons, mems) of
+        ``calculate_anomaly_scores``."""
+        if frames.dtype != torch.float32:
+            raise TypeError(f"MultiStreamAutoEncoderScorer takes float32 frames in the model's input range, got {frames.dtype}")
+        if frames.dim() == 4:
+            frames = frames.unsqueeze(2)
+        if frames.dim() != 5 or tuple(frames.shape[2:]) != (1, 64, 64):
+            raise ValueError(f"expected (S, n, 1, 64, 64) or (S, n, 64, 64) frames, got {tuple(frames.shape)}")
+        return [(s, w0, r, mem) for (s, r, mem), w0 in self._push(frames, counts, ())]

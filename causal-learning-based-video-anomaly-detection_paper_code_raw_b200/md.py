@@ -98,16 +98,23 @@ class VideoAutoEncoder(nn.Module):
         self.memory_ptr.fill_(new)
 
     # ---- encoder / decoder
-    def encode_sequence(self, frames):
-        B, T, C, H, W = frames.shape
+    def encode_frames(self, x, groups=1):
+        """The frame encoder (cad1:227-234): x (N, C, 64, 64) -> latents (N, 64).  In train mode the BatchNorms take their batch
+        statistics over each of ``groups`` equal, contiguous blocks of frames (one time step each); in eval mode a frame's latent depends
+        on that frame alone."""
         e = self.encoder
-        groups = T if self.training else 1           # per-time-step batch statistics in train mode (cad1:227-231)
-        h = frames.transpose(0, 1).reshape(T * B, C, H, W)      # time-major: each step's B frames are contiguous
+        h = x
         for ci in (0, 3, 6, 9):
             conv, bn = e[ci], e[ci + 1]
             h = ops.conv_act(h, conv.weight, conv.bias, 2, 1, ACT_NONE)
             h = _bn(h, bn, groups)
-        lat = ops.linear_act(h.reshape(T * B, -1), e[13].weight, e[13].bias, ACT_TANH)           # (T*B, 64)
+        return ops.linear_act(h.reshape(x.shape[0], -1), e[13].weight, e[13].bias, ACT_TANH)
+
+    def encode_sequence(self, frames):
+        B, T, C, H, W = frames.shape
+        groups = T if self.training else 1           # per-time-step batch statistics in train mode (cad1:227-231)
+        h = frames.transpose(0, 1).reshape(T * B, C, H, W)      # time-major: each step's B frames are contiguous
+        lat = self.encode_frames(h, groups)                                                       # (T*B, 64)
         frame_features = lat.reshape(T, B, -1).transpose(0, 1)                                    # (B, T, 64) view
         lstm = self.temporal_encoder
         gi = ops.linear_act(frame_features.reshape(B * T, -1), lstm.weight_ih_l0, lstm.bias_ih_l0).reshape(B, T, -1)

@@ -376,6 +376,19 @@ int cvad_memory_score_f32(const float* seq, const float* memory, int B, int n_fi
  * error, loss = mean over everything, drecon = d loss / d recon in recon's own shape; any of the three may be NULL. */
 int cvad_recon_mse_f32(const float* recon, long long recon_t_stride, const float* frames, int B, int T, long long E, double* ws,
                        float* clip_err, float* loss, float* drecon, float* nonfinite_flag, void* stream);
+/* calculate_anomaly_scores (cad1:526-564) for every window slot of S streams whose frames live in rings (infer.MultiStreamAutoEncoderScorer):
+ * frame_rings (S, capacity, E) fp32; cursors, push and the window rule as for cvad_streams_ring_write_f32; slot (k, j) of the (S*m)
+ * outputs is window next_k + j of stream k (frames (next_k + j)*stride + [0,T) modulo capacity) when j < n_win_k.  recon (S*m, E) = one
+ * decoded frame per slot, z (S*m, D) = its sequence feature.  recon_err = mean over the window's T*E values of (recon - x_t)^2; mem_score =
+ * the cvad_memory_score_f32 value over the first clamp(*memory_ptr, 0, memory_rows) rows of memory (memory_rows, D), exactly 0 when fewer
+ * than 10 are filled (memory_ptr is read on the device, so a captured graph follows update_memory / load_state_dict); score = 0.7 *
+ * recon_err + 0.3 * mem_score.  Unused slots (j >= n_win_k) get zeros in all three.  Issue before cvad_streams_cursor_advance.
+ * Returns cudaErrorInvalidValue for a NULL pointer, E <= 0 or E % 4 != 0, frame_rings / recon not 16-byte aligned, a non-positive S / T /
+ * stride / capacity / D / memory_rows or a negative m, and 0 without a launch for m = 0. */
+int cvad_streams_md_scores_f32(const float* frame_rings, int S, long long capacity, long long E, int T, int stride, long long m,
+                               const long long* cursors, const long long* push, const float* recon, const float* z, const float* memory,
+                               int memory_rows, const long long* memory_ptr, int D, float* score, float* recon_err, float* mem_score,
+                               void* stream);
 
 /* ---- evaluation tail on the device (SURVEY.md 8(f2)): the numpy / sklearn host code that follows the hot path in the reference.
  * workspace: cvad_eval_workspace_bytes(n) bytes of device memory (caller-owned, any contents).
