@@ -147,11 +147,15 @@ class TrajectoryEncoder(nn.Module):
         self.gru = nn.GRU(input_dim, hidden_dim, batch_first=True, bidirectional=False)
         self.encoder = nn.Linear(hidden_dim, latent_dim)
 
-    def forward(self, traj, ntr):
+    def last_state(self, traj, ntr):
+        """traj (B,K,T,F) -> the GRU's last hidden state (B*K,64); zeros for track slots >= ntr."""
         B, K, T, F = traj.shape
         gi = ops.linear_act(traj.reshape(B * K * T, F), self.gru.weight_ih_l0, self.gru.bias_ih_l0)      # input projection GEMM
-        hT = ma_ops.gru_last(gi.view(B * K, T, -1), self.gru.weight_hh_l0, self.gru.bias_hh_l0, ntr)
-        return ops.linear_act(hT, self.encoder.weight, self.encoder.bias).view(B, K, -1)
+        return ma_ops.gru_last(gi.view(B * K, T, -1), self.gru.weight_hh_l0, self.gru.bias_hh_l0, ntr)
+
+    def forward(self, traj, ntr):
+        hT = self.last_state(traj, ntr)
+        return ops.linear_act(hT, self.encoder.weight, self.encoder.bias).view(traj.shape[0], traj.shape[1], -1)
 
 
 class CausalFactorExtractor(nn.Module):
@@ -205,6 +209,8 @@ class DynamicsPredictor(nn.Module):
 
 
 class EnhancedAnomalyScorer(nn.Module):
+    """cad:428-502.  Holds the three scorers' parameters; M-A runs them inside ma_ops.causal_branch."""
+
     def __init__(self, num_factors):
         super().__init__()
         self.num_factors = num_factors
@@ -214,28 +220,6 @@ class EnhancedAnomalyScorer(nn.Module):
                                            nn.Sigmoid())
         self.temporal_scorer = nn.Sequential(nn.Linear(num_factors, 32), nn.ReLU(), nn.Linear(32, 16), nn.ReLU(), nn.Linear(16, 1),
                                              nn.Sigmoid())
-
-    def forward(self, z, pred, ntr, noise, training):
-        cin, mn, tin = ma_ops.scorer_inputs(z, pred, ntr)
-        B = cin.shape[0]
-        keeps = [noise.keep_mask("scorer0", (B, 64), 0.2, cin.device), None, None] if training else None
-        # three independent chains: the motion / temporal scorers run on two further streams beside the causal scorer (forward and, through
-        # autograd's stream bookkeeping, backward)
-        cur = torch.cuda.current_stream()
-        sides = [ops.aux_stream(cin.device, 2), ops.aux_stream(cin.device, 3)] if TAIL_BRANCHES else [None, None]
-        for sd in sides:
-            if sd is not None:
-                sd.wait_stream(cur)
-        with (torch.cuda.stream(sides[0]) if sides[0] is not None else contextlib.nullcontext()):
-            ms = _mlp(self.motion_scorer, (0, 2, 4), mn, (ACT_RELU, ACT_RELU, ACT_SIGMOID))
-        with (torch.cuda.stream(sides[1]) if sides[1] is not None else contextlib.nullcontext()):
-            ts = _mlp(self.temporal_scorer, (0, 2, 4), tin, (ACT_RELU, ACT_RELU, ACT_SIGMOID))
-        cs = _mlp(self.causal_scorer, (0, 3, 5), cin, (ACT_RELU, ACT_RELU, ACT_SIGMOID), keeps, (0.2, 0, 0))
-        for sd, t in zip(sides, (ms, ts)):
-            if sd is not None:
-                cur.wait_stream(sd)
-                t.record_stream(cur)
-        return ma_ops.lincomb3(cs.reshape(B), 0.5, ms.reshape(B), 0.3, ts.reshape(B), 0.2)
 
 
 class _LazyList(collections.abc.Sequence):
@@ -290,6 +274,16 @@ class CausalAnomalyDetector(nn.Module):
         slots[id(self.structure_learner.structure_params)] = SLOT_NEVER
         return slots
 
+    def causal_branch_params(self):
+        """The 40 weight / bias tensors of the causal branch behind the GRU, in the order of ma_ops.causal_branch."""
+        sc = self.anomaly_scorer
+        layers = [self.traj_encoder.encoder, self.causal_extractor.encoder[0], self.causal_extractor.encoder[2], self.causal_extractor.mu_head,
+                  self.causal_extractor.logvar_head, self.structure_learner.node_encoder, self.structure_learner.edge_predictor[0],
+                  self.structure_learner.edge_predictor[2], *(self.dynamics_predictor.dynamics_net[i] for i in (0, 2, 4)),
+                  *(sc.causal_scorer[i] for i in (0, 3, 5)), *(sc.motion_scorer[i] for i in (0, 2, 4)),
+                  *(sc.temporal_scorer[i] for i in (0, 2, 4))]
+        return [t for lin in layers for t in (lin.weight, lin.bias)]
+
     def forward(self, video_frames, feature_cut=None):
         """``feature_cut``: a list that receives ``(features, leaf)`` -- the autograd graph is cut behind the backbone (``leaf`` is a
         detached copy the rest of the model consumes), so a trainer can run the tail's backward first and the backbone's backward
@@ -308,9 +302,10 @@ class CausalAnomalyDetector(nn.Module):
         dev = features.device
         f_det = self.flags[SLOT_DETECTOR:SLOT_DETECTOR + 1] if self.flags is not None else None
         f_str = self.flags[SLOT_STRUCTURE:SLOT_STRUCTURE + 1] if self.flags is not None else None
-        # The direct classifier (cad:525-538, 568-571) depends on the features only: it runs on a second stream beside the ~35 dependent
-        # launches of the causal branch (autograd replays the fork in the backward: the classifier's data-gradient chain and its 6144-wide
-        # GEMM run beside the causal branch's); in a captured step the two become parallel branches of the graph.
+        # The direct classifier (cad:525-538, 568-571) depends on the features only: it runs on a second stream beside the dependent
+        # launches of the detector, tracker, GRU and causal branch (autograd replays the fork in the backward: the classifier's
+        # data-gradient chain and its 6144-wide GEMM run beside the causal branch's); in a captured step the two become parallel branches
+        # of the graph.
         cur = torch.cuda.current_stream()
         side = ops.aux_stream(dev, 1) if TAIL_BRANCHES else None
         keeps = None
@@ -328,12 +323,11 @@ class CausalAnomalyDetector(nn.Module):
             direct = ma_ops.softmax_rows(logits)
         box, cnt, _src = self.detector(features, self.noise, self.training, f_det)
         traj, ntr = self.tracker(box, cnt, f_str)
-        enc = self.traj_encoder(traj, ntr)
+        hT = self.traj_encoder.last_state(traj, ntr)
         eps = self.noise.normal("eps", (B, 5, 6), dev)          # drawn in eval mode too (cad:328-331)
-        z, kl = self.causal_extractor(enc, ntr, eps)
-        adj = self.structure_learner(z, ntr)
-        pred = self.dynamics_predictor(z, adj)
-        causal = self.anomaly_scorer(z, pred, ntr, self.noise, self.training)
+        keep0 = self.noise.keep_mask("scorer0", (B, 64), 0.2, dev) if self.training else None
+        # everything from the GRU's last state to (z, kl, adj, causal score): one kernel forward, one backward
+        z, kl, adj, causal = ma_ops.causal_branch(hT, ntr, eps, keep0, self.causal_branch_params())
         if side is not None:
             cur.wait_stream(side)
             direct.record_stream(cur)

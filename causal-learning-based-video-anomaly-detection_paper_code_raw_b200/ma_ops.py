@@ -1,9 +1,9 @@
-"""autograd glue for the M-A causal-branch kernels (csrc/ma_tail.cu; ABI in include/cvad_b200.h)."""
+"""autograd glue for the M-A causal-branch kernels (csrc/ma_tail.cu, csrc/ma_branch.cu; ABI in include/cvad_b200.h)."""
 from __future__ import annotations
 
 import torch
 
-from .ops import _call, _cuda, _f32c, _ptr, _st, grad_buffer, _wants_grad
+from .ops import _call, _cuda, _f32c, _ptr, _ptr_array, _st, grad_buffer, _wants_grad
 
 MAXDET, NF, HID = 5, 6, 64
 
@@ -205,57 +205,55 @@ def structured(adj, z):
     return _Structured.apply(adj, z)
 
 
-class _ScorerInputs(torch.autograd.Function):
+# (in, out) of the 20 nn.Linear layers of the causal branch, in the order of cvad_ma_branch_*_f32's params (include/cvad_b200.h)
+BRANCH_LAYERS = ((64, 32), (32, 32), (32, 32), (32, 6), (32, 6), (6, 32), (64, 32), (32, 1), (6, 32), (32, 32), (32, 6), (18, 64), (64, 32),
+                 (32, 1), (12, 32), (32, 16), (16, 1), (6, 32), (32, 16), (16, 1))
+
+
+class _CausalBranch(torch.autograd.Function):
+    """hT (B*5,64), ntr (B) int32, eps (B,5,6), keep (B,64) or None, 40 parameters -> z (B,5,6), kl (B), adj (B,6,6), causal (B).
+    Parameter gradients are added into ``grad_buffer(p)`` on the current stream; the backward recomputes the forward."""
+
     @staticmethod
-    def forward(ctx, z, pred, ntr):
-        _cuda(z, pred, ntr)
-        z, pred = _f32c(z), _f32c(pred)
+    def forward(ctx, hT, ntr, eps, keep, *params):
+        _cuda(hT, ntr, eps, keep, *params)
+        for i, p in enumerate(params):
+            din, dout = BRANCH_LAYERS[i // 2]
+            if tuple(p.shape) != ((dout, din) if i % 2 == 0 else (dout,)) or p.dtype != torch.float32 or not p.is_contiguous():
+                raise ValueError(f"causal_branch: parameter {i} has shape {tuple(p.shape)} / {p.dtype}; the kernel is built for the "
+                                 "reference's layer widths (num_factors = 6) in contiguous fp32")
+        hT, eps = _f32c(hT), _f32c(eps)
+        keep = None if keep is None else _f32c(keep)
+        ntr = ntr.to(torch.int32).contiguous()
         B = ntr.shape[0]
-        cin = torch.empty((B, 18), device=z.device, dtype=torch.float32)
-        mn = torch.empty((B, 12), device=z.device, dtype=torch.float32)
-        tin = torch.empty((B, 6), device=z.device, dtype=torch.float32)
-        _call("cvad_scorer_inputs_f32", _ptr(z), _ptr(pred), _ptr(ntr), B, _ptr(cin), _ptr(mn), _ptr(tin), _st())
-        ctx.save_for_backward(cin, ntr)
-        return cin, mn, tin
+        dev = hT.device
+        z = torch.empty((B, MAXDET, NF), device=dev, dtype=torch.float32)
+        kl = torch.empty((B,), device=dev, dtype=torch.float32)
+        adj = torch.empty((B, NF, NF), device=dev, dtype=torch.float32)
+        causal = torch.empty((B,), device=dev, dtype=torch.float32)
+        _call("cvad_ma_branch_fwd_f32", _ptr(hT), _ptr(ntr), _ptr(eps), _ptr(keep), B, _ptr_array(params), _ptr(z), _ptr(kl), _ptr(adj),
+              _ptr(causal), _st())
+        ctx.save_for_backward(hT, ntr, eps, keep)
+        ctx.params = params
+        ctx.set_materialize_grads(False)      # an output without a gradient reaches the kernel as NULL, not as a tensor of zeros
+        return z, kl, adj, causal
 
     @staticmethod
-    def backward(ctx, dcin, dmn, dtin):
-        cin, ntr = ctx.saved_tensors
-        B = ntr.shape[0]
-        dcin, dmn, dtin = _f32c(dcin), _f32c(dmn), _f32c(dtin)
-        dz = torch.empty((B, MAXDET, NF), device=cin.device, dtype=torch.float32)
-        dpred = torch.empty_like(dz)
-        _call("cvad_scorer_inputs_bwd_f32", _ptr(cin), _ptr(ntr), B, _ptr(dcin), _ptr(dmn), _ptr(dtin), _ptr(dz), _ptr(dpred), _st())
-        return dz, dpred, None
+    def backward(ctx, dz, dkl, dadj, dcausal):
+        hT, ntr, eps, keep = ctx.saved_tensors
+        params = ctx.params
+        dz, dkl, dadj, dcausal = (None if g is None else _f32c(g) for g in (dz, dkl, dadj, dcausal))
+        dhT = torch.empty_like(hT)
+        grads = [grad_buffer(p) if _wants_grad(p) else None for p in params]
+        _call("cvad_ma_branch_bwd_f32", _ptr(hT), _ptr(ntr), _ptr(eps), _ptr(keep), ntr.shape[0], _ptr_array(params), _ptr(dz), _ptr(dkl),
+              _ptr(dadj), _ptr(dcausal), _ptr(dhT), _ptr_array(grads), _st())
+        return (dhT if ctx.needs_input_grad[0] else None, None, None, None) + (None,) * len(params)
 
 
-def scorer_inputs(z, pred, ntr):
-    return _ScorerInputs.apply(z, pred, ntr)
-
-
-class _LinComb3(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, x, a, y, b, z, c):
-        _cuda(x, y, z)
-        x, y, z = _f32c(x), _f32c(y), _f32c(z)
-        out = torch.empty_like(x)
-        _call("cvad_lincomb3_f32", _ptr(out), _ptr(x), float(a), _ptr(y), float(b), _ptr(z), float(c), x.numel(), _st())
-        ctx.coef = (a, b, c)
-        return out
-
-    @staticmethod
-    def backward(ctx, g):
-        g = _f32c(g)
-        outs = []
-        for coef in ctx.coef:
-            d = torch.empty_like(g)
-            _call("cvad_lincomb3_f32", _ptr(d), _ptr(g), float(coef), _ptr(g), 0.0, _ptr(g), 0.0, g.numel(), _st())
-            outs.append(d)
-        return outs[0], None, outs[1], None, outs[2], None
-
-
-def lincomb3(x, a, y, b, z, c):
-    return _LinComb3.apply(x, a, y, b, z, c)
+def causal_branch(hT, ntr, eps, keep, params):
+    """M-A's causal branch behind the GRU (cad:300-502) as one kernel forward and one backward.  ``params``: the 40 weight / bias tensors
+    in the order of BRANCH_LAYERS; ``keep``: the causal scorer's dropout keep-mask (training) or None."""
+    return _CausalBranch.apply(hT, ntr, eps, keep, *params)
 
 
 class _SoftmaxRows(torch.autograd.Function):

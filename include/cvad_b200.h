@@ -213,6 +213,24 @@ int cvad_scorer_inputs_bwd_f32(const float* cin, const int* ntr, int B, const fl
                                float* dpred, void* stream);
 /* cad:497: 0.5*causal + 0.3*motion + 0.2*temporal */
 int cvad_lincomb3_f32(float* out, const float* x, float a, const float* y, float b, const float* z, float c, long long n, void* stream);
+/* ---- M-A causal branch behind the GRU in one launch forward and one backward (ma_branch.cu), cad:300-502 -------------------
+ * hT (B*5,64) last GRU states (rows of slots >= ntr[b] are ignored), ntr (B) int32 in [1,5], eps (B,5,6), keep_scorer0 (B,64) the dropout
+ * keep-mask of the causal scorer's first layer (scaled by 1/0.8) or NULL (eval) ->
+ *   z (B,5,6) (0 for slots >= ntr[b]), kl (B) = mean over the clip's tracks, adj (B,6,6) (entries only for i != j, i,j < ntr[b]),
+ *   causal (B) = 0.5 causal_scorer + 0.3 motion_scorer + 0.2 temporal_scorer.
+ * params: 40 pointers, weight (out,in) row-major then bias of each nn.Linear, in this order:
+ *   traj_encoder.encoder (64->32); causal_extractor.encoder.0 (32->32), .2 (32->32); causal_extractor.mu_head (32->6), .logvar_head
+ *   (32->6); structure_learner.node_encoder (6->32), .edge_predictor.0 (64->32), .2 (32->1); dynamics_predictor.dynamics_net.0 (6->32),
+ *   .2 (32->32), .4 (32->6); anomaly_scorer.causal_scorer.0 (18->64), .3 (64->32), .5 (32->1); .motion_scorer.0 (12->32), .2 (32->16),
+ *   .4 (16->1); .temporal_scorer.0 (6->32), .2 (32->16), .4 (16->1).
+ * backward: recomputes the forward from (hT, ntr, eps, keep_scorer0); any of the upstream gradients dz (B,5,6), dkl (B), dadj (B,6,6),
+ * dcausal (B) may be NULL (= zero); writes dhT (B*5,64) (0 for inactive slots) and ADDS the parameter gradients into grads (40 pointers in
+ * the order of params; a NULL entry = that parameter needs no gradient).  The pointer arrays are host arrays, read during the call. */
+int cvad_ma_branch_fwd_f32(const float* hT, const int* ntr, const float* eps, const float* keep_scorer0, int B, const void* const* params,
+                           float* z, float* kl, float* adj, float* causal, void* stream);
+int cvad_ma_branch_bwd_f32(const float* hT, const int* ntr, const float* eps, const float* keep_scorer0, int B, const void* const* params,
+                           const float* dz, const float* dkl, const float* dadj, const float* dcausal, float* dhT, void* const* grads,
+                           void* stream);
 /* cad:537: nn.Softmax(dim=-1) over rows of C (small) entries */
 int cvad_softmax_rows_f32(const float* x, long long rows, int C, float* y, void* stream);
 int cvad_softmax_rows_bwd_f32(const float* y, const float* dy, long long rows, int C, float* dx, void* stream);
